@@ -3,7 +3,7 @@
 dominant kernel, an end-to-end number with host buffers and a CPU baseline.  Contract: task statement / DESIGN.md 5.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c5-weak|c5-strong] [--ftype f64|f32]
-                  [--size n] [--impl ours|reference]
+                  [--size n] [--impl ours|reference] [--dump-outputs DIR]
 
 Configurations (BASELINE.json `configs`, SURVEY.md 8(d)):
   c2        (default, the headline) 256^3 triply periodic, WENO5 + tracer b + BuoyancyTracer, FFT solver, RK3.
@@ -17,6 +17,10 @@ Configurations (BASELINE.json `configs`, SURVEY.md 8(d)):
 
 N > 1 is launched by torchrun (one rank per GPU).  One "step" = one full RK3 time step (3 stages, 3 pressure solves) of
 every cell of the workload.  Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR writes the prognostic fields (u, v, w and the tracers) as they stand after the last timed step to
+DIR/<name>.npy (rank 0's slab with several GPUs), so that two builds run with the same arguments -- hence the same seeded
+inputs -- can be compared output for output.
 """
 import argparse
 import json
@@ -44,6 +48,9 @@ NCU_TRAFFIC_BYTES_PER_FUSED_LAUNCH_C3 = 1.04e10
 
 METRIC = "grid-point updates/sec (RK3 step, 256^3 WENO5+FFT)"
 UNIT = "grid-point updates/s"
+
+# --dump-outputs writes at most this many bytes in all
+DUMP_BYTES = 64 * 10 ** 6
 
 
 def synthetic_state(shape, seed=2):
@@ -154,6 +161,23 @@ def cpu_reference_run(steps, warmup, sample_n=256, budget_s=150.0):
             f"(compiled OpenMP twin of the oracle, {cores} threads)", N)
 
 
+def dump_outputs(model, out_dir, seed=0):
+    """Writes every prognostic field's interior to out_dir/<name>.npy in the run's float type.  When the fields together
+    exceed DUMP_BYTES, each is replaced by its values at a seeded, sorted sample of flat column-major interior indices:
+    the sample depends only on the seed and the field's shape, so it is the same from run to run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {n: model.fields[n].interior() for n in model.names}
+    budget = DUMP_BYTES - 4096 * len(arrays)                   # room for the .npy headers
+    sample = sum(x.nbytes for x in arrays.values()) > budget
+    for n, x in arrays.items():
+        if sample:
+            k = budget // (len(arrays) * x.itemsize)
+            idx = np.unique(np.random.default_rng(seed).integers(0, x.size, k))
+            x = x.ravel(order="F")[idx]
+        np.save(os.path.join(out_dir, f"{n}.npy"), np.ascontiguousarray(x))
+
+
 def build_config(ob, np, a, arch, world, rank, FTYPE):
     """returns (model, dt, points per GPU, global shape, workload string, fields, algorithmic words per point per step)"""
     cfg = a.config
@@ -254,7 +278,11 @@ def main():
     ap.add_argument("--no-dist-parity", action="store_true")
     ap.add_argument("--ftype", default="f64", choices=["f64", "f32"],
                     help="arithmetic type of the run (the headline configuration is Float64; f32 is reported for reference)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the fields computed by the last timed step to DIR/<name>.npy (at most 64 MB in all)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -262,7 +290,7 @@ def main():
     if a.impl == "reference":
         if rank != 0:
             return
-        steps, warmup = max(1, a.steps), max(0, a.warmup)
+        steps, warmup = a.steps, a.warmup
         v, spstep, cores, sample, Ns = cpu_reference_run(steps, warmup, sample_n=a.size or 256)
         workload = (f"C2: {Ns}^3 triply-periodic NonhydrostaticModel, WENO5 + tracer b + BuoyancyTracer, FFT pressure solve, "
                     f"RK3, Float64 (CPU arm: bounded sample of the 256^3 workload; the per-point cost does not depend on N)")
@@ -325,6 +353,8 @@ def main():
     ms = ev0.elapsed_time(ev1)
     launches = ob.launch_count() - n0
     lib.ob200_profile_enable(0)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(model, a.dump_outputs)
     phases = {}
     fft_names = ("fft_x_fwd", "fft_y", "fft_z", "fft_z_fwd", "fft_z_inv", "fft_sync", "fft_x_inv", "fft_y_butterfly",
                  "fft_y_lines", "fft_y_copywait")
