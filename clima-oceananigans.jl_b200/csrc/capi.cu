@@ -758,6 +758,11 @@ template <class FT> static Phys<FT>& physOf(ob200_model* m);
 template <> Phys<float>& physOf<float>(ob200_model* m) { return m->P32; }
 template <> Phys<double>& physOf<double>(ob200_model* m) { return m->P64; }
 
+// interior node count of prognostic field q (u, v, w: Face along q) along dimension d
+static int forcing_table_length(const ob200_grid_desc& G, int q, int d) {
+    return G.N[d] + ((q == d && G.topology[d] == OB200_BOUNDED) ? 1 : 0);
+}
+
 template <class FT>
 static void build_phys(ob200_model* m) {
     Phys<FT>& P = physOf<FT>(m);
@@ -831,6 +836,27 @@ static void build_phys(ob200_model* m) {
     P.tilted = D.gravity_tilted;
     for (int d = 0; d < 3; ++d) P.ghat[d] = (FT)D.g_hat[d];
     P.ntr = D.ntracers;
+    // Relaxation forcings: the host's tables rounded to FT, stored at index 1..n (Julia index) of a model-owned buffer
+    auto table = [&](const double* src, int n) -> const FT* {
+        std::vector<FT> h(n + 1, FT(0));
+        for (int q = 0; q < n; ++q) h[q + 1] = (FT)src[q];
+        FT* dp = nullptr;
+        OB_CUDA(cudaMalloc(&dp, h.size() * sizeof(FT)));
+        m->owned.push_back(dp);
+        OB_CUDA(cudaMemcpy(dp, h.data(), h.size() * sizeof(FT), cudaMemcpyHostToDevice));
+        return dp;
+    };
+    for (int q = 0; q < 3 + 8; ++q) {
+        Relax<FT>& r = P.frc[q];
+        r = Relax<FT>{0, -1, -1, nullptr, nullptr, FT(0), FT(0)};
+        const ob200_forcing& F = D.forcing[q];
+        if (q >= m->nf || !F.active) continue;
+        r.on = 1;
+        r.md = F.mask_dim; r.td = F.target_dim;
+        r.mc = (FT)F.rate; r.tc = (FT)F.target_value;
+        if (r.md >= 0) r.M = table(F.mask, forcing_table_length(m->grid->desc, q, r.md));
+        if (r.td >= 0) r.T = table(F.target, forcing_table_length(m->grid->desc, q, r.td));
+    }
 }
 
 extern "C" int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model** out) {
@@ -859,6 +885,21 @@ extern "C" int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model*
             throw Error("SeawaterBuoyancy needs an active temperature or salinity tracer");
     }
     const ob200_grid_desc& GD = desc->grid->desc;
+    // Relaxation forcings (Forcings/relaxation.jl): tables along non-Flat dimensions only, present where a dimension is given
+    for (int q = 0; q < 3 + OB200_MAX_TRACERS; ++q) {
+        const ob200_forcing& F = desc->forcing[q];
+        if (!F.active) continue;
+        const std::string who = "forcing of prognostic field " + std::to_string(q);
+        if (q >= 3 + desc->ntracers) throw Error(who + ": the model has no such field");
+        for (int pass = 0; pass < 2; ++pass) {
+            const int d = pass ? F.target_dim : F.mask_dim;
+            const double* t = pass ? F.target : F.mask;
+            const char* what = pass ? "target" : "mask";
+            if (d < -1 || d > 2) throw Error(who + ": " + what + " dimension out of range");
+            if (d >= 0 && GD.topology[d] == OB200_FLAT) throw Error(who + ": " + what + " along a Flat dimension");
+            if (d >= 0 && !t) throw Error(who + ": " + what + " table missing");
+        }
+    }
     // required halo: Advection.jl:40 (buffer + 1), closures need 1
     static const int need[7] = {1, 1, 2, 2, 2, 3, 3};
     for (int d = 0; d < 3; ++d)
@@ -890,6 +931,7 @@ extern "C" int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model*
     if (m->grid->ftype == OB200_F32) build_phys<float>(m.get());
     else build_phys<double>(m.get());
     for (int d = 0; d < 3; ++d) for (int l = 0; l < 2; ++l) m->desc.weno_coeff[d][l] = nullptr;
+    for (ob200_forcing& F : m->desc.forcing) F.mask = F.target = nullptr;      // borrowed host tables: copied to the device
     *out = m.release();
     if (ob200_model_update_state(*out)) { delete *out; *out = nullptr; throw Error(ob::g_err); }
     API_END

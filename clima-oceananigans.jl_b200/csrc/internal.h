@@ -69,6 +69,7 @@ struct FusedFields {
     Substep<FT> ss;
     FluxBC<FT> fbc[FUSED_MAXF];      // constant Flux boundary conditions (Bounded z variant)
     bool accumulate = false;         // G^n already holds the closure's part (launch_tendency_general closure_only): add to it
+    bool forcing_in_gn = false;      // G^n already holds the forcing (tendency_fused.cu launch_frc): add to it
 };
 // part: 0 = every tile; 1 = the tile rows whose stencils stay inside the rows this rank owns along a slab-decomposed y (they
 // need no neighbour data); 2 = the remaining (boundary) tile rows.  Returns the number of fields handled, 0 = not applicable.

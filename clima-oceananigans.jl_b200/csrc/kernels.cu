@@ -489,6 +489,8 @@ __global__ void __launch_bounds__(256, (CO ? 4 : 3)) tendency_shared_kernel(cons
                 if (A.pHY) G = G - deriv(g, A.pHY, q, 1, OB_F);
             }
             if (COMP < 2 && P.tilted && A.b.mode) G = G + P.ghat[COMP] * buoyancy_at(A.b, q.p);      // x/y_dot_g_b (g_dot_b.jl:1-3)
+            // + forcing, last in the sum (the descriptor read from the kernel parameter: `comp` may be run-time data)
+            if (Pin.frc[comp].on) G = G + relaxation(Pin.frc[comp], q.i[0], q.i[1], q.i[2], A.psi[q.p]);
             // apply_x/y/z_bcs! (apply_flux_bcs.jl:35-160): constant Flux BCs of this field
 #pragma unroll
             for (int d = 0; d < 3; ++d) {

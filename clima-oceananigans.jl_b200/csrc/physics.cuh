@@ -39,6 +39,24 @@ OBD FT buoyancy_at(const Buoy<FT>& B, long long p) {
     }
 }
 
+// Relaxation(; rate, mask, target) of one prognostic field (Forcings/relaxation.jl): rate * mask and target tabulated by the
+// host at the field's own nodes along one dimension each (capi.cu build_phys); md / td = -1: the constant mc / tc
+template <class FT>
+struct Relax {
+    int on;
+    int md, td;                      // dimension of the mask / target table, -1 = constant
+    const FT* M;                     // rate * mask, Julia index 1..n along md
+    const FT* T;                     // target, Julia index 1..n along td
+    FT mc, tc;
+};
+// the forcing term rate * mask * (target - ψ) at Julia indices (i, j, k), ψ = the forced field there
+template <class FT>
+OBD FT relaxation(const Relax<FT>& r, int i, int j, int k, FT psi) {
+    const FT M = r.md < 0 ? r.mc : __ldg(r.M + (r.md == 0 ? i : (r.md == 1 ? j : k)));
+    const FT T = r.td < 0 ? r.tc : __ldg(r.T + (r.td == 0 ? i : (r.td == 1 ? j : k)));
+    return M * (T - psi);
+}
+
 template <class FT>
 struct Phys {
     GridD<FT> g;
@@ -58,6 +76,7 @@ struct Phys {
     int btr, tilted;                 // buoyancy tracer index (-1 none); tilted gravity flag
     FT ghat[3];
     int ntr;
+    Relax<FT> frc[3 + 8];            // forcing of u, v, w, tracers (on = 0: none)
 };
 
 struct Pt {
@@ -779,6 +798,7 @@ OBD FT tendency(const Phys<FT>& P, int comp, const FT* const* U, const FT* psi, 
     if (comp >= 3) {
         FT G = -div_Uc(P, U, psi, q);
         G = G - div_q(P, P.kappa[comp - 3], psi, q, P.kappae[comp - 3]);
+        if (P.frc[comp].on) G = G + relaxation(P.frc[comp], q.i[0], q.i[1], q.i[2], psi[q.p]);     // + forcing (:231)
         return G;
     }
     FT G = -div_Uu(P, comp, U, psi, q);
@@ -799,6 +819,7 @@ OBD FT tendency(const Phys<FT>& P, int comp, const FT* const* U, const FT* psi, 
     }
     G = G - div_tau(P, comp, U, q);
     if (comp < 2 && P.tilted && b.mode) G = G + P.ghat[comp] * buoyancy_at(b, q.p);      // x/y_dot_g_b (g_dot_b.jl:1-3)
+    if (P.frc[comp].on) G = G + relaxation(P.frc[comp], q.i[0], q.i[1], q.i[2], psi[q.p]);     // + forcings.u/v/w (:71, :128, :180)
     return G;
 }
 

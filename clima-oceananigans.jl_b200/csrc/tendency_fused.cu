@@ -39,6 +39,7 @@
 #include "tma_util.cuh"
 #include <algorithm>
 #include <cstdlib>
+#include <type_traits>
 
 namespace ob {
 namespace fz {
@@ -85,6 +86,12 @@ struct Args {
     FT th[2], t2;          // -2 κ / Δx, -2 κ / Δy, -2 κ       (diffusive fluxes of the tracer, 2 x units)
     FT fbb[NF], fbt[NF];   // constant Flux boundary conditions at the bottom / top (0: none)
 };
+// the forced instantiations (FRC) take the relaxation forcing of every field in addition; the unforced ones keep Args
+template <class FT, int NF>
+struct ArgsF : Args<FT, NF> {
+    Relax<FT> frc[NF];
+};
+template <class FT, int NF, bool FRC> using KArgs = std::conditional_t<FRC, ArgsF<FT, NF>, Args<FT, NF>>;
 
 // ---- work decomposition: whole tiles in lockstep rounds, then the leftover tiles split along z ----------------
 // (all 32-bit and a pure function of blockIdx / gridDim / kernel parameters, so that the level index and the ring-slot
@@ -308,8 +315,8 @@ __device__ __forceinline__ void cell_flux_z(const Args<FT, NF>& c, int k, const 
     Fz = Fn;
 }
 
-template <class FT, bool ZW, int ZT, int NT, bool HAS_GM, bool ACC, int R, int GRP>
-__device__ __forceinline__ void group_main(const Args<FT, 3 + NT>& c, FT* S, FT* sX, unsigned long long* full,
+template <class FT, bool ZW, int ZT, int NT, bool HAS_GM, bool ACC, int R, int GRP, bool FRC>
+__device__ __forceinline__ void group_main(const KArgs<FT, 3 + NT, FRC>& c, FT* S, FT* sX, unsigned long long* full,
                                            unsigned long long* done) {
     using GR = Groups<NT>;
     constexpr int NF = GR::NF, FPG = GR::FPG;
@@ -443,6 +450,9 @@ __device__ __forceinline__ void group_main(const Args<FT, 3 + NT>& c, FT* S, FT*
                         }
                         if (c.pHY) Gv = Gv - (ph - phy) * c.invdy;
                     }
+                    if constexpr (FRC) {          // + forcing, last in the sum (Relaxation at the field's own nodes)
+                        if (c.frc[f].on) Gv = Gv + relaxation(c.frc[f], i0 + tx, j0 + ty, k, S[f * SLOTS * PE + so[3] + e]);
+                    }
                     if constexpr (ACC) Gv = Gv + c.Gn[f][p];
                     c.Gn[f][p] = Gv;
                     if (c.do_sub) {
@@ -458,9 +468,9 @@ __device__ __forceinline__ void group_main(const Args<FT, 3 + NT>& c, FT* S, FT*
     }
 }
 
-template <class FT, bool ZW, int ZT, int NT, bool HAS_GM, bool ACC, int R>
+template <class FT, bool ZW, int ZT, int NT, bool HAS_GM, bool ACC, int R, bool FRC>
 __global__ void __launch_bounds__(TX*(Groups<NT>::NG*(R + 1) + 1), 1)
-tendency_fused_kernel(const __grid_constant__ Args<FT, 3 + NT> c) {
+tendency_fused_kernel(const __grid_constant__ KArgs<FT, 3 + NT, FRC> c) {
     using GR = Groups<NT>;
     constexpr int NF = GR::NF, NG = GR::NG;
     using G_ = Geo<FT, R, NF>;
@@ -511,23 +521,61 @@ tendency_fused_kernel(const __grid_constant__ Args<FT, 3 + NT> c) {
         return;
     }
     const int grp = warp / (R + 1);
-    if (grp == 0) group_main<FT, ZW, ZT, NT, HAS_GM, ACC, R, 0>(c, S, sX, full, done);
-    else if (grp == 1) group_main<FT, ZW, ZT, NT, HAS_GM, ACC, R, 1>(c, S, sX, full, done);
-    else if (NG > 2) group_main<FT, ZW, ZT, NT, HAS_GM, ACC, R, (NG > 2 ? 2 : 0)>(c, S, sX, full, done);
+    if (grp == 0) group_main<FT, ZW, ZT, NT, HAS_GM, ACC, R, 0, FRC>(c, S, sX, full, done);
+    else if (grp == 1) group_main<FT, ZW, ZT, NT, HAS_GM, ACC, R, 1, FRC>(c, S, sX, full, done);
+    else if (NG > 2) group_main<FT, ZW, ZT, NT, HAS_GM, ACC, R, (NG > 2 ? 2 : 0), FRC>(c, S, sX, full, done);
 }
 
 // ---- host side --------------------------------------------------------------------------------
-template <class FT, bool ZW, int ZT, int NT, bool HAS_GM, bool ACC, int R>
+// part launches (FusedFields / launch): whether the grid has interior tile rows to split off
+template <int R>
+static bool part_applicable(int Ny, int part) {
+    if (!part) return true;
+    const int nty = cdiv(Ny, R);
+    int nb_hi = 0;
+    while (nb_hi < nty && (nty - nb_hi) * R + HALO > Ny) ++nb_hi;
+    return nty - nb_hi - 1 >= 1 && R >= HALO;
+}
+
+// Relaxation forcing of the fused fields as a pointwise pass into G^n (G^n = F, or G^n += F over the closure's part), for the
+// accumulate instantiations to add the rest: the forced FP64 variants with a tracer that would spill with the term in the
+// epilogue (launch_frc).  The accumulate form adds G^n of EVERY field, so without the closure's part the unforced fields'
+// G^n are cleared here
+template <class FT>
+struct RelaxPass {
+    int nf, acc;
+    const FT* psi[FUSED_MAXF];
+    FT* Gn[FUSED_MAXF];
+    Relax<FT> frc[FUSED_MAXF];
+    long long sy, sz;
+    int N[3];
+};
+template <class FT>
+__global__ void __launch_bounds__(128) relaxation_pass_kernel(const __grid_constant__ RelaxPass<FT> a) {
+    const int i = 1 + blockIdx.x * blockDim.x + threadIdx.x, j = 1 + blockIdx.y * blockDim.y + threadIdx.y, k = 1 + blockIdx.z;
+    if (i > a.N[0] || j > a.N[1]) return;
+    const long long p = i + j * a.sy + k * a.sz;
+    for (int f = 0; f < a.nf; ++f) {
+        if (!a.frc[f].on) {
+            if (!a.acc) a.Gn[f][p] = FT(0);
+            continue;
+        }
+        const FT F = relaxation(a.frc[f], i, j, k, a.psi[f][p]);
+        a.Gn[f][p] = a.acc ? a.Gn[f][p] + F : F;
+    }
+}
+template <class FT, bool ZW, int ZT, int NT, bool HAS_GM, bool ACC, int R, bool FRC>
 static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
     using GR = Groups<NT>;
     constexpr int NF = GR::NF;
     using G_ = Geo<FT, R, NF>;
     static_assert(G_::SMEM <= 227 * 1024 - 64, "shared memory budget");
     const GridD<FT>& g = P.g;
-    Args<FT, NF> c;
+    KArgs<FT, NF, FRC> c;
     for (int f = 0; f < NF; ++f) {
         c.tm[f] = tmau::make_map<FT>(g, a.state[f] - g.off0, BX, G_::BY);
         c.Gm[f] = a.Gm[f]; c.Gn[f] = a.Gn[f]; c.nw[f] = a.nw[f];
+        if constexpr (FRC) c.frc[f] = P.frc[f];
     }
     c.pHY = a.pHY;
     c.sy = g.st[1]; c.sz = g.st[2];
@@ -539,6 +587,7 @@ static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part
         c.ntiles = c.ntx * nty;
         c.tile0 = 0; c.tsplit = 1 << 30; c.tskip = 0;
         if (part) {
+            if (!part_applicable<R>(g.N[1], part)) return false;
             // tile rows at the high end whose stencil (HALO rows beyond the tile) reaches past row Ny
             int nb_hi = 0;
             while (nb_hi < nty && (nty - nb_hi) * R + HALO > g.N[1]) ++nb_hi;
@@ -570,7 +619,7 @@ static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part
     c.do_sub = ss.mode != SUB_NONE;
     c.ca = ss.mode == SUB_RK3_FIRST ? ss.c1 : ss.dt * ss.c1;
     c.cb = ss.mode == SUB_RK3 ? ss.dt * ss.c2 : (ss.mode == SUB_AB2 ? -(ss.dt * ss.c2) : FT(0));
-    auto kern = tendency_fused_kernel<FT, ZW, ZT, NT, HAS_GM, ACC, R>;
+    auto kern = tendency_fused_kernel<FT, ZW, ZT, NT, HAS_GM, ACC, R, FRC>;
     static bool attr_set = false;      // per instantiation
     if (!attr_set) {
         OB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM));
@@ -593,20 +642,50 @@ static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part
     return true;
 }
 
-template <class FT, bool ZW, int ZT, int NT, int R>
+template <class FT, bool ZW, int ZT, int NT, int R, bool FRC>
 static bool launch_gm(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
     const bool has_gm = a.ss.mode == SUB_RK3 || a.ss.mode == SUB_AB2;
-    // the accumulate form (closure's part precomputed into G^n) exists for the variants with a tracer
+    // the accumulate form (closure's part and / or the forcing precomputed into G^n) exists for the variants with a tracer
     if constexpr (NT == 1) {
-        if (a.accumulate) {
-            if (has_gm) return launch_variant<FT, ZW, ZT, NT, true, true, R>(P, a, part);
-            return launch_variant<FT, ZW, ZT, NT, false, true, R>(P, a, part);
+        if (a.accumulate || a.forcing_in_gn) {
+            if (has_gm) return launch_variant<FT, ZW, ZT, NT, true, true, R, FRC>(P, a, part);
+            return launch_variant<FT, ZW, ZT, NT, false, true, R, FRC>(P, a, part);
         }
     } else {
-        if (a.accumulate) return false;
+        if (a.accumulate || a.forcing_in_gn) return false;
     }
-    if (has_gm) return launch_variant<FT, ZW, ZT, NT, true, false, R>(P, a, part);
-    return launch_variant<FT, ZW, ZT, NT, false, false, R>(P, a, part);
+    if (has_gm) return launch_variant<FT, ZW, ZT, NT, true, false, R, FRC>(P, a, part);
+    return launch_variant<FT, ZW, ZT, NT, false, false, R, FRC>(P, a, part);
+}
+// a model with a forced field among the fused ones takes the FRC instantiations (the term in the per-cell epilogue); every
+// other keeps the unforced kernels.  The FP64 variants with a tracer are at the 72-register cap already and would spill
+// 16-100 bytes more with the term (ptxas -v, sm_100a): there a pointwise pass writes the forcing into G^n and the
+// accumulate instantiation adds the rest, one extra read and write of G^n and a read of the field per forced field
+template <class FT, bool ZW, int ZT, int NT, int R>
+static bool launch_frc(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
+    constexpr int NF = 3 + NT;
+    bool frc = false;
+    for (int f = 0; f < NF; ++f) frc = frc || P.frc[f].on;
+    if (!frc) return launch_gm<FT, ZW, ZT, NT, R, false>(P, a, part);
+    if constexpr (sizeof(FT) == 4 || NT == 0) {
+        return launch_gm<FT, ZW, ZT, NT, R, true>(P, a, part);
+    } else {
+        const GridD<FT>& g = P.g;
+        if (!part_applicable<R>(g.N[1], part)) return false;
+        if (part != 2) {               // once per stage: before the first (or the only) part
+            RelaxPass<FT> r;
+            r.nf = NF; r.acc = a.accumulate ? 1 : 0;
+            for (int f = 0; f < NF; ++f) { r.psi[f] = a.state[f]; r.Gn[f] = a.Gn[f]; r.frc[f] = P.frc[f]; }
+            r.sy = g.st[1]; r.sz = g.st[2];
+            for (int d = 0; d < 3; ++d) r.N[d] = g.N[d];
+            dim3 blk(32, 4, 1), grd(cdiv(g.N[0], 32), cdiv(g.N[1], 4), g.N[2]);
+            relaxation_pass_kernel<FT><<<grd, blk, 0, stream()>>>(r);
+            OB_LAUNCH_CHECK();
+        }
+        FusedFields<FT> b = a;
+        b.forcing_in_gn = true;
+        return launch_gm<FT, ZW, ZT, NT, R, false>(P, b, part);
+    }
 }
 
 // the configuration checks: returns -1 (not applicable) or the z variant (0 Periodic regular, 1 Bounded); `native` = the kernel
@@ -662,7 +741,7 @@ int launch(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
     (void)g;
     bool ok = false;
 #define GO(ZTV, NTV, RV)                                                                        \
-    { ok = P.zweno ? launch_gm<FT, true, ZTV, NTV, RV>(P, a, part) : launch_gm<FT, false, ZTV, NTV, RV>(P, a, part); }
+    { ok = P.zweno ? launch_frc<FT, true, ZTV, NTV, RV>(P, a, part) : launch_frc<FT, false, ZTV, NTV, RV>(P, a, part); }
     // rows per tile: the largest for which the block (NG (R + 1) + 1 warps) keeps 72 registers per thread and the rings
     // + exchange buffers fit 227 KB; measured at 256^3: R = 12 3.13 ms per step, 11: 3.16, 10: 3.26, 9: 3.19
     if (zt) GO(1, 1, 12)         // Bounded z at 512 x 512 x 256: R = 12 15.4 ms per step of tendencies, 10: 17.2, 8: 15.4

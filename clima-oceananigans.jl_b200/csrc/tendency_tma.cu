@@ -362,6 +362,7 @@ template <class FT>
 bool launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, const FT* pHY, FT* Gn, const FT* Gm,
             FT* psi_new, const Substep<FT>& ss) {
     const GridD<FT>& g = P.g;
+    if (P.frc[comp].on) return false;          // forced fields run on the general kernels
     if (g.topo[2] == OB_FLAT || g.N[0] % TX) return false;
     if ((g.S[0] * sizeof(FT)) % 16) return false;
     Ctx<FT> c;

@@ -30,6 +30,8 @@ using Oceananigans.TimeSteppers: RungeKutta3TimeStepper, QuasiAdamsBashforth2Tim
 using Oceananigans.Solvers: FFTBasedPoissonSolver, FourierTridiagonalPoissonSolver, BatchedTridiagonalSolver
 using Oceananigans.Models.NonhydrostaticModels: NonhydrostaticModel
 using Oceananigans.Utils: tupleit
+using Oceananigans.Forcings: Relaxation, GaussianMask, LinearTarget
+using Oceananigans.Grids: xnodes, ynodes, znodes, topology
 
 import Base: zeros, size, Array, copyto!
 import Oceananigans.Architectures: device, array_type, arch_array, architecture, device_event, unsafe_free!
@@ -131,6 +133,10 @@ struct GridDesc
 end
 struct BC; kind::Int32; value::Float64; end
 const MAX_TRACERS = 8
+struct ForcingDesc          # ob200_forcing
+    active::Int32; mask_dim::Int32; rate::Float64; mask::Ptr{Float64}
+    target_dim::Int32; target_value::Float64; target::Ptr{Float64}
+end
 struct ModelDesc
     grid::Ptr{Cvoid}; timestepper::Int32; chi::Float64; advection::Int32; weno_zweno::Int32
     weno_coeff::NTuple{6,Ptr{Float64}}                     # [d][loc], d-major
@@ -142,6 +148,7 @@ struct ModelDesc
     smagorinsky_C::Float64; smagorinsky_Cb::Float64; prandtl::NTuple{MAX_TRACERS,Float64}
     amd_Cnu::Float64; amd_Ckappa::NTuple{MAX_TRACERS,Float64}; amd_Cb::Float64; amd_has_Cb::Int32
     closure_vertically_implicit::Int32
+    forcing::NTuple{3 + MAX_TRACERS, ForcingDesc}
 end
 
 topo_code(::Type{Periodic}) = Int32(0); topo_code(::Type{Bounded}) = Int32(1); topo_code(::Type{Flat}) = Int32(2)
@@ -311,13 +318,60 @@ function weno_tables(a::WENO5)
 end
 weno_tables(::Any) = ntuple(_ -> Float64[], 6)
 
+# ---- forcing: Relaxation(; rate, mask, target) (Forcings/relaxation.jl) tabulated at the forced field's nodes ----------------
+# the types of the defaults mask = onefunction, target = zerofunction, taken from the constructor itself
+const OneFunction = typeof(Relaxation(rate = 1).mask)
+const ZeroFunction = typeof(Relaxation(rate = 1).target)
+const SupportedRelaxation = Relaxation{<:Number, <:Union{OneFunction, GaussianMask}, <:Union{Number, ZeroFunction, LinearTarget}}
+dim_code(::GaussianMask{D}) where D = D === :x ? 0 : D === :y ? 1 : 2
+dim_code(::LinearTarget{D}) where D = D === :x ? 0 : D === :y ? 1 : 2
+function forcing_nodes(grid, loc, d, what)
+    topology(grid, d + 1) === Flat && throw(ArgumentError("B200(): Relaxation $what along the Flat dimension $("xyz"[d + 1])"))
+    ξ = (xnodes, ynodes, znodes)[d + 1](loc[d + 1](), grid)
+    return ξ
+end
+"(active, mask_dim, rate, mask table, target_dim, target value, target table) of one Relaxation at location `loc`"
+function relaxation_tables(r::SupportedRelaxation, grid, loc)
+    node(d, ξ) = ntuple(q -> q == d + 1 ? ξ : zero(ξ), 3)
+    md, M = -1, Float64[]
+    if r.mask isa GaussianMask
+        md = dim_code(r.mask)
+        M = Float64[r.rate * r.mask(node(md, ξ)...) for ξ in forcing_nodes(grid, loc, md, "mask")]     # rate * mask first
+    end
+    td, T, tv = -1, Float64[], r.target isa Number ? Float64(r.target) : 0.0
+    if r.target isa LinearTarget
+        td = dim_code(r.target)
+        T = Float64[r.target(node(td, ξ)..., 0) for ξ in forcing_nodes(grid, loc, td, "target")]
+    end
+    return md, Float64(r.rate), M, td, tv, T
+end
+relaxation_tables(f, grid, loc) =
+    throw(ArgumentError("B200(): only Relaxation(; rate::Number, mask = onefunction | GaussianMask, target = Number | " *
+                        "zerofunction | LinearTarget) forcings cross the C ABI; got $(typeof(f))"))
+
+function forcing_desc(forcing, grid, names)
+    for n in keys(forcing)
+        n in names || throw(ArgumentError("forcing name $n is not one of the model's fields $names"))   # model_forcing.jl
+    end
+    locs = (u = (Face, Center, Center), v = (Center, Face, Center), w = (Center, Center, Face))
+    keep = Vector{Float64}[]
+    none = ForcingDesc(0, -1, 0.0, C_NULL, -1, 0.0, C_NULL)
+    descs = ntuple(3 + MAX_TRACERS) do q
+        q <= length(names) && haskey(forcing, names[q]) || return none
+        n = names[q]
+        md, rate, M, td, tv, T = relaxation_tables(forcing[n], grid, haskey(locs, n) ? locs[n] : (Center, Center, Center))
+        push!(keep, M, T)
+        ForcingDesc(1, md, rate, isempty(M) ? C_NULL : pointer(M), td, tv, isempty(T) ? C_NULL : pointer(T))
+    end
+    return descs, keep
+end
+
 "Translate the model configuration into ob200_model_desc; everything outside the supported set is an ArgumentError."
 function model_desc(grid, gh; advection, buoyancy, coriolis, closure, tracers, timestepper, boundary_conditions, χ = 0.1,
                     stokes_drift = nothing, forcing = NamedTuple(), background_fields = NamedTuple(), particles = nothing,
                     immersed_boundary = nothing)
-    isnothing(stokes_drift) && isempty(forcing) && isempty(background_fields) && isnothing(particles) &&
-        isnothing(immersed_boundary) ||
-        throw(ArgumentError("B200(): stokes_drift, forcing, background_fields, particles and immersed boundaries are not supported"))
+    isnothing(stokes_drift) && isempty(background_fields) && isnothing(particles) && isnothing(immersed_boundary) ||
+        throw(ArgumentError("B200(): stokes_drift, background_fields, particles and immersed boundaries are not supported"))
     length(tracers) <= MAX_TRACERS || throw(ArgumentError("B200(): at most $MAX_TRACERS tracers"))
     ts = timestepper === :RungeKutta3 ? 1 : timestepper === :QuasiAdamsBashforth2 ? 0 :
          throw(ArgumentError("B200(): timestepper must be :RungeKutta3 or :QuasiAdamsBashforth2"))
@@ -350,12 +404,14 @@ function model_desc(grid, gh; advection, buoyancy, coriolis, closure, tracers, t
         fidx, side = divrem(q - 1, 6)
         fidx < length(names) ? bc_codes(boundary_conditions[names[fidx + 1]])[side + 1] : BC(0, 0.0)
     end
+    frc, frc_tabs = forcing_desc(forcing, grid, names)
     ptr(v) = isempty(v) ? Ptr{Float64}(C_NULL) : pointer(v)
     desc = ModelDesc(gh, ts, χ, adv_code(advection), advection isa WENO5 ? Int32(advection.zweno) : Int32(1),
                      map(ptr, tabs), clo, ν, κ, fplane, f, btr, tilted, ĝ, length(tracers), bcs, 0,
                      bkind, iT, iS, grav, α, β, smagorinsky_desc(closure, tracers)..., amd_desc(closure, tracers)...,
-                     vertically_implicit(closure))
-    return desc, tabs           # `tabs` must be GC.@preserve'd across ob200_model_create (host pointers are borrowed)
+                     vertically_implicit(closure), frc)
+    # the tables must be GC.@preserve'd across ob200_model_create (host pointers are borrowed)
+    return desc, (tabs, frc_tabs)
 end
 
 model_field(mh, name) = (h = Ref{Ptr{Cvoid}}(); check(ccall((:ob200_model_field, lib), Int32,

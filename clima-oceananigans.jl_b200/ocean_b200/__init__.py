@@ -12,7 +12,7 @@ from .model import (Field, CenterField, XFaceField, YFaceField, ZFaceField, fill
                     UpwindBiasedFifthOrder, ScalarDiffusivity, SmagorinskyLilly, AnisotropicMinimumDissipation,
                     VerticalScalarDiffusivity,
                     HorizontalScalarDiffusivity, FPlane, BuoyancyTracer, Buoyancy, SeawaterBuoyancy,
-                    LinearEquationOfState, BoundaryCondition,
+                    LinearEquationOfState, BoundaryCondition, Relaxation, GaussianMask, LinearTarget,
                     FluxBoundaryCondition, ValueBoundaryCondition, GradientBoundaryCondition,
                     update_state, calculate_tendencies, set_model, time_step, sync)
 from .output_writers import FieldSlicer, fetch_output, horizontal_average, Checkpointer  # noqa: F401

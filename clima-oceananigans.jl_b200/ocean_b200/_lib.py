@@ -30,6 +30,11 @@ class BC(C.Structure):
     _fields_ = [("kind", C.c_int32), ("value", C.c_double)]
 
 
+class Forcing(C.Structure):
+    _fields_ = [("active", C.c_int32), ("mask_dim", C.c_int32), ("rate", C.c_double), ("mask", C.POINTER(C.c_double)),
+                ("target_dim", C.c_int32), ("target_value", C.c_double), ("target", C.POINTER(C.c_double))]
+
+
 class ModelDesc(C.Structure):
     _fields_ = [("grid", C.c_void_p), ("timestepper", C.c_int32), ("chi", C.c_double),
                 ("advection", C.c_int32), ("weno_zweno", C.c_int32),
@@ -44,7 +49,8 @@ class ModelDesc(C.Structure):
                 ("haline_contraction", C.c_double),
                 ("smagorinsky_C", C.c_double), ("smagorinsky_Cb", C.c_double), ("prandtl", C.c_double * MAX_TRACERS),
                 ("amd_Cnu", C.c_double), ("amd_Ckappa", C.c_double * MAX_TRACERS), ("amd_Cb", C.c_double),
-                ("amd_has_Cb", C.c_int32), ("closure_vertically_implicit", C.c_int32)]
+                ("amd_has_Cb", C.c_int32), ("closure_vertically_implicit", C.c_int32),
+                ("forcing", Forcing * (3 + MAX_TRACERS))]
 
 
 #: every symbol include/ocean_b200.h declares: name -> (restype, argtypes)

@@ -430,6 +430,88 @@ class Buoyancy:
         self.g = gravity_unit_vector
 
 
+# ---- forcing (src/Forcings/relaxation.jl) ------------------------------------------------------------
+_DIMS = {"x": 0, "y": 1, "z": 2}
+
+
+def _param(v):
+    """a parameter as Julia would hold it: a Python float is a Float64 (it promotes Float32 nodes), everything else as given"""
+    return np.float64(v) if isinstance(v, float) else v
+
+
+def _is_number(v):
+    return isinstance(v, (int, float, np.integer, np.floating)) and not isinstance(v, bool)
+
+
+class GaussianMask:
+    """GaussianMask{D}(center, width) (relaxation.jl): exp(-(ξ - center)² / (2 width²)) along dimension D = "x", "y" or "z"."""
+
+    def __init__(self, dim, center, width):
+        if dim not in _DIMS:
+            raise ValueError(f"GaussianMask dimension must be one of 'x', 'y', 'z', got {dim!r}")
+        if not (_is_number(center) and _is_number(width)):
+            raise ValueError("GaussianMask center and width must be numbers")
+        self.dim, self.center, self.width = dim, center, width
+
+    def __call__(self, xi):
+        c, w = _param(self.center), _param(self.width)
+        return np.exp(-(xi - c) ** 2 / (2 * w ** 2))
+
+
+class LinearTarget:
+    """LinearTarget{D}(intercept, gradient) (relaxation.jl): intercept + gradient ξ along dimension D, independent of time."""
+
+    def __init__(self, dim, intercept, gradient):
+        if dim not in _DIMS:
+            raise ValueError(f"LinearTarget dimension must be one of 'x', 'y', 'z', got {dim!r}")
+        if not (_is_number(intercept) and _is_number(gradient)):
+            raise ValueError("LinearTarget intercept and gradient must be numbers")
+        self.dim, self.intercept, self.gradient = dim, intercept, gradient
+
+    def __call__(self, xi):
+        return _param(self.intercept) + _param(self.gradient) * xi
+
+
+class Relaxation:
+    """Relaxation(; rate, mask=onefunction, target=zerofunction) (src/Forcings/relaxation.jl): the forcing
+    rate * mask(x, y, z) * (target(x, y, z, t) - ψ) of the field ψ it is given for.  mask: None (onefunction) or a
+    GaussianMask; target: None (zerofunction), a number or a LinearTarget."""
+
+    def __init__(self, rate, mask=None, target=None):
+        if not _is_number(rate):
+            raise ValueError(f"Relaxation rate must be a number, got {type(rate).__name__}")
+        if mask is not None and not isinstance(mask, GaussianMask):
+            raise ValueError("Relaxation mask must be None (onefunction) or a GaussianMask on the B200 architecture")
+        if target is not None and not (_is_number(target) or isinstance(target, LinearTarget)):
+            raise ValueError("Relaxation target must be None (zerofunction), a number or a LinearTarget on the B200 architecture")
+        self.rate, self.mask, self.target = rate, mask, target
+
+
+def relaxation_tables(relaxation, loc, grid):
+    """Host tables of a Relaxation for a field at `loc` of `grid` (anything with .topology and .nodes(loc), the interior nodes
+    broadcast-shaped): (mask_dim, M, target_dim, T) with M = rate * mask at the field's nodes along mask_dim (-1: M is the
+    number rate) and T = the target there (-1: the number target).  Evaluated as the reference evaluates the forcing at a point:
+    parameters and nodes in their promoted type, rate * mask first.  No library call."""
+    def nodes(d, what):
+        if grid.topology[d] == Flat:
+            raise ValueError(f"Relaxation {what} along the Flat dimension {'xyz'[d]}")
+        return np.asarray(grid.nodes(loc)[d]).ravel()
+    rate = _param(relaxation.rate)
+    m = relaxation.mask
+    if m is None:
+        md, M = -1, rate
+    else:
+        md = _DIMS[m.dim]
+        M = rate * m(nodes(md, "mask"))
+    t = relaxation.target
+    if isinstance(t, LinearTarget):
+        td = _DIMS[t.dim]
+        T = t(nodes(td, "target"))
+    else:
+        td, T = -1, (0 if t is None else _param(t))
+    return md, M, td, T
+
+
 class Clock:
     def __init__(self, model):
         self._m = model
@@ -451,15 +533,15 @@ class NonhydrostaticModel:
     """NonhydrostaticModel(; grid, advection, closure, coriolis, buoyancy, tracers, timestepper,
     boundary_conditions) (src/Models/NonhydrostaticModels/nonhydrostatic_model.jl:102-203).
     Defaults as in the reference: advection = CenteredSecondOrder(), timestepper =
-    :QuasiAdamsBashforth2.  Unsupported pieces (forcings, function BCs, immersed boundaries, background
-    fields, particles, closures other than ScalarDiffusivity / SmagorinskyLilly / AnisotropicMinimumDissipation)
-    raise ArgumentError-like ValueErrors."""
+    :QuasiAdamsBashforth2.  `forcing` = {field name: Relaxation(...)}.  Unsupported pieces (function-valued forcings,
+    function BCs, immersed boundaries, background fields, particles, closures other than ScalarDiffusivity /
+    SmagorinskyLilly / AnisotropicMinimumDissipation) raise ArgumentError-like ValueErrors."""
 
     def __init__(self, grid, advection="default", closure=None, coriolis=None, buoyancy=None, tracers=(),
                  timestepper="QuasiAdamsBashforth2", boundary_conditions=None, forcing=None,
                  background_fields=None, particles=None, immersed_boundary=None, stokes_drift=None,
                  pressure_solver=None, chi=0.1):
-        for name, v in (("forcing", forcing), ("background_fields", background_fields), ("particles", particles),
+        for name, v in (("background_fields", background_fields), ("particles", particles),
                         ("immersed_boundary", immersed_boundary), ("stokes_drift", stokes_drift)):
             if v:
                 raise ValueError(f"`{name}` is not supported on the B200 architecture (SURVEY.md 8(b))")
@@ -481,6 +563,21 @@ class NonhydrostaticModel:
             raise ValueError("too many tracers")
         if isinstance(advection, WENO5) and advection.FT != grid.FT:
             raise ValueError("WENO5 float type differs from the grid's; construct it as WENO5(grid.FT) or WENO5(grid=grid)")
+        names = ("u", "v", "w") + tracers
+        locs = [(Face, Center, Center), (Center, Face, Center), (Center, Center, Face)] + [(Center,) * 3] * len(tracers)
+        # model_forcing (Forcings/model_forcing.jl): every name must be a prognostic field; the tables come from the interior
+        # nodes, which halo inflation does not change
+        frc = {}
+        if forcing:
+            if not isinstance(forcing, dict):
+                raise ValueError("forcing must be a dict {field name: Relaxation(...)}")
+            for n, fr in forcing.items():
+                if n not in names:
+                    raise ValueError(f"{n} is not a prognostic field of the model; forcing names must be among {names}")
+                if not isinstance(fr, Relaxation):
+                    raise ValueError(f"the forcing of {n} is a {type(fr).__name__}: only Relaxation crosses the C ABI of the B200 "
+                                     "architecture (function-valued forcings are outside its supported set)")
+                frc[names.index(n)] = relaxation_tables(fr, locs[names.index(n)], grid)
         # halo inflation (nonhydrostatic_model.jl:140-148)
         H = list(grid.H)
         for term in (advection, closure):
@@ -542,13 +639,27 @@ class NonhydrostaticModel:
             d.g_hat[k] = float(g_hat[k])
         d.ntracers = len(tracers)
         bcs = boundary_conditions or {}
-        names = ("u", "v", "w") + tracers
-        locs = [(Face, Center, Center), (Center, Face, Center), (Center, Center, Face)] + [(Center,) * 3] * len(tracers)
         for q, (n, loc) in enumerate(zip(names, locs)):
             arr = _bc_array(grid, loc, bcs.get(n))
             for s in range(6):
                 d.bcs[q][s].kind, d.bcs[q][s].value = arr[s].kind, arr[s].value
         d.pressure_solver = L.SOLVER_AUTO if pressure_solver is None else pressure_solver
+        for q, (md, M, td, T) in frc.items():
+            F = d.forcing[q]
+            F.active, F.mask_dim, F.target_dim = 1, md, td
+            if md < 0:
+                F.rate = float(M)
+            else:
+                a = np.ascontiguousarray(M, dtype=np.float64)
+                self._keep.append(a)
+                F.mask = a.ctypes.data_as(C.POINTER(C.c_double))
+            if td < 0:
+                F.target_value = float(T)
+            else:
+                a = np.ascontiguousarray(T, dtype=np.float64)
+                self._keep.append(a)
+                F.target = a.ctypes.data_as(C.POINTER(C.c_double))
+        self.forcing = dict(forcing or {})
         h = C.c_void_p()
         check(lib.ob200_model_create(C.byref(d), C.byref(h)))
         self.handle = h

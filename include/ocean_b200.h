@@ -80,6 +80,21 @@ typedef struct { int32_t kind; double value; } ob200_bc;
 
 #define OB200_MAX_TRACERS 8
 
+/* Relaxation(; rate, mask, target) (Forcings/relaxation.jl) of one prognostic field, tabulated by the host at the field's
+ * own nodes: G += M[ξ_mask] * (T[ξ_target] - ψ), M = rate * mask, added last in the tendency sum as the reference's
+ * `forcings.ψ(i, j, k, grid, clock, model_fields)`.  A table along dimension d holds the values at the field's interior
+ * nodes along d, Julia index 1..n (n = N[d], + 1 for a Face location on a Bounded dimension); the library rounds them to
+ * the grid's float type.  A zero-initialised descriptor is "no forcing".  Function-valued forcings are rejected by the shim. */
+typedef struct {
+    int32_t active;                /* 0: no forcing                                                                    */
+    int32_t mask_dim;              /* -1: mask = onefunction (M = rate everywhere); 0/1/2: GaussianMask{:x/:y/:z}        */
+    double  rate;                  /* M where mask_dim = -1                                                            */
+    const double* mask;            /* rate * mask at the field's interior nodes along mask_dim                         */
+    int32_t target_dim;            /* -1: constant target (Number, zerofunction -> 0); 0/1/2: LinearTarget{:x/:y/:z}   */
+    double  target_value;          /* T where target_dim = -1                                                          */
+    const double* target;          /* target at the field's interior nodes along target_dim                            */
+} ob200_forcing;
+
 /* NonhydrostaticModel(; grid, advection, closure, coriolis, buoyancy, tracers, timestepper,
  * boundary_conditions) (Models/NonhydrostaticModels/nonhydrostatic_model.jl:102-203). */
 typedef struct {
@@ -124,6 +139,9 @@ typedef struct {
      * abstract_scalar_diffusivity_closure.jl:214-255): 1 = the z-derivative parts of the vertical fluxes are integrated
      * implicitly by a tridiagonal solve after every substep (ThreeDimensional / Vertical formulation, Bounded z only) */
     int32_t closure_vertically_implicit;
+    /* forcing = (u = Relaxation(...), ...) (nonhydrostatic_model.jl:102-203, Forcings/model_forcing.jl): per prognostic
+     * field u, v, w, tracers...; appended last so that every earlier member keeps its offset */
+    ob200_forcing forcing[3 + OB200_MAX_TRACERS];
 } ob200_model_desc;
 
 /* ---- library / device ----------------------------------------------------------------- */
