@@ -1110,8 +1110,7 @@ static void model_update_state_after_projection(ob200_model* m, bool fused, bool
 // latency-bound column walk that leaves most of the machine idle).  Returns true if it was started.
 template <class FT>
 static bool model_hydrostatic_async_begin(ob200_model* m) {
-    static const bool off = getenv("OB200_NO_STREAM_SPREAD") != nullptr;
-    if (off || !m->pHY) return false;
+    if (!m->pHY) return false;
     if (!m->hy_stream) {
         OB_CUDA(cudaStreamCreateWithFlags(&m->hy_stream, cudaStreamNonBlocking));
         OB_CUDA(cudaEventCreateWithFlags(&m->hy_fork, cudaEventDisableTiming));
@@ -1130,8 +1129,7 @@ static void model_hydrostatic_async_end(ob200_model* m) { OB_CUDA(cudaStreamWait
 // the fused path: every non-Flat dimension Periodic (not slab-decomposed) and regular, fast FFT solver
 template <class FT>
 static bool model_fused_periodic(ob200_model* m) {
-    static const bool off = getenv("OB200_NO_FUSED_HALOS") != nullptr;
-    return !off && periodic_wrap_supported<FT>(gridD<FT>(m->grid)) && poisson_has_fast<FT>(planOf<FT>(m->solver.get()));
+    return periodic_wrap_supported<FT>(gridD<FT>(m->grid)) && poisson_has_fast<FT>(planOf<FT>(m->solver.get()));
 }
 extern "C" int32_t ob200_model_update_state(ob200_model* m) {
     API_BEGIN
@@ -1149,11 +1147,10 @@ static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
     // The launches of the prognostic fields are independent (each reads the old state and writes its own G^n and
     // new-state buffer), so they go to side streams forked from the library stream: the tail of one launch (its last,
     // partly filled wave of blocks) overlaps the head of the next instead of leaving SMs idle four times per stage.
-    static const bool spread = getenv("OB200_NO_STREAM_SPREAD") == nullptr;
     cudaStream_t* side = m->side;
     cudaEvent_t& ev_fork = m->ev_fork;
     cudaEvent_t* ev_join = m->ev_join;
-    const bool fork = spread && m->use_fast && m->nf > 1;
+    const bool fork = m->use_fast && m->nf > 1;
     if (fork && !ev_fork) {
         OB_CUDA(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
         for (int q = 0; q < 3; ++q) {
@@ -1177,8 +1174,7 @@ static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
         }
         // a closure the fused kernel does not evaluate itself (LES closures; any closure on the triply periodic variant): its flux
         // divergence alone goes into G^n through the general shared-face kernel, and the fused kernel adds everything else
-        static const bool no_split = getenv("OB200_NO_CLOSURE_SPLIT") != nullptr;
-        if (fz::supported<FT>(P, m->nf) == 2 && !no_split && closure_only_supported<FT>(P)) {
+        if (fz::supported<FT>(P, m->nf) == 2 && closure_only_supported<FT>(P)) {
             model_halo_join(m);
             const int nfused = 3 + std::min(m->nf - 3, 1);
             const Substep<FT> none{SUB_NONE, FT(0), FT(0), FT(0)};

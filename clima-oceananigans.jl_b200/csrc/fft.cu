@@ -25,7 +25,6 @@
 #include <vector>
 #include <cmath>
 #include <algorithm>
-#include <cstdlib>
 
 namespace ob {
 
@@ -542,9 +541,9 @@ PoissonPlan<FT>* poisson_plan_create(const GridD<FT>& g, int kind, const double*
     using CT = typename Cx<FT>::T;
     auto* p = new PoissonPlan<FT>();
     p->kind = kind;
-    if (kind == 1 && ff::fast_poisson_supported<FT>(g) && getenv("OB200_NO_FAST_FFT") == nullptr)
+    if (kind == 1 && ff::fast_poisson_supported<FT>(g))
         p->fast = ff::fast_poisson_create<FT>(g);
-    if (kind == 2 && ff::fast_ft_supported<FT>(g) && getenv("OB200_NO_FAST_FFT") == nullptr && getenv("OB200_NO_FAST_FT") == nullptr) {
+    if (kind == 2 && ff::fast_ft_supported<FT>(g)) {
         // half-spectrum x / y passes + Thomas sweep on the half spectrum (fft_fast.cu); none of the general path's
         // full-spectrum arrays is needed
         int Nz = g.N[2];
@@ -572,13 +571,12 @@ PoissonPlan<FT>* poisson_plan_create(const GridD<FT>& g, int kind, const double*
         int n = g.N[d];
         p->N[d] = n; p->topo[d] = g.topo[d];
         bool pow2 = n >= 2 && (n & (n - 1)) == 0;
-        static const bool force_direct = getenv("OB200_DIRECT_TRANSFORMS") != nullptr;
         int M = 1;
         while (M < 2 * n - 1) M <<= 1;
         const bool blue_ok = n >= 2 && M <= 4096;
         int tk;
-        if (g.topo[d] == OB_BOUNDED) tk = force_direct ? TK_DCT : (pow2 ? TK_DCT_POW2 : (blue_ok ? TK_DCT_BLUE : TK_DCT));
-        else tk = pow2 ? TK_POW2 : (!force_direct && blue_ok ? TK_BLUE : TK_DFT);
+        if (g.topo[d] == OB_BOUNDED) tk = pow2 ? TK_DCT_POW2 : (blue_ok ? TK_DCT_BLUE : TK_DCT);
+        else tk = pow2 ? TK_POW2 : (blue_ok ? TK_BLUE : TK_DFT);
         p->tkind[d] = tk; p->log2n[d] = ilog2(n);
         const bool blue = tk == TK_BLUE || tk == TK_DCT_BLUE;
         if (blue) { p->M[d] = M; p->log2M[d] = ilog2(M); }
@@ -650,7 +648,7 @@ PoissonPlan<FT>* poisson_plan_create(const GridD<FT>& g, int kind, const double*
     }
     // (Periodic, Periodic, Bounded) on a regular grid: the half-spectrum x / y passes of fft_fast.cu around a z pass of this
     // file's line kernel (Makhoul DCT, eigenvalue divide, inverse DCT) applied to the half spectrum in place
-    if (kind == 1 && !p->fast && g.regular[2] && ff::fast_ft_supported<FT>(g) && getenv("OB200_NO_FAST_FFT") == nullptr &&
+    if (kind == 1 && !p->fast && g.regular[2] && ff::fast_ft_supported<FT>(g) &&
         (p->tkind[2] == TK_DCT_POW2 || p->tkind[2] == TK_DCT_BLUE)) {
         p->fast = ff::fast_poisson_create<FT>(g);
         ff::fast_poisson_set_zhook<FT>(p->fast, [p]() {
@@ -668,7 +666,7 @@ PoissonPlan<FT>* poisson_plan_create(const GridD<FT>& g, int kind, const double*
     }
     // Bounded y (channels): the same half-spectrum x passes, this file's DCT over the y lines of the half spectrum (forward and
     // backward pass), and for z the Periodic lines of fft_fast.cu, the DCT hook above's twin, or the Thomas sweep
-    if (!p->fast && ff::fast_bounded_y_supported<FT>(g) && getenv("OB200_NO_FAST_FFT") == nullptr && p->tkind[1] == TK_DCT_POW2 &&
+    if (!p->fast && ff::fast_bounded_y_supported<FT>(g) && p->tkind[1] == TK_DCT_POW2 &&
         ((kind == 1 && g.regular[2] && (g.topo[2] == OB_PERIODIC || p->tkind[2] == TK_DCT_POW2 || p->tkind[2] == TK_DCT_BLUE)) ||
          (kind == 2 && g.topo[2] == OB_BOUNDED))) {
         p->fast = ff::fast_poisson_create<FT>(g);
@@ -760,19 +758,16 @@ static void launch_lines(FftArgs<FT>& A, int mode, bool contiguous_lines) {
             : A.kind == TK_DCT_POW2 ? A.n / 2 + A.n : A.kind == TK_BLUE ? A.M / 2 + A.n : A.M / 2 + 2 * A.n;
     // lines per block: 8 adjacent lines = 128-byte runs of the strided passes; more lines per block mean fewer resident
     // blocks to cover the per-stage barriers (256^3, ms per solve: T = 16 2.83, 8 2.32, 4 2.37; 512 threads 2.39)
-    static const int t_env = getenv("OB200_LINES_T") ? atoi(getenv("OB200_LINES_T")) : 0;
-    static const int thr_env = getenv("OB200_LINES_THREADS") ? atoi(getenv("OB200_LINES_THREADS")) : 0;
-    int T = t_env > 0 ? t_env : 8;
+    int T = 8;
     while (T > 1 && ((size_t)nbuf * T * LS + ntw) * sizeof(CT) > 96 * 1024) T >>= 1;
     if (contiguous_lines) { int Tm = std::max(1, 4096 / A.n); T = std::min(T, Tm); }
     T = std::min(T, A.nA);
     A.T = T;
     size_t smem = ((size_t)nbuf * T * LS + ntw) * sizeof(CT);
     dim3 grd(cdiv(A.nA, T), A.nB);
-    int threads = thr_env > 0 ? thr_env : 256;
     auto launch = [&](auto kern) {
         OB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-        kern<<<grd, threads, smem, stream()>>>(A);
+        kern<<<grd, 256, smem, stream()>>>(A);
         OB_LAUNCH_CHECK();
     };
     if (smem > 200 * 1024) throw Error("transform line too long for shared memory");

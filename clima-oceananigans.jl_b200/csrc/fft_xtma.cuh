@@ -1,10 +1,10 @@
-// fft_xtma.cuh -- persistent, bulk-copy-pipelined x passes of the fast FFT Poisson solver (single GPU).
+// fft_xtma.cuh -- persistent, bulk-copy-pipelined backward x pass of the fast FFT Poisson solver (single GPU).
 // Included by fft_fast.cu after fft_tma.cuh (uses its mbarrier helpers and the radix engine of fft_fast.cu).
 //
-// A tile is T consecutive y rows of one level k.  In both directions the rows of a tile are CONTIGUOUS in memory
-// (half spectrum: T x NXP complex; fields: T padded rows of Sx reals), so a tile is staged with 1-D bulk copies
-// (`cp.async.bulk.shared::cluster.global`, SASS UBLKCP) that complete on an mbarrier.  A block is persistent and
-// keeps STAGES tiles in flight: while the threads transform tile i the copies of tiles i+1 .. i+STAGES-1 are running.
+// A tile is T consecutive y rows of one level k of the half spectrum.  They are CONTIGUOUS in memory (T x NXP complex),
+// so a tile is staged with 1-D bulk copies (`cp.async.bulk.shared::cluster.global`, SASS UBLKCP) that complete on an
+// mbarrier.  A block is persistent and keeps STAGES tiles in flight: while the threads transform tile i the copies of
+// tiles i+1 .. i+STAGES-1 are running.
 // The first x kernels loaded with ordinary instructions and sat at 24 % occupancy with long-scoreboard (global load
 // latency) as the dominant stall (ncu r1h: 156 us / 93 us for 537 MB / 268 MB of compulsory traffic).
 #pragma once
@@ -12,13 +12,15 @@
 namespace tx {
 using namespace tl;
 
+constexpr int STAGES = 3;      // tiles in flight per block
+
 __device__ __forceinline__ void bulk_load(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
 // ---- backward x: half spectrum -> real line, written into the haloed field (+ periodic x halos) -----------------
-template <class FT, int LOG2M, int STAGES>
+template <class FT, int LOG2M>
 __global__ void __launch_bounds__(256) x_c2r_tma_kernel(const __grid_constant__ XArgs<FT> A) {
     using CT = typename Cx<FT>::T;
     using P2 = typename Pair<FT>::T;
@@ -85,101 +87,6 @@ __global__ void __launch_bounds__(256) x_c2r_tma_kernel(const __grid_constant__ 
             if (i + 1 <= H) orow[i + 1 + Nx] = r.y;
         }
         __syncthreads();                      // work lines are rewritten by the next tile's tangle
-    }
-}
-
-// ---- forward x: divergence of the predictor velocities -> real line -> half spectrum ---------------------------
-// staged per tile: u rows, v rows + the next v row, w rows of level k and of level k+1 (index N+1 of a Periodic
-// dimension is fetched as index 1, so the velocities' halos need not be valid)
-template <class FT, int LOG2M, int STAGES>
-__global__ void __launch_bounds__(256) x_r2c_tma_kernel(const __grid_constant__ XArgs<FT> A) {
-    using CT = typename Cx<FT>::T;
-    using G = Geo<LOG2M>;
-    constexpr int M = 1 << LOG2M;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ __align__(8) unsigned long long full[STAGES];
-    const int T = A.T;
-    const int Sx = (int)A.st[1];                                         // padded row length (reals)
-    const unsigned row_bytes = (unsigned)Sx * sizeof(FT);
-    const int nrows = A.has_z ? 4 * T + 1 : 2 * T + 1;                   // u: T, v: T + 1, w(k): T, w(k+1): T
-    const size_t stage_stride = ((size_t)nrows * row_bytes + 127) / 128 * 128;
-    CT* s = reinterpret_cast<CT*>(smem_raw + STAGES * stage_stride);
-    CT* stw = s + T * G::LS;
-    for (int w = threadIdx.x; w < M; w += blockDim.x) stw[w] = A.twM[w];
-    const bool lead = threadIdx.x == 0;
-    if (lead) {
-        for (int q = 0; q < STAGES; ++q) mbar_init(&full[q], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    const int tiles_y = A.Ny / T, ntiles = tiles_y * A.Nz;
-    const int first = blockIdx.x, step = gridDim.x;
-    const int mine = first < ntiles ? (ntiles - first + step - 1) / step : 0;
-    auto issue = [&](int n) {
-        const int tile = first + n * step;
-        const int k = tile / tiles_y, j0 = (tile - k * tiles_y) * T;
-        unsigned long long* bar = &full[n % STAGES];
-        unsigned char* dst = smem_raw + (n % STAGES) * stage_stride;
-        mbar_expect_tx(bar, (unsigned)nrows * row_bytes);
-        // row (j, k) of a field starts at Julia index (0, j, k) minus the x offset of the layout: p0 + j st1 + k st2 + x0
-        const long long r0 = (j0 + 1) * A.st[1] + (k + 1) * A.st[2] + A.x0;
-        const int jn = j0 + T + 1;                                                       // next row (Julia), wrapped
-        const long long rn = (jn > A.Ny && A.wrap[1] ? jn - A.Ny : jn) * A.st[1] + (k + 1) * A.st[2] + A.x0;
-        bulk_load(dst, A.u + r0, T * row_bytes, bar);
-        bulk_load(dst + (size_t)T * row_bytes, A.v + r0, T * row_bytes, bar);
-        bulk_load(dst + (size_t)2 * T * row_bytes, A.v + rn, row_bytes, bar);
-        if (A.has_z) {
-            const int kn = k + 2;                                                        // next level (Julia), wrapped
-            const long long rz = (j0 + 1) * A.st[1] + (kn > A.Nz && A.wrap[2] ? kn - A.Nz : kn) * A.st[2] + A.x0;
-            bulk_load(dst + (size_t)(2 * T + 1) * row_bytes, A.w + r0, T * row_bytes, bar);
-            bulk_load(dst + (size_t)(3 * T + 1) * row_bytes, A.w + rz, T * row_bytes, bar);
-        }
-    };
-    if (lead) for (int n = 0; n < STAGES && n < mine; ++n) issue(n);
-
-    const int tpl = blockDim.x / T, t = threadIdx.x / tpl, l = threadIdx.x - t * tpl;
-    CT* const sl = s + t * G::LS;
-    const int Nx = A.Nx;
-    const FT inv_dt = FT(1) / A.dt;
-    const int xo = -(int)A.x0;                     // position of Julia index 0 inside a staged row
-    for (int n = 0; n < mine; ++n) {
-        const int slot = n % STAGES;
-        const int tile = first + n * step;
-        const int k = tile / tiles_y, j0 = (tile - k * tiles_y) * T;
-        mbar_wait(&full[slot], (n / STAGES) & 1);
-        const FT* st0 = reinterpret_cast<const FT*>(smem_raw + slot * stage_stride);
-        const FT* ur = st0 + (size_t)t * Sx + xo;                       // Julia-0 pointers of this thread's rows
-        const FT* va = st0 + (size_t)(T + t) * Sx + xo;
-        const FT* vb = st0 + (size_t)(T + t + 1) * Sx + xo;
-        const FT* wa = st0 + (size_t)(2 * T + 1 + t) * Sx + xo;
-        const FT* wb = st0 + (size_t)(3 * T + 1 + t) * Sx + xo;
-        // divᶜᶜᶜ on a regular grid: 1/V (Ax δx u + Ay δy v + Az δz w), then / Δt (solve_for_pressure.jl:15-18)
-        for (int m = l; m < M; m += tpl) {
-            const int i = 2 * m + 1;
-            const FT u0 = ur[i], u1 = ur[i + 1], u2 = ur[i + 2 == Nx + 1 && A.wrap[0] ? 1 : i + 2];
-            FT tx0 = A.ax * u1 - A.ax * u0, tx1 = A.ax * u2 - A.ax * u1;
-            FT ty0 = A.ay * vb[i] - A.ay * va[i], ty1 = A.ay * vb[i + 1] - A.ay * va[i + 1];
-            FT tz0 = FT(0), tz1 = FT(0);
-            if (A.has_z) { tz0 = A.az * wb[i] - A.az * wa[i]; tz1 = A.az * wb[i + 1] - A.az * wa[i + 1]; }
-            CT c;
-            c.x = (A.invV * ((tx0 + ty0) + tz0)) * inv_dt;
-            c.y = (A.invV * ((tx1 + ty1) + tz1)) * inv_dt;
-            sl[G::pos(m)] = c;
-        }
-        __syncthreads();
-        if (lead && n + STAGES < mine) issue(n + STAGES);
-        fft_fwd<LOG2M>(s, stw, T);
-        // untangle: X[k] = E[k] + w_N^k O[k], E = (Z[k] + conj Z[M-k]) / 2, O = (Z[k] - conj Z[M-k]) / (2i)
-        CT* out = A.spec + (long long)A.NXP * ((j0 + t) + (long long)A.Ny * k);
-        for (int kk = l; kk <= M; kk += tpl) {
-            CT a = sl[G::pos(A.kpos[kk & (M - 1)])];
-            CT b = sl[G::pos(A.kpos[(M - kk) & (M - 1)])];
-            CT E, O;
-            E.x = FT(0.5) * (a.x + b.x); E.y = FT(0.5) * (a.y - b.y);
-            O.x = FT(0.5) * (a.y + b.y); O.y = FT(-0.5) * (a.x - b.x);
-            out[kk] = cadd(E, cmul(O, A.twN[kk]));
-        }
-        __syncthreads();
     }
 }
 

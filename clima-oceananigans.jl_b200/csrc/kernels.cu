@@ -100,8 +100,6 @@ __global__ void __launch_bounds__(256) fill_halo_shell_kernel(GridD<FT> g, HaloB
 // `with_comm`: a FullyConnected dimension is allowed (the caller exchanges it first)
 template <class FT>
 static bool shell_fill_supported(const GridD<FT>& g, bool with_comm) {
-    static const bool off = getenv("OB200_NO_SHELL_FILL") != nullptr;
-    if (off) return false;
     bool any = false;
     for (int d = 0; d < 3; ++d) {
         if (g.topo[d] == OB_FLAT) continue;
@@ -516,7 +514,7 @@ __global__ void __launch_bounds__(256, (CO ? 4 : 3)) tendency_shared_kernel(cons
 
 template <class FT>
 bool closure_only_supported(const Phys<FT>& P) {
-    if (getenv("OB200_NO_SHARED_GENERAL") != nullptr || P.closure == CLO_NONE) return false;
+    if (P.closure == CLO_NONE) return false;
     for (int d = 0; d < 3; ++d) if (P.g.topo[d] == OB_FLAT || P.g.N[d] < 2) return false;
     return true;
 }
@@ -533,12 +531,10 @@ void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], 
     A.ss = ss; A.fbc = fbc; A.comp = comp; A.closure_only = closure_only ? 1 : 0;
     // shared-face variant: 3-D grids (every direction has two faces to pair) with a halo wide enough for the one
     // extra face position per direction
-    static const bool no_shared = getenv("OB200_NO_SHARED_GENERAL") != nullptr;
-    bool shared = !no_shared && (P.scheme != ADV_NONE || P.closure != CLO_NONE);
+    bool shared = P.scheme != ADV_NONE || P.closure != CLO_NONE;
     for (int d = 0; d < 3; ++d) shared = shared && P.g.topo[d] != OB_FLAT && P.g.N[d] >= 2;
     if (closure_only && !shared) throw Error("closure-only tendencies need the shared-face kernel (3-D grid)");
-    static const bool no_spec = getenv("OB200_NO_SPEC_GENERAL") != nullptr;
-    const bool spec = !no_spec && P.g.topo[0] == OB_PERIODIC && P.g.topo[1] == OB_PERIODIC && P.g.topo[2] == OB_BOUNDED &&
+    const bool spec = P.g.topo[0] == OB_PERIODIC && P.g.topo[1] == OB_PERIODIC && P.g.topo[2] == OB_BOUNDED &&
                       P.g.regular[0] && P.g.regular[1] && P.scheme == ADV_WENO5 && P.buffer == 2 && !P.tilted && !P.vitd &&
                       !P.wc[0][0] && !P.wc[0][1] && !P.wc[1][0] && !P.wc[1][1];
     if (shared) {
@@ -719,10 +715,9 @@ template bool periodic_wrap_supported<double>(const GridD<double>&);
 template <class FT>
 void launch_pressure_correct(const GridD<FT>& g, FT* u, FT* v, FT* w, const FT* p, FT dt, bool periodic_wrap) {
     dim3 blk(64, 4, 1), grd(cdiv(g.N[0], 64), cdiv(g.N[1], 4), g.N[2]);
-    static const bool no_v2 = getenv("OB200_NO_PC_V2") != nullptr;
     // v2: two cells x two levels per thread.  With valid halos of p (not periodic_wrap) it serves every 3-D grid with regular
     // x, y and even Nx, Nz: Periodic dimensions are read with wrap-around (the same values), the others from their halos
-    bool v2 = !no_v2 && g.N[0] % 2 == 0 && g.N[2] % 2 == 0 && g.regular[0] && g.regular[1] && (periodic_wrap || g.regular[2] || g.dF[2]);
+    bool v2 = g.N[0] % 2 == 0 && g.N[2] % 2 == 0 && g.regular[0] && g.regular[1] && (periodic_wrap || g.regular[2] || g.dF[2]);
     for (int d = 0; d < 3; ++d) v2 = v2 && g.topo[d] != OB_FLAT;      // 3-D only: all three corrections active
     if (v2) {
         dim3 b2(32, 4, 1), g2(cdiv(g.N[0] / 2, 32), cdiv(g.N[1], 4), g.N[2] / 2);

@@ -18,7 +18,6 @@
 // Parity with the oracle stays <= 1e-12 per step (tests/test_gpu_parity.py).
 #include "internal.h"
 #include "weno_fast.cuh"
-#include <cstdlib>
 
 namespace ob {
 
@@ -189,7 +188,7 @@ bool launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], con
         if (g.topo[d] != OB_FLAT && g.H[d] < 3) return false;
     }
     if (g.N[0] % fast::TX || g.N[1] % (fast::ROWS * fast::TY)) return false;
-    if (hasz && getenv("OB200_NO_TMA") == nullptr && tma::launch<FT>(P, comp, U, psi, pHY, Gn, Gm, psi_new, ss)) return true;
+    if (hasz && tma::launch<FT>(P, comp, U, psi, pHY, Gn, Gm, psi_new, ss)) return true;
     fast::Ctx<FT> c;
     for (int d = 0; d < 3; ++d) { c.U[d] = U[d]; c.s[d] = g.st[d]; c.N[d] = g.N[d]; c.invd[d] = 1 / g.d[d]; }
     c.psi = psi; c.pHY = pHY; c.Gm = Gm; c.Gn = Gn; c.psi_new = psi_new; c.ss = ss;

@@ -38,7 +38,6 @@
 #include "weno_fast.cuh"
 #include "tma_util.cuh"
 #include <algorithm>
-#include <cstdlib>
 #include <type_traits>
 
 namespace ob {
@@ -633,9 +632,7 @@ static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part
     }
     const long long T = (long long)c.ntiles * c.Nz;
     if (T >= (1LL << 30)) throw Error("tendency_fused: grid too large for the 32-bit work decomposition");
-    static const int forced = getenv("OB200_FUSED_GRID") ? atoi(getenv("OB200_FUSED_GRID")) : 0;
-    int grid = forced > 0 ? forced : sms;
-    grid = (int)std::max(1LL, std::min((long long)grid, T / 8));
+    const int grid = (int)std::max(1LL, std::min((long long)sms, T / 8));
     c.chunk = cdiv((long long)(c.ntiles - (c.ntiles / grid) * grid) * c.Nz, grid);
     kern<<<grid, TX * (GR::NG * (R + 1) + 1), G_::SMEM, stream()>>>(c);
     OB_LAUNCH_CHECK();
@@ -693,10 +690,7 @@ static bool launch_frc(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
 template <class FT>
 static int classify(const Phys<FT>& P, int nf, bool& native) {
     const GridD<FT>& g = P.g;
-    static const bool off = getenv("OB200_NO_FUSED_TENDENCY") != nullptr;
-    static const bool offb = getenv("OB200_NO_FUSED_BOUNDED") != nullptr;
     native = false;
-    if (off) return -1;
     if (P.scheme != ADV_WENO5 || P.tilted || P.vitd) return -1;
     if (g.topo[0] != OB_PERIODIC || (g.topo[1] != OB_PERIODIC && g.topo[1] != OB_COMM)) return -1;
     for (int d = 0; d < 3; ++d)
@@ -712,7 +706,7 @@ static int classify(const Phys<FT>& P, int nf, bool& native) {
         return 0;
     }
     if (g.topo[2] == OB_BOUNDED) {
-        if (offb || nt == 0 || !g.izC || !g.izF || !P.wzp[0] || !P.wzp[1] || g.N[2] < 6) return -1;
+        if (nt == 0 || !g.izC || !g.izF || !P.wzp[0] || !P.wzp[1] || g.N[2] < 6) return -1;
         if (!g.regular[2] && (!P.wc[2][0] || !P.wc[2][1])) return -1;      // stretched z without coefficient tables
         native = P.closure == CLO_NONE || P.closure == CLO_3D;
         return 1;

@@ -23,7 +23,6 @@
 #include "tma_util.cuh"
 #include <cuda.h>
 #include <cmath>
-#include <algorithm>
 #include <map>
 #include <mutex>
 #include <tuple>
@@ -95,8 +94,8 @@ size_t cached_maps() {
 namespace ob {
 namespace tma {
 
-constexpr int TX = 32, HALO = 3, COL0 = HALO + 1;
-template <class FT, int NW> struct Box {
+constexpr int TX = 32, NW = 8, HALO = 3, COL0 = HALO + 1;   // NW warps per block
+template <class FT> struct Box {
     // The box must START on a 16-byte boundary in x (measured on B200: an odd FP64 start coordinate raises
     // "illegal instruction", tools/tma_probe4.cu), so it starts one column left of the halo: 1 + 3 + 32 + 3 + 1.
     static constexpr int R = NW - 1;                 // rows of cells
@@ -146,42 +145,42 @@ template <int D> __device__ __forceinline__ P3 shp(P3 q, int n) {
     return q;
 }
 
-template <class FT, int B, int NW>
+template <class FT, int B>
 struct Rings {
     const FT* psi;
     const FT* aux[3];
     __device__ __forceinline__ FT P(P3 q) const {
-        return psi[((q.L + 8) & (PSI_SL - 1)) * Box<FT, NW>::PE + q.row * Box<FT, NW>::BX + q.col];
+        return psi[((q.L + 8) & (PSI_SL - 1)) * Box<FT>::PE + q.row * Box<FT>::BX + q.col];
     }
     template <int COMP> __device__ __forceinline__ FT V(P3 q) const {
         if constexpr (COMP == B) return P(q);
         else {
             constexpr int a = Cfg<B>::comp(0) == COMP ? 0 : (Cfg<B>::comp(1) == COMP ? 1 : 2);
-            return aux[a][((q.L + 60) % Cfg<B>::sl(a)) * Box<FT, NW>::PE + q.row * Box<FT, NW>::BX + q.col];
+            return aux[a][((q.L + 60) % Cfg<B>::sl(a)) * Box<FT>::PE + q.row * Box<FT>::BX + q.col];
         }
     }
 };
 
 // (I(q) + I(q + 1))/2 along direction D of velocity component COMP (see wf::interp4)
-template <class FT, int B, int NW, int COMP, int D>
-__device__ __forceinline__ FT I4r(const Rings<FT, B, NW>& r, P3 q) {
+template <class FT, int B, int COMP, int D>
+__device__ __forceinline__ FT I4r(const Rings<FT, B>& r, P3 q) {
     return wf::interp4<FT>(r.template V<COMP>(shp<D>(q, -1)), r.template V<COMP>(q), r.template V<COMP>(shp<D>(q, 1)),
                            r.template V<COMP>(shp<D>(q, 2)));
 }
 
 // area * upwind flux of psi (component B or tracer) in direction A at position q
 // (A == B: cell-centre index; otherwise face index along A)
-template <class FT, bool ZW, int A, int B, int NW>
-__device__ __forceinline__ FT flux_at(const Rings<FT, B, NW>& r, const Ctx<FT>& c, P3 q) {
+template <class FT, bool ZW, int A, int B>
+__device__ __forceinline__ FT flux_at(const Rings<FT, B>& r, const Ctx<FT>& c, P3 q) {
     FT ut;
     P3 pf = q;
     if constexpr (B == 3) {
         ut = r.template V<A>(q);
     } else if constexpr (A == B) {
-        ut = I4r<FT, B, NW, A, A>(r, q);
+        ut = I4r<FT, B, A, A>(r, q);
         pf = shp<A>(q, 1);
     } else {
-        ut = I4r<FT, B, NW, A, B>(r, shp<B>(q, -1));
+        ut = I4r<FT, B, A, B>(r, shp<B>(q, -1));
     }
     const FT w0 = r.P(shp<A>(pf, -3)), w1 = r.P(shp<A>(pf, -2)), w2 = r.P(shp<A>(pf, -1)), w3 = r.P(pf),
              w4 = r.P(shp<A>(pf, 1)), w5 = r.P(shp<A>(pf, 2));
@@ -189,9 +188,9 @@ __device__ __forceinline__ FT flux_at(const Rings<FT, B, NW>& r, const Ctx<FT>& 
     return c.area[A] * (ut * rec);
 }
 
-template <class FT, bool ZW, int B, int NW>
-__global__ void __launch_bounds__(TX* NW, NW <= 8 ? 3 : 2) tendency_tma_kernel(const __grid_constant__ Ctx<FT> c) {
-    using BXs = Box<FT, NW>;
+template <class FT, bool ZW, int B>
+__global__ void __launch_bounds__(TX * NW, 3) tendency_tma_kernel(const __grid_constant__ Ctx<FT> c) {
+    using BXs = Box<FT>;
     using CF = Cfg<B>;
     constexpr int R = BXs::R;
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -238,7 +237,7 @@ __global__ void __launch_bounds__(TX* NW, NW <= 8 ? 3 : 2) tendency_tma_kernel(c
             for (int L = k0 + CF::lo(a); L <= k0 + CF::hi(a); ++L) load_aux(a, L, &bars[0]);
     }
 
-    Rings<FT, B, NW> Rg;
+    Rings<FT, B> Rg;
     Rg.psi = ring_psi;
     Rg.aux[0] = ring_aux[0]; Rg.aux[1] = ring_aux[1]; Rg.aux[2] = ring_aux[2];
 
@@ -271,21 +270,21 @@ __global__ void __launch_bounds__(TX* NW, NW <= 8 ? 3 : 2) tendency_tma_kernel(c
         const P3 q{k, ty + HALO, tx + COL0};
         FT Fx = FT(0), Fy = FT(0), dFz = FT(0);
         if (cell) {
-            if (it == 0) Fz_carry = flux_at<FT, ZW, 2, B, NW>(Rg, c, ZLOW ? shp<2>(q, -1) : q);
-            Fx = flux_at<FT, ZW, 0, B, NW>(Rg, c, q);
-            Fy = flux_at<FT, ZW, 1, B, NW>(Rg, c, q);
+            if (it == 0) Fz_carry = flux_at<FT, ZW, 2, B>(Rg, c, ZLOW ? shp<2>(q, -1) : q);
+            Fx = flux_at<FT, ZW, 0, B>(Rg, c, q);
+            Fy = flux_at<FT, ZW, 1, B>(Rg, c, q);
             sFx[buf][ty][XLOW ? tx + 1 : tx] = Fx;
             sFy[buf][YLOW ? ty + 1 : ty][tx] = Fy;
-            FT Fz_new = flux_at<FT, ZW, 2, B, NW>(Rg, c, ZLOW ? q : shp<2>(q, 1));
+            FT Fz_new = flux_at<FT, ZW, 2, B>(Rg, c, ZLOW ? q : shp<2>(q, 1));
             dFz = Fz_new - Fz_carry;
             Fz_carry = Fz_new;
         } else if (edge) {
             if (tx < nrows) {
                 P3 e{k, tx + HALO, (XLOW ? -1 : TX) + COL0};
-                sFx[buf][tx][XLOW ? 0 : TX] = flux_at<FT, ZW, 0, B, NW>(Rg, c, e);
+                sFx[buf][tx][XLOW ? 0 : TX] = flux_at<FT, ZW, 0, B>(Rg, c, e);
             }
             P3 e{k, (YLOW ? -1 : nrows) + HALO, tx + COL0};
-            sFy[buf][YLOW ? 0 : nrows][tx] = flux_at<FT, ZW, 1, B, NW>(Rg, c, e);
+            sFy[buf][YLOW ? 0 : nrows][tx] = flux_at<FT, ZW, 1, B>(Rg, c, e);
         }
         __syncthreads();
         if (cell) {
@@ -320,10 +319,10 @@ __global__ void __launch_bounds__(TX* NW, NW <= 8 ? 3 : 2) tendency_tma_kernel(c
 // ---- host side --------------------------------------------------------------------------------
 using tmau::make_map;
 
-template <class FT, bool ZW, int B, int NW>
+template <class FT, bool ZW, int B>
 static void launch_one(Ctx<FT>& c, const GridD<FT>& g, const FT* const U[3], const FT* psi) {
     using CF = Cfg<B>;
-    using BXs = Box<FT, NW>;
+    using BXs = Box<FT>;
     c.tm_psi = make_map<FT>(g, psi - g.off0, BXs::BX, BXs::BY);
     int slots = PSI_SL;
     for (int a = 0; a < CF::NA; ++a) {
@@ -331,7 +330,7 @@ static void launch_one(Ctx<FT>& c, const GridD<FT>& g, const FT* const U[3], con
         c.tm_aux[a] = make_map<FT>(g, U[CF::comp(a)] - g.off0, BXs::BX, BXs::BY);
     }
     size_t smem = (size_t)slots * BXs::PLANE_BYTES;
-    auto kern = tendency_tma_kernel<FT, ZW, B, NW>;
+    auto kern = tendency_tma_kernel<FT, ZW, B>;
     static bool attr_set = false;      // one flag per kernel instantiation (function-local static of a template)
     if (!attr_set) {
         OB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
@@ -339,23 +338,11 @@ static void launch_one(Ctx<FT>& c, const GridD<FT>& g, const FT* const U[3], con
     }
     // chunks of 32 levels in z (the last one may be shorter).  A wave-quantisation model (blocks as a multiple of the
     // resident block count, prologue of ~2 levels per chunk) picked 6 chunks at 256^3 and measured SLOWER than 8
-    // (3.82 vs 3.74 ms per step), so the plain rule stays; OB200_TMA_NCHUNK overrides it.
-    static const int forced = getenv("OB200_TMA_NCHUNK") ? atoi(getenv("OB200_TMA_NCHUNK")) : 0;
-    const int nchunks = forced > 0 ? std::min(forced, g.N[2]) : cdiv(g.N[2], 32);
-    c.Kc = cdiv(g.N[2], nchunks);
+    // (3.82 vs 3.74 ms per step), so the plain rule stays.
+    c.Kc = cdiv(g.N[2], cdiv(g.N[2], 32));
     dim3 blk(TX, NW), grd(g.N[0] / TX, cdiv(g.N[1], BXs::R), cdiv(g.N[2], c.Kc));
     kern<<<grd, blk, smem, stream()>>>(c);
     OB_LAUNCH_CHECK();
-}
-
-static int warps_per_block() {
-    static int nw = 0;
-    if (!nw) {
-        const char* e = getenv("OB200_TMA_NW");
-        nw = e ? atoi(e) : 8;
-        if (nw != 8 && nw != 12) nw = 8;
-    }
-    return nw;
 }
 
 template <class FT>
@@ -374,15 +361,14 @@ bool launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, co
     c.f = P.f; c.fplane = P.fplane;
     c.Ny = g.N[1]; c.Nz = g.N[2];
     c.Kc = g.N[2];
-#define GO(ZWV, NWV)                                                         \
-    switch (comp) {                                                          \
-        case 0: launch_one<FT, ZWV, 0, NWV>(c, g, U, psi); break;            \
-        case 1: launch_one<FT, ZWV, 1, NWV>(c, g, U, psi); break;            \
-        case 2: launch_one<FT, ZWV, 2, NWV>(c, g, U, psi); break;            \
-        default: launch_one<FT, ZWV, 3, NWV>(c, g, U, psi); break;           \
+#define GO(ZWV)                                                         \
+    switch (comp) {                                                     \
+        case 0: launch_one<FT, ZWV, 0>(c, g, U, psi); break;            \
+        case 1: launch_one<FT, ZWV, 1>(c, g, U, psi); break;            \
+        case 2: launch_one<FT, ZWV, 2>(c, g, U, psi); break;            \
+        default: launch_one<FT, ZWV, 3>(c, g, U, psi); break;           \
     }
-    if (warps_per_block() == 8) { if (P.zweno) { GO(true, 8) } else { GO(false, 8) } }
-    else { if (P.zweno) { GO(true, 12) } else { GO(false, 12) } }
+    if (P.zweno) { GO(true) } else { GO(false) }
 #undef GO
     return true;
 }

@@ -7,7 +7,7 @@
   ft   FourierTridiagonalPoissonSolver, (Periodic, Periodic, Bounded) with the vertical stretching of the ocean
        wind-mixing / convection example (examples/ocean_wind_mixing_and_convection.jl:41-54)
   topo FFTBasedPoissonSolver on a regular grid for all eight (Periodic | Bounded)^3 topologies (Bounded = DCT by Makhoul's
-       algorithm; a non-power-of-two N runs Bluestein's); OB200_DIRECT_TRANSFORMS=1 times the O(n^2) transforms instead
+       algorithm; a non-power-of-two N runs Bluestein's)
   cpu  the CPU stand-in of SURVEY.md 8(d)(iii): the same triply periodic solve with scipy.fft (pocketfft, all host
        threads) -- rfftn, eigenvalue divide, irfftn -- timed on the box's host cores (bounded: N <= 256)
 
@@ -122,8 +122,7 @@ def main():
                        (w[I, I, H + 1:N + H + 1] - w[I, I, I])) / d_
                 res = float(np.max(np.abs(lap - div)) / np.max(np.abs(div)))
                 out.append({"solver": "FFTBasedPoissonSolver", "topology": "".join(topo), "N": N, "ms_per_solve": ms,
-                            "points_per_s": N ** 3 / (ms * 1e-3), "residual": res,
-                            "transforms": "direct O(n^2)" if os.environ.get("OB200_DIRECT_TRANSFORMS") else "fast"})
+                            "points_per_s": N ** 3 / (ms * 1e-3), "residual": res})
                 del s, phi, U, g
         print(json.dumps(out))
         return
