@@ -19,43 +19,7 @@
 
 namespace tl {
 
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned long long* bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-    unsigned ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* tm, int x, int y, int z, unsigned long long* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-        ::"r"(smem_u32(dst)), "l"(tm), "r"(x), "r"(y), "r"(z), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* tm, int x, int y, int z, int w, unsigned long long* bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
-        ::"r"(smem_u32(dst)), "l"(tm), "r"(x), "r"(y), "r"(z), "r"(w), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* tm, int x, int y, int z, const void* src) {
-    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%1, %2, %3}], [%4];"
-                 ::"l"(tm), "r"(x), "r"(y), "r"(z), "r"(smem_u32(src)) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void bulk_wait_read() {
-    asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
-}
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+using namespace tmau;     // tma_util.cuh
 
 // addressing of a tile (which tensor maps, which coordinates):
 //   ADDR_NAT  in place on the natural half spectrum [Nz][Ny][NXP] (single GPU)
@@ -155,7 +119,7 @@ __global__ void __launch_bounds__(256) line_tma_kernel(const __grid_constant__ T
     const bool lead = threadIdx.x == 0;
     if (lead) {
         for (int q = 0; q < STAGES; ++q) mbar_init(&full[q], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     __syncthreads();
 

@@ -1,5 +1,5 @@
 // fft_xtma.cuh -- persistent, bulk-copy-pipelined backward x pass of the fast FFT Poisson solver (single GPU).
-// Included by fft_fast.cu after fft_tma.cuh (uses its mbarrier helpers and the radix engine of fft_fast.cu).
+// Included by fft_fast.cu (uses its radix engine).
 //
 // A tile is T consecutive y rows of one level k of the half spectrum.  They are CONTIGUOUS in memory (T x NXP complex),
 // so a tile is staged with 1-D bulk copies (`cp.async.bulk.shared::cluster.global`, SASS UBLKCP) that complete on an
@@ -10,14 +10,9 @@
 #pragma once
 
 namespace tx {
-using namespace tl;
+using namespace tmau;     // tma_util.cuh
 
 constexpr int STAGES = 3;      // tiles in flight per block
-
-__device__ __forceinline__ void bulk_load(void* dst, const void* src, unsigned bytes, unsigned long long* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
 
 // ---- backward x: half spectrum -> real line, written into the haloed field (+ periodic x halos) -----------------
 template <class FT, int LOG2M>
@@ -37,7 +32,7 @@ __global__ void __launch_bounds__(256) x_c2r_tma_kernel(const __grid_constant__ 
     const bool lead = threadIdx.x == 0;
     if (lead) {
         for (int q = 0; q < STAGES; ++q) mbar_init(&full[q], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     __syncthreads();
     const int tiles_y = A.Ny / T, ntiles = tiles_y * A.Nz;          // Ny is a multiple of T (checked on the host)

@@ -48,14 +48,15 @@ void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], 
                              const FT* Gm, FT* psi_new, const Substep<FT>& ss, bool closure_only = false);
 // true if launch_tendency_general(..., closure_only = true) is available for this model (3-D grid)
 template <class FT> bool closure_only_supported(const Phys<FT>& P);
-// fast path (triply periodic, regular, WENO5 uniform, no closure/coriolis); returns false if
-// the configuration is not covered
+// fast path (all non-Flat dimensions periodic, regular, WENO5 uniform, no closure, optional FPlane, field not forced):
+// the TMA-staged kernel on 3-D grids, the direct-load kernel on 2-D grids; returns false if the configuration is not
+// covered
 template <class FT>
 bool launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
                           const FT* pHY, FT* Gn, const FT* Gm, FT* psi_new, const Substep<FT>& ss);
 
 // tendency_fused.cu: all prognostic fields of the specialised configuration in ONE launch.  Returns how many leading
-// fields (u, v, w, first tracers) it handled: 0 if the configuration is not covered, otherwise 3 + min(ntracers, 2);
+// fields (u, v, w, first tracer) it handled: 0 if the configuration is not covered, otherwise 3 + min(ntracers, 1);
 // the caller steps the remaining tracers with the per-field kernels.
 constexpr int FUSED_MAXF = 5;
 template <class FT>

@@ -1,11 +1,12 @@
-// tendency_fast.cu -- specialised tendency (+ fused RK3/AB2 substep) kernels for the headline
+// tendency_fast.cu -- specialised tendency (+ fused RK3/AB2 substep) kernel for the headline
 // configuration: every non-Flat dimension Periodic, regular spacing, WENO5 with uniform
 // coefficients (Z or JS weights), closure = nothing, optional FPlane and hydrostatic pressure.
+// launch_tendency_fast sends 3-D grids to the TMA-staged kernel (tendency_tma.cu); the kernel here
+// runs the 2-D grids (z Flat).
 //
 // Same quantities as physics.cuh (reference files cited there), reorganised for the FP64 pipe,
 // which is what bounds this kernel on B200 (about 20-30 flop per byte of compulsory traffic):
-//   * every face flux is evaluated ONCE and shared: z faces are carried in registers while a
-//     thread marches up its column, x / y faces go through shared memory; the one extra column
+//   * every face flux is evaluated ONCE and shared through shared memory; the one extra column
 //     and row of faces a 32x8 tile needs are computed by two otherwise idle warps
 //     (the reference evaluates every face twice, momentum_advection_operators.jl:52-56);
 //   * only the UPWIND-side WENO reconstruction is evaluated: ((u+|u|) L + (u-|u|) R)/2 is exactly
@@ -23,31 +24,27 @@ namespace ob {
 
 namespace tma {   // tendency_tma.cu
 template <class FT>
-bool launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, const FT* pHY, FT* Gn, const FT* Gm,
+void launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, const FT* pHY, FT* Gn, const FT* Gm,
             FT* psi_new, const Substep<FT>& ss);
 }
 
 namespace fast {
 
-#ifndef OB_ROWS
-#define OB_ROWS 1
-#endif
-constexpr int TX = 32, TY = 8, ROWS = OB_ROWS;   // tile = TX x (ROWS*TY) cells, TX*TY threads
+constexpr int TX = 32, TY = 8;   // tile = TX x TY cells, one thread per cell
 
 template <class FT>
 struct Ctx {
-    const FT* U[3];
+    const FT* U[2];
     const FT* psi;
     const FT* pHY;
     const FT* Gm;
     FT* Gn;
     FT* psi_new;
     long long s[3];
-    FT area[3], invV, invd[3];
+    FT area[2], invV, invd[2];
     FT f;
     int fplane;
-    int N[3];
-    int Kc;
+    int N[2];
     Substep<FT> ss;
 };
 
@@ -57,23 +54,21 @@ __device__ __forceinline__ FT I4f(const FT* c, long long p, long long s) {
     return wf::interp4<FT>(c[p - s], c[p], c[p + s], c[p + 2 * s]);
 }
 
-// area * upwind flux of psi (component B, or tracer B = 3) in direction A at position p
+// area * upwind flux of psi (component B, or tracer B = 3) in direction A (x or y) at position p
 // (A == B: cell-centre index; otherwise face index along A)
-template <class FT, bool ZW, bool HASZ, int A, int B>
+template <class FT, bool ZW, int A, int B>
 __device__ __forceinline__ FT flux_at(const Ctx<FT>& c, long long p) {
     const long long sA = c.s[A];
     FT ut;
     long long pf = p;
-    if (B == 3) {
+    if constexpr (B >= 2) {       // a tracer, or w, which is centred in the Flat z: U[A] is already at the face
         ut = c.U[A][p];
-    } else if (A == B) {
+    } else if constexpr (A == B) {
         ut = I4f<FT>(c.U[A], p, sA);
         pf = p + sA;
     } else {
-        constexpr int BB = B == 3 ? 0 : B;
-        const long long sB = c.s[BB];
-        if (!HASZ && BB == 2) ut = c.U[A][p];
-        else ut = I4f<FT>(c.U[A], p - sB, sB);
+        const long long sB = c.s[B];
+        ut = I4f<FT>(c.U[A], p - sB, sB);
     }
     // all six loads are issued independently of ut (no dependent second memory round trip);
     // the upwind window is then selected in registers
@@ -83,91 +78,61 @@ __device__ __forceinline__ FT flux_at(const Ctx<FT>& c, long long p) {
     return c.area[A] * (ut * rec);
 }
 
-template <class FT, bool ZW, bool HASZ, int B>
+template <class FT, bool ZW, int B>
 __global__ void __launch_bounds__(TX* TY, 2) tendency_fast_kernel(Ctx<FT> c) {
-    // tile = TX x (ROWS*TY) cells; thread (tx, ty) owns rows ty and ty + TY of the tile
-    __shared__ FT sFx[2][ROWS * TY][TX + 1];
-    __shared__ FT sFy[2][ROWS * TY + 1][TX];
+    __shared__ FT sFx[TY][TX + 1];
+    __shared__ FT sFy[TY + 1][TX];
     const int tx = threadIdx.x, ty = threadIdx.y, tid = ty * TX + tx;
-    const int i0 = 1 + blockIdx.x * TX, j0 = 1 + blockIdx.y * (ROWS * TY);
+    const int i0 = 1 + blockIdx.x * TX, j0 = 1 + blockIdx.y * TY;
     const int i = i0 + tx;
-    const int k0 = 1 + blockIdx.z * c.Kc;
     const long long sx = c.s[0], sy = c.s[1], sz = c.s[2];
-    // x: B == 0 needs F(i) - F(i-1) (extra column at i0-1), otherwise F(i+1) - F(i) (extra at i0+TX)
-    constexpr bool XLOW = (B == 0), YLOW = (B == 1), ZLOW = (B == 2);
-    long long p0 = i * sx + (j0 + ty) * sy + k0 * sz;
-    // extra faces: warp 0 lanes 0..ROWS*TY-1 -> x column ; warp 1 -> y row
-    const bool xextra = tid < ROWS * TY, yextra = tid >= 32 && tid < 32 + TX;
-    long long pxe = (XLOW ? (i0 - 1) : (i0 + TX)) * sx + (j0 + tid) * sy + k0 * sz;
-    long long pye = (i0 + (tid - 32)) * sx + (YLOW ? (j0 - 1) : (j0 + ROWS * TY)) * sy + k0 * sz;
+    // x: B == 0 needs F(i) - F(i-1) (extra column at i0-1), otherwise F(i+1) - F(i) (extra at i0+TX); y alike
+    constexpr bool XLOW = (B == 0), YLOW = (B == 1);
+    const long long p = i * sx + (j0 + ty) * sy + sz;       // the one level, k = 1
+    // extra faces: warp 0 lanes 0..TY-1 -> x column ; warp 1 -> y row
+    const bool xextra = tid < TY, yextra = tid >= 32 && tid < 32 + TX;
+    const long long pxe = (XLOW ? (i0 - 1) : (i0 + TX)) * sx + (j0 + tid) * sy + sz;
+    const long long pye = (i0 + (tid - 32)) * sx + (YLOW ? (j0 - 1) : (j0 + TY)) * sy + sz;
 
-    FT Fz_carry[ROWS];
-#pragma unroll
-    for (int r = 0; r < ROWS; ++r) {
-        long long p = p0 + r * TY * sy;
-        Fz_carry[r] = HASZ ? flux_at<FT, ZW, HASZ, 2, B>(c, ZLOW ? p - sz : p) : FT(0);
-    }
-
-    for (int kk = 0; kk < c.Kc; ++kk) {
-        const int buf = kk & 1;
-        FT Fx[ROWS], Fy[ROWS], dFz[ROWS];
-#pragma unroll
-        for (int r = 0; r < ROWS; ++r) {
-            long long p = p0 + r * TY * sy;
-            const int row = ty + r * TY;
-            Fx[r] = flux_at<FT, ZW, HASZ, 0, B>(c, p);
-            Fy[r] = flux_at<FT, ZW, HASZ, 1, B>(c, p);
-            sFx[buf][row][XLOW ? tx + 1 : tx] = Fx[r];
-            sFy[buf][YLOW ? row + 1 : row][tx] = Fy[r];
-            dFz[r] = FT(0);
-            if (HASZ) {
-                FT Fz_new = flux_at<FT, ZW, HASZ, 2, B>(c, ZLOW ? p : p + sz);
-                dFz[r] = Fz_new - Fz_carry[r];
-                Fz_carry[r] = Fz_new;
-            }
+    const FT Fx = flux_at<FT, ZW, 0, B>(c, p);
+    const FT Fy = flux_at<FT, ZW, 1, B>(c, p);
+    sFx[ty][XLOW ? tx + 1 : tx] = Fx;
+    sFy[YLOW ? ty + 1 : ty][tx] = Fy;
+    if (xextra) sFx[tid][XLOW ? 0 : TX] = flux_at<FT, ZW, 0, B>(c, pxe);
+    if (yextra) sFy[YLOW ? 0 : TY][tid - 32] = flux_at<FT, ZW, 1, B>(c, pye);
+    __syncthreads();
+    const FT dFx = XLOW ? (Fx - sFx[ty][tx]) : (sFx[ty][tx + 1] - Fx);
+    const FT dFy = YLOW ? (Fy - sFy[ty][tx]) : (sFy[ty + 1][tx] - Fy);
+    FT G = -(c.invV * (dFx + dFy));
+    if (B == 0) {
+        if (c.fplane) {      // - x_f_cross_U = + f * ℑxyᶠᶜᵃ(v)
+            const FT* v = c.U[1];
+            FT a0 = FT(0.5) * (v[p - sx] + v[p]), a1 = FT(0.5) * (v[p - sx + sy] + v[p + sy]);
+            G = G - (-c.f * (FT(0.5) * (a0 + a1)));
         }
-        if (xextra) sFx[buf][tid][XLOW ? 0 : TX] = flux_at<FT, ZW, HASZ, 0, B>(c, pxe);
-        if (yextra) sFy[buf][YLOW ? 0 : ROWS * TY][tid - 32] = flux_at<FT, ZW, HASZ, 1, B>(c, pye);
-        __syncthreads();
-#pragma unroll
-        for (int r = 0; r < ROWS; ++r) {
-            long long p = p0 + r * TY * sy;
-            const int row = ty + r * TY;
-            FT dFx = XLOW ? (Fx[r] - sFx[buf][row][tx]) : (sFx[buf][row][tx + 1] - Fx[r]);
-            FT dFy = YLOW ? (Fy[r] - sFy[buf][row][tx]) : (sFy[buf][row + 1][tx] - Fy[r]);
-            FT G = -(c.invV * ((dFx + dFy) + dFz[r]));
-            if (B == 0) {
-                if (c.fplane) {      // - x_f_cross_U = + f * ℑxyᶠᶜᵃ(v)
-                    const FT* v = c.U[1];
-                    FT a0 = FT(0.5) * (v[p - sx] + v[p]), a1 = FT(0.5) * (v[p - sx + sy] + v[p + sy]);
-                    G = G - (-c.f * (FT(0.5) * (a0 + a1)));
-                }
-                if (c.pHY) G = G - (c.pHY[p] - c.pHY[p - sx]) * c.invd[0];
-            } else if (B == 1) {
-                if (c.fplane) {      // - y_f_cross_U = - f * ℑxyᶜᶠᵃ(u)
-                    const FT* u = c.U[0];
-                    FT a0 = FT(0.5) * (u[p - sy] + u[p + sx - sy]), a1 = FT(0.5) * (u[p] + u[p + sx]);
-                    G = G - (c.f * (FT(0.5) * (a0 + a1)));
-                }
-                if (c.pHY) G = G - (c.pHY[p] - c.pHY[p - sy]) * c.invd[1];
-            }
-            c.Gn[p] = G;
-            if (c.ss.mode == SUB_RK3_FIRST) c.psi_new[p] = c.psi[p] + c.ss.c1 * G;
-            else if (c.ss.mode == SUB_RK3) c.psi_new[p] = c.psi[p] + c.ss.dt * (c.ss.c1 * G + c.ss.c2 * c.Gm[p]);
-            else if (c.ss.mode == SUB_AB2) c.psi_new[p] = c.psi[p] + c.ss.dt * (c.ss.c1 * G - c.ss.c2 * c.Gm[p]);
+        if (c.pHY) G = G - (c.pHY[p] - c.pHY[p - sx]) * c.invd[0];
+    } else if (B == 1) {
+        if (c.fplane) {      // - y_f_cross_U = - f * ℑxyᶜᶠᵃ(u)
+            const FT* u = c.U[0];
+            FT a0 = FT(0.5) * (u[p - sy] + u[p + sx - sy]), a1 = FT(0.5) * (u[p] + u[p + sx]);
+            G = G - (c.f * (FT(0.5) * (a0 + a1)));
         }
-        p0 += sz; pxe += sz; pye += sz;
+        if (c.pHY) G = G - (c.pHY[p] - c.pHY[p - sy]) * c.invd[1];
     }
+    c.Gn[p] = G;
+    if (c.ss.mode == SUB_RK3_FIRST) c.psi_new[p] = c.psi[p] + c.ss.c1 * G;
+    else if (c.ss.mode == SUB_RK3) c.psi_new[p] = c.psi[p] + c.ss.dt * (c.ss.c1 * G + c.ss.c2 * c.Gm[p]);
+    else if (c.ss.mode == SUB_AB2) c.psi_new[p] = c.psi[p] + c.ss.dt * (c.ss.c1 * G - c.ss.c2 * c.Gm[p]);
 }
 
-template <class FT, bool ZW, bool HASZ>
+template <class FT, bool ZW>
 void launch(const Ctx<FT>& c, int comp) {
-    dim3 blk(TX, TY), grd(c.N[0] / TX, c.N[1] / (ROWS * TY), HASZ ? c.N[2] / c.Kc : 1);
+    dim3 blk(TX, TY), grd(c.N[0] / TX, c.N[1] / TY);
     switch (comp) {
-        case 0: tendency_fast_kernel<FT, ZW, HASZ, 0><<<grd, blk, 0, stream()>>>(c); break;
-        case 1: tendency_fast_kernel<FT, ZW, HASZ, 1><<<grd, blk, 0, stream()>>>(c); break;
-        case 2: tendency_fast_kernel<FT, ZW, HASZ, 2><<<grd, blk, 0, stream()>>>(c); break;
-        default: tendency_fast_kernel<FT, ZW, HASZ, 3><<<grd, blk, 0, stream()>>>(c); break;
+        case 0: tendency_fast_kernel<FT, ZW, 0><<<grd, blk, 0, stream()>>>(c); break;
+        case 1: tendency_fast_kernel<FT, ZW, 1><<<grd, blk, 0, stream()>>>(c); break;
+        case 2: tendency_fast_kernel<FT, ZW, 2><<<grd, blk, 0, stream()>>>(c); break;
+        default: tendency_fast_kernel<FT, ZW, 3><<<grd, blk, 0, stream()>>>(c); break;
     }
     OB_LAUNCH_CHECK();
 }
@@ -187,19 +152,22 @@ bool launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], con
         if (P.wc[d][0] || P.wc[d][1]) return false;
         if (g.topo[d] != OB_FLAT && g.H[d] < 3) return false;
     }
-    if (g.N[0] % fast::TX || g.N[1] % (fast::ROWS * fast::TY)) return false;
-    if (hasz && tma::launch<FT>(P, comp, U, psi, pHY, Gn, Gm, psi_new, ss)) return true;
+    // the TMA kernel takes a ragged last tile in y, but Ny % 8 gates 3-D grids too: which kernel a grid takes decides
+    // the rounding of its results
+    if (g.N[0] % fast::TX || g.N[1] % fast::TY) return false;
+    if (hasz) {
+        if ((g.S[0] * sizeof(FT)) % 16) return false;     // tensor-map row strides are multiples of 16 bytes
+        tma::launch<FT>(P, comp, U, psi, pHY, Gn, Gm, psi_new, ss);
+        return true;
+    }
     fast::Ctx<FT> c;
-    for (int d = 0; d < 3; ++d) { c.U[d] = U[d]; c.s[d] = g.st[d]; c.N[d] = g.N[d]; c.invd[d] = 1 / g.d[d]; }
+    for (int d = 0; d < 2; ++d) { c.U[d] = U[d]; c.N[d] = g.N[d]; c.invd[d] = 1 / g.d[d]; }
+    for (int d = 0; d < 3; ++d) c.s[d] = g.st[d];
     c.psi = psi; c.pHY = pHY; c.Gm = Gm; c.Gn = Gn; c.psi_new = psi_new; c.ss = ss;
-    c.area[0] = g.d[1] * g.d[2]; c.area[1] = g.d[0] * g.d[2]; c.area[2] = g.d[0] * g.d[1];
+    c.area[0] = g.d[1] * g.d[2]; c.area[1] = g.d[0] * g.d[2];
     c.invV = 1 / ((g.d[0] * g.d[1]) * g.d[2]);
     c.f = P.f; c.fplane = P.fplane;
-    int Kc = 1;
-    if (hasz) { Kc = 16; while (g.N[2] % Kc) Kc >>= 1; }
-    c.Kc = Kc;
-    if (hasz) { if (P.zweno) fast::launch<FT, true, true>(c, comp); else fast::launch<FT, false, true>(c, comp); }
-    else { if (P.zweno) fast::launch<FT, true, false>(c, comp); else fast::launch<FT, false, false>(c, comp); }
+    if (P.zweno) fast::launch<FT, true>(c, comp); else fast::launch<FT, false>(c, comp);
     return true;
 }
 template bool launch_tendency_fast<float>(const Phys<float>&, int, const float* const[3], const float*,

@@ -122,9 +122,6 @@ struct Work {
 __device__ __forceinline__ void named_sync(int id, int nthreads) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
-__device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tmau::smem_u32(bar)) : "memory");
-}
 
 template <class FT>
 __device__ __forceinline__ FT interp12(FT cm, FT c0, FT c1, FT c2) {      // 12 x wf::interp4
@@ -412,7 +409,7 @@ __device__ __forceinline__ void group_main(const KArgs<FT, 3 + NT, FRC>& c, FT* 
                 }
             }
             named_sync(1 + GRP, GT);              // faces published; this group's stencil reads of the level are finished:
-            if (edge && tx == 0) mbar_arrive(&done[git & 3]);     // the producer may refill the slot of level k-2 two levels on
+            if (edge && tx == 0) tmau::mbar_arrive(&done[git & 3]);     // the producer may refill the slot of level k-2 two levels on
             if (cell) {
 #pragma unroll
                 for (int s = 0; s < FPG; ++s) {
@@ -481,7 +478,7 @@ tendency_fused_kernel(const __grid_constant__ KArgs<FT, 3 + NT, FRC> c) {
     const int warp = threadIdx.x >> 5;
     if (threadIdx.x == 0) {
         for (int q = 0; q < 4; ++q) { tmau::mbar_init(&full[q], 1); tmau::mbar_init(&done[q], NG); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        tmau::mbar_init_fence();
     }
     __syncthreads();
     if (warp == NG * (R + 1)) {
@@ -624,15 +621,9 @@ static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part
         OB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G_::SMEM));
         attr_set = true;
     }
-    static int sms = 0;
-    if (!sms) {
-        int dev = 0;
-        OB_CUDA(cudaGetDevice(&dev));
-        OB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    }
     const long long T = (long long)c.ntiles * c.Nz;
     if (T >= (1LL << 30)) throw Error("tendency_fused: grid too large for the 32-bit work decomposition");
-    const int grid = (int)std::max(1LL, std::min((long long)sms, T / 8));
+    const int grid = (int)std::max(1LL, std::min((long long)tmau::sm_count(), T / 8));
     c.chunk = cdiv((long long)(c.ntiles - (c.ntiles / grid) * grid) * c.Nz, grid);
     kern<<<grid, TX * (GR::NG * (R + 1) + 1), G_::SMEM, stream()>>>(c);
     OB_LAUNCH_CHECK();

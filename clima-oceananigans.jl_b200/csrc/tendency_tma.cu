@@ -21,75 +21,7 @@
 #include "internal.h"
 #include "weno_fast.cuh"
 #include "tma_util.cuh"
-#include <cuda.h>
 #include <cmath>
-#include <map>
-#include <mutex>
-#include <tuple>
-
-
-namespace ob {
-namespace tmau {
-
-typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                             const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                             CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeFn get_encode() {
-    static EncodeFn fn = nullptr;
-    if (!fn) {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qr;
-        OB_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qr));
-        if (!p || qr != cudaDriverEntryPointSuccess) throw Error("cuTensorMapEncodeTiled not available");
-        fn = (EncodeFn)p;
-    }
-    return fn;
-}
-
-typedef std::tuple<const void*, int, int, int, int, int, int> MapKey;
-static std::map<MapKey, CUtensorMap>& map_cache() { static std::map<MapKey, CUtensorMap> c; return c; }
-static std::mutex& map_mutex() { static std::mutex m; return m; }
-
-template <class FT>
-CUtensorMap make_map(const GridD<FT>& g, const FT* base, int box_x, int box_y) {
-    std::lock_guard<std::mutex> lk(map_mutex());
-    auto& cache = map_cache();
-    auto key = std::make_tuple((const void*)base, g.S[0], g.S[1], g.S[2], (int)sizeof(FT), box_x, box_y);
-    auto it = cache.find(key);
-    if (it != cache.end()) return it->second;
-    CUtensorMap m;
-    cuuint64_t dims[3] = {(cuuint64_t)g.S[0], (cuuint64_t)g.S[1], (cuuint64_t)g.S[2]};
-    cuuint64_t strides[2] = {(cuuint64_t)g.S[0] * sizeof(FT), (cuuint64_t)g.S[0] * g.S[1] * sizeof(FT)};
-    cuuint32_t box[3] = {(cuuint32_t)box_x, (cuuint32_t)box_y, 1};
-    cuuint32_t es[3] = {1, 1, 1};
-    CUresult r = get_encode()(&m, sizeof(FT) == 8 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT64 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3,
-                              (void*)base, dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                              CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) throw Error("cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")");
-    cache[key] = m;
-    return m;
-}
-template CUtensorMap make_map<float>(const GridD<float>&, const float*, int, int);
-template CUtensorMap make_map<double>(const GridD<double>&, const double*, int, int);
-
-void evict_maps(const void* base, size_t bytes) {
-    std::lock_guard<std::mutex> lk(map_mutex());
-    auto& cache = map_cache();
-    const char* lo = (const char*)base;
-    const char* hi = lo + bytes;
-    for (auto it = cache.begin(); it != cache.end();) {
-        const char* p = (const char*)std::get<0>(it->first);
-        if (p >= lo && p < hi) it = cache.erase(it); else ++it;
-    }
-}
-size_t cached_maps() {
-    std::lock_guard<std::mutex> lk(map_mutex());
-    return map_cache().size();
-}
-
-}  // namespace tmau
-}  // namespace ob
 
 namespace ob {
 namespace tma {
@@ -136,7 +68,7 @@ struct Ctx {
     Substep<FT> ss;
 };
 
-using tmau::smem_u32; using tmau::mbar_init; using tmau::mbar_expect_tx; using tmau::mbar_wait; using tmau::tma_load_3d;
+using tmau::mbar_init; using tmau::mbar_init_fence; using tmau::mbar_expect_tx; using tmau::mbar_wait; using tmau::tma_load_3d;
 
 // position inside the staged data: level L (Julia k), tile row / column including the halo offset
 struct P3 { int L, row, col; };
@@ -215,7 +147,7 @@ __global__ void __launch_bounds__(TX * NW, 3) tendency_tma_kernel(const __grid_c
     if (producer) {
         mbar_init(&bars[0], 1);
         mbar_init(&bars[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     __syncthreads();
 
@@ -345,13 +277,11 @@ static void launch_one(Ctx<FT>& c, const GridD<FT>& g, const FT* const U[3], con
     OB_LAUNCH_CHECK();
 }
 
+// eligibility (3-D grid, Nx % 32 == 0, 16-byte row strides, field not forced) is checked by launch_tendency_fast
 template <class FT>
-bool launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, const FT* pHY, FT* Gn, const FT* Gm,
+void launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, const FT* pHY, FT* Gn, const FT* Gm,
             FT* psi_new, const Substep<FT>& ss) {
     const GridD<FT>& g = P.g;
-    if (P.frc[comp].on) return false;          // forced fields run on the general kernels
-    if (g.topo[2] == OB_FLAT || g.N[0] % TX) return false;
-    if ((g.S[0] * sizeof(FT)) % 16) return false;
     Ctx<FT> c;
     c.psi = psi; c.pHY = pHY; c.Gm = Gm; c.Gn = Gn; c.psi_new = psi_new; c.ss = ss;
     c.cor = comp == 0 ? U[1] : U[0];
@@ -370,11 +300,10 @@ bool launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, co
     }
     if (P.zweno) { GO(true) } else { GO(false) }
 #undef GO
-    return true;
 }
-template bool launch<float>(const Phys<float>&, int, const float* const[3], const float*, const float*, float*,
+template void launch<float>(const Phys<float>&, int, const float* const[3], const float*, const float*, float*,
                             const float*, float*, const Substep<float>&);
-template bool launch<double>(const Phys<double>&, int, const double* const[3], const double*, const double*, double*,
+template void launch<double>(const Phys<double>&, int, const double* const[3], const double*, const double*, double*,
                              const double*, double*, const Substep<double>&);
 }  // namespace tma
 }  // namespace ob

@@ -58,8 +58,9 @@ def test_cuda_path_reproduces_golden_poisson(ob, name):
 
 
 # ---- the specialised kernels of the headline path, at sizes the oracle finishes in seconds ---------------------
-# (Nx multiple of 32 -> tendency_tma_kernel; power-of-two sizes -> fast FFT + TMA line passes; all Periodic -> fused
-# stage with wrap-around reads and the shell fill).  Ny = 20 and 9 give ragged last tiles in y.
+# (all Periodic -> fused tendency kernel for u, v, w and the first tracer, fused stage with wrap-around reads and the
+# shell fill; power-of-two sizes -> fast FFT + TMA line passes; Nx % 32 == 0 and Ny % 8 == 0 -> tendency_tma_kernel for
+# the tracers beyond the first).  Ny = 20 and 9 give ragged last tiles in y.
 FAST_CASES = {
     "rk3_zweno": dict(size=(32, 16, 16), ts="RungeKutta3", zweno=True, f=None, steps=3),
     "rk3_zweno_ragged": dict(size=(64, 20, 8), ts="RungeKutta3", zweno=True, f=None, steps=2),
@@ -70,6 +71,11 @@ FAST_CASES = {
     "rk3_two_tracers": dict(size=(32, 12, 16), ts="RungeKutta3", zweno=True, f=None, steps=2, tracers=("b", "c")),
     "ab2_three_tracers": dict(size=(64, 9, 8), ts="QuasiAdamsBashforth2", zweno=True, f=0.5, steps=2,
                               tracers=("b", "c", "d")),
+    # c and d on the per-field TMA kernel (Ny % 8 == 0), in both weight kinds and substep modes
+    "rk3_three_tracers_tma": dict(size=(32, 16, 16), ts="RungeKutta3", zweno=True, f=None, steps=2,
+                                  tracers=("b", "c", "d")),
+    "ab2_js_fplane_three_tracers_tma": dict(size=(32, 16, 16), ts="QuasiAdamsBashforth2", zweno=False, f=0.5, steps=2,
+                                            tracers=("b", "c", "d")),
 }
 
 
