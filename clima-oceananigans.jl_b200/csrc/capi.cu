@@ -122,8 +122,10 @@ struct ob200_field {
     int psize[3];
     void* staging = nullptr;                // device copy in the reference's parent layout (uploads)
     void* staging_out = nullptr;            // ... and a second one for asynchronous downloads
+    void* bcv[6] = {};                      // array condition per side (ob200_field_set_boundary_values), null = bcs[s].value
     cudaEvent_t ev_in_ready = nullptr, ev_in_free = nullptr, ev_out_ready = nullptr, ev_out_free = nullptr;
     ~ob200_field() {
+        for (void* p : bcv) if (p) cudaFree(p);
         if (owns) {
             // tensor maps over these buffers (tendency kernels) must not outlive them: the allocator may hand the same
             // address to a field of another grid
@@ -540,6 +542,26 @@ extern "C" int32_t ob200_field_device_view(const ob200_field* f, void** base, in
     return 0;
 }
 
+// entry q of a halo batch: field f with its boundary conditions (constant values and array tables)
+template <class FT>
+static void halo_entry(HaloBatch<FT>& hb, int q, const ob200_field* f) {
+    hb.p0[q] = f->p0<FT>();
+    for (int d = 0; d < 3; ++d) hb.loc[q][d] = f->loc[d];
+    for (int s = 0; s < 6; ++s) {
+        hb.bc_kind[q][s] = f->bcs[s].kind;
+        hb.bc_val[q][s] = (FT)f->bcs[s].value;
+        hb.bc_tab[q][s] = (const FT*)f->bcv[s];
+    }
+}
+// the constant Flux boundary conditions the tendency kernels add themselves: a side with an array condition is "no constant
+// flux" there, because the boundary-plane pass (model_boundary_fluxes) adds it
+template <class FT>
+static FluxBC<FT> constant_flux_bcs(const ob200_field* f) {
+    FluxBC<FT> fbc;
+    for (int s = 0; s < 6; ++s) { fbc.kind[s] = f->bcs[s].kind; fbc.val[s] = f->bcv[s] ? FT(0) : (FT)f->bcs[s].value; }
+    return fbc;
+}
+
 template <class FT>
 static void fill_halos(ob200_field* const* fields, int n) {
     if (n == 0) return;
@@ -551,9 +573,7 @@ static void fill_halos(ob200_field* const* fields, int n) {
         for (int q = 0; q < hb.n; ++q) {
             ob200_field* f = fields[start + q];
             if (f->grid != G) throw Error("fill_halo_regions: fields live on different grids");
-            hb.p0[q] = f->p0<FT>();
-            for (int d = 0; d < 3; ++d) hb.loc[q][d] = f->loc[d];
-            for (int s = 0; s < 6; ++s) { hb.bc_kind[q][s] = f->bcs[s].kind; hb.bc_val[q][s] = (FT)f->bcs[s].value; }
+            halo_entry<FT>(hb, q, f);
         }
         launch_fill_halos<FT>(g, hb);
     }
@@ -563,6 +583,47 @@ extern "C" int32_t ob200_fill_halo_regions(ob200_field* const* fields, int32_t n
     if (n <= 0) return 0;
     if (fields[0]->grid->ftype == OB200_F32) fill_halos<float>(fields, n);
     else fill_halos<double>(fields, n);
+    API_END
+}
+
+// FluxBoundaryCondition(Q) / ValueBoundaryCondition(Q) / GradientBoundaryCondition(Q) with a 2-D array Q
+// (BoundaryConditions/boundary_condition.jl: getbc(bc::BC{<:Any,<:AbstractArray}, i, j, grid, ...) = bc.condition[i, j])
+extern "C" int32_t ob200_field_set_boundary_values(ob200_field* f, int32_t side, const void* values) {
+    API_BEGIN
+    if (!f) throw Error("null argument");
+    if (side < 0 || side > 5) throw Error("boundary values: side out of range");
+    static const char* names[6] = {"west", "east", "south", "north", "bottom", "top"};
+    const std::string who = std::string("boundary values of the ") + names[side] + " side: ";
+    const ob200_grid_desc& D = f->grid->desc;
+    const int d = side / 2;
+    for (int e = 0; e < 3; ++e)
+        if (D.topology[e] == OB200_FULLY_CONNECTED)
+            throw Error(who + "array conditions are not supported on a slab-decomposed (FullyConnected) grid");
+    if (D.topology[d] != OB200_BOUNDED) throw Error(who + "the dimension is not Bounded (Periodic, Flat or FullyConnected)");
+    const int kind = f->bcs[side].kind;
+    if (kind != OB200_BC_FLUX && kind != OB200_BC_VALUE && kind != OB200_BC_GRADIENT)
+        throw Error(who + "array conditions need a Flux, Value or Gradient boundary condition (not Open / None)");
+    if (f->loc[d] == OB200_FACE)
+        throw Error(who + "the field is located on the faces normal to this side (the impenetrable wall)");
+    if (!values) {
+        if (f->bcv[side]) {
+            OB_CUDA(cudaStreamSynchronize(stream()));      // kernels enqueued so far may still read the table
+            OB_CUDA(cudaFree(f->bcv[side]));
+            f->bcv[side] = nullptr;
+        }
+        return 0;
+    }
+    size_t count = 1;
+    for (int e = 0; e < 3; ++e)
+        if (e != d) count *= (size_t)D.N[e];           // a Flat dimension has N = 1
+    const size_t bytes = count * fsize(f->grid);
+    if (!f->bcv[side]) OB_CUDA(cudaMalloc(&f->bcv[side], bytes));
+    // on the library stream: after every step enqueued so far (a step joins its side streams before its last kernel), before
+    // the next one.  A pageable source is staged before the call returns; a pinned one is read by the DMA itself, so wait for it
+    OB_CUDA(cudaMemcpyAsync(f->bcv[side], values, bytes, cudaMemcpyHostToDevice, stream()));
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, values) != cudaSuccess) cudaGetLastError();    // the query's own error only
+    else if (pa.type == cudaMemoryTypeHost) OB_CUDA(cudaStreamSynchronize(stream()));
     API_END
 }
 
@@ -1053,12 +1114,7 @@ static void fill_halos_overlapped(ob200_model* m, ob200_field* const* fields, in
     auto batch = [&](int start) {
         HaloBatch<FT> hb;
         hb.n = std::min(MAXF, n - start);
-        for (int q = 0; q < hb.n; ++q) {
-            ob200_field* f = fields[start + q];
-            hb.p0[q] = f->p0<FT>();
-            for (int d = 0; d < 3; ++d) hb.loc[q][d] = f->loc[d];
-            for (int s = 0; s < 6; ++s) { hb.bc_kind[q][s] = f->bcs[s].kind; hb.bc_val[q][s] = (FT)f->bcs[s].value; }
-        }
+        for (int q = 0; q < hb.n; ++q) halo_entry<FT>(hb, q, fields[start + q]);
         return hb;
     };
     for (int start = 0; start < n; start += MAXF) launch_fill_halos_phase<FT>(g, batch(start), 0);
@@ -1138,6 +1194,37 @@ extern "C" int32_t ob200_model_update_state(ob200_model* m) {
     API_END
 }
 
+// calculate_boundary_tendency_contributions! of the array Flux conditions (constant ones are added inside the tendency
+// kernels): after every tendency launch of the stage, while the state buffer still holds the old state and the second buffer
+// the new one; one launch per Bounded dimension that carries an array Flux, in the reference's x, y, z order
+template <class FT>
+static void model_boundary_fluxes(ob200_model* m, const Substep<FT>& ss) {
+    const GridD<FT>& g = gridD<FT>(m->grid);
+    for (int d = 0; d < 3; ++d) {
+        if (g.topo[d] != OB_BOUNDED) continue;
+        BoundaryFluxes<FT> a;
+        a.n = 0;
+        a.ss = ss;
+        for (int q = 0; q < m->nf; ++q) {
+            const ob200_field* f = m->F[q].get();
+            const FT* lo = f->bcs[2 * d].kind == OB200_BC_FLUX ? (const FT*)f->bcv[2 * d] : nullptr;
+            const FT* hi = f->bcs[2 * d + 1].kind == OB200_BC_FLUX ? (const FT*)f->bcv[2 * d + 1] : nullptr;
+            if (!lo && !hi) continue;
+            const int k = a.n++;
+            a.comp[k] = std::min(q, 3);
+            a.Q[k][0] = lo; a.Q[k][1] = hi;
+            a.Gn[k] = m->Gn[q]->template p0<FT>();
+            a.Gm[k] = m->Gm[q]->template p0<FT>();
+            a.psi[k] = f->template p0<FT>();
+            a.psi_new[k] = ss.mode == SUB_NONE ? nullptr : f->template alt0<FT>();
+        }
+        if (a.n) {
+            ScopedPhase ph("boundary_flux");
+            launch_boundary_fluxes<FT>(g, d, a);
+        }
+    }
+}
+
 template <class FT>
 static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
     Phys<FT>& P = physOf<FT>(m);
@@ -1170,7 +1257,7 @@ static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
             ff.Gm[q] = m->Gm[q]->template p0<FT>();
             ff.Gn[q] = m->Gn[q]->template p0<FT>();
             ff.nw[q] = ss.mode == SUB_NONE ? nullptr : f->template alt0<FT>();
-            for (int s = 0; s < 6; ++s) { ff.fbc[q].kind[s] = f->bcs[s].kind; ff.fbc[q].val[s] = (FT)f->bcs[s].value; }
+            ff.fbc[q] = constant_flux_bcs<FT>(f);
         }
         // a closure the fused kernel does not evaluate itself (LES closures; any closure on the triply periodic variant): its flux
         // divergence alone goes into G^n through the general shared-face kernel, and the fused kernel adds everything else
@@ -1198,8 +1285,7 @@ static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
     bool lane_forked[3] = {false, false, false};        // a side stream waits for the fork event before its first launch
     for (int q = first; q < m->nf; ++q) {
         ob200_field* f = m->F[q].get();
-        FluxBC<FT> fbc;
-        for (int s = 0; s < 6; ++s) { fbc.kind[s] = f->bcs[s].kind; fbc.val[s] = (FT)f->bcs[s].value; }
+        const FluxBC<FT> fbc = constant_flux_bcs<FT>(f);
         FT* newp = ss.mode == SUB_NONE ? nullptr : f->template alt0<FT>();
         bool done = false;
         const int lane = fork ? q % 4 : 0;               // lane 0 = the library stream itself
@@ -1222,6 +1308,7 @@ static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
             OB_CUDA(cudaEventRecord(ev_join[q], side[q]));
             OB_CUDA(cudaStreamWaitEvent(g_stream, ev_join[q], 0));
         }
+    model_boundary_fluxes<FT>(m, ss);
     if (ss.mode != SUB_NONE) {
         // the out-of-place substep wrote the new state into the second buffer: swap.  Cells the
         // kernels never write (wall faces, outer halos of Bounded dims) are refreshed by the halo
@@ -1260,9 +1347,8 @@ static void model_pressure_step(ob200_model* m, FT dt, bool tracers_too = false,
     auto exchange_one = [&](ob200_field* f, bool need_lo, bool need_hi) {
         ScopedPhase ph("halo");
         HaloBatch<FT> hb;
-        hb.n = 1; hb.p0[0] = f->template p0<FT>();
-        for (int d = 0; d < 3; ++d) hb.loc[0][d] = f->loc[d];
-        for (int s = 0; s < 6; ++s) { hb.bc_kind[0][s] = f->bcs[s].kind; hb.bc_val[0][s] = (FT)f->bcs[s].value; }
+        hb.n = 1;
+        halo_entry<FT>(hb, 0, f);
         launch_exchange_planes<FT>(g, hb, dc, 1, need_lo, need_hi);
     };
     if (!fused) { ScopedPhase ph("halo"); model_fill_state_halos<FT>(m, 0, tracers_too ? m->nf : 3); }

@@ -16,6 +16,7 @@ struct HaloBatch {
     int loc[MAXF][3];
     int bc_kind[MAXF][6];
     FT bc_val[MAXF][6];
+    const FT* bc_tab[MAXF][6];   // array condition of a Bounded side (ob200_field_set_boundary_values), null = bc_val
 };
 template <class FT> void launch_fill_halos(const GridD<FT>& g, const HaloBatch<FT>& hb);
 // the slab-decomposed fill in two phases (kernels.cu): 0 = Periodic halos of the owned rows, 1 = neighbour exchange + Periodic
@@ -41,6 +42,21 @@ struct FluxBC {            // constant Flux boundary conditions of the field bei
     int kind[6];
     FT val[6];
 };
+// array Flux boundary conditions (FluxBoundaryCondition(Q), Q a 2-D array) of the Bounded dimension d, for all fields that
+// have one, after the tendency kernels: G^n += Q A / V at the boundary cells (apply_flux_bcs.jl:35-160) and, with a substep,
+// the new state of those cells recomputed from the old state, the final G^n and G^-
+template <class FT>
+struct BoundaryFluxes {
+    int n;
+    int comp[MAXF];                  // 0, 1, 2 = u, v, w; 3 = a tracer
+    const FT* Q[MAXF][2];            // low / high side table, (N_a, N_b) column-major, null = no array there
+    FT* Gn[MAXF];
+    const FT* Gm[MAXF];
+    const FT* psi[MAXF];             // old state
+    FT* psi_new[MAXF];               // new state (unused with SUB_NONE)
+    Substep<FT> ss;
+};
+template <class FT> void launch_boundary_fluxes(const GridD<FT>& g, int d, const BoundaryFluxes<FT>& a);
 // general tendency (+ optional fused substep) for prognostic field `comp`
 template <class FT>
 void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,

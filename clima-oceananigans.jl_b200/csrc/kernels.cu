@@ -34,7 +34,10 @@ __global__ void fill_halo_kernel(GridD<FT> g, HaloBatch<FT> hb, int d, int a, in
             FT* f = hb.p0[n] + base;
             for (int side = 0; side < 2; ++side) {
                 int kind = hb.bc_kind[n][2 * d + side];
-                FT val = hb.bc_val[n][2 * d + side];
+                // getbc(bc::BC{<:Any,<:AbstractArray}, i, j, grid) = bc.condition[i, j] (boundary_condition.jl): the array
+                // spans the interior extent (1..ahi) x (1..bhi) of the tangential dimensions, alo = blo = 1 here
+                const FT* tab = hb.bc_tab[n][2 * d + side];
+                FT val = tab ? tab[(ia - 1) + (long long)(ib - 1) * ahi] : hb.bc_val[n][2 * d + side];
                 if (kind == 2) {                            // Flux: mirror (fill_halo_regions_flux.jl:16-28)
                     if (side == 0) f[0] = f[s];
                     else f[(N + 1) * s] = f[N * s];
@@ -324,6 +327,8 @@ void launch_fill_halos(const GridD<FT>& g, const HaloBatch<FT>& hb) {
             }
             dim3 blk(a == 0 ? 64 : 16, a == 0 ? 4 : 16);
             dim3 grd(cdiv(hi[0] - lo[0] + 1, blk.x), cdiv(hi[1] - lo[1] + 1, blk.y));
+            static_assert(sizeof(GridD<double>) + sizeof(HaloBatch<double>) + 6 * sizeof(int) <= 4096,
+                          "fill_halo_kernel parameters must stay within the 4 KB kernel-parameter space");
             fill_halo_kernel<FT><<<grd, blk, 0, stream()>>>(g, hb, d, a, b, lo[0], hi[0], lo[1], hi[1]);
             OB_LAUNCH_CHECK();
         }
@@ -383,6 +388,61 @@ __global__ void __launch_bounds__(128) tendency_general_kernel(const __grid_cons
     else if (s.mode == SUB_RK3) A.psi_new[q.p] = A.psi[q.p] + s.dt * (s.c1 * G + s.c2 * A.Gm[q.p]);
     else if (s.mode == SUB_AB2) A.psi_new[q.p] = A.psi[q.p] + s.dt * (s.c1 * G - s.c2 * A.Gm[q.p]);
 }
+
+// =============================================================================================
+// array Flux boundary conditions: one boundary-plane pass per Bounded dimension after the tendency kernels of every path
+// (apply_x/y/z_bcs!, apply_flux_bcs.jl:35-160, run in the reference as a separate step after the interior tendencies, in
+// dimension order).  One thread per tangential point (ia, ib) walks the fields and both sides of dimension d in sequence, so a
+// cell that is first and last at once (N = 1) gets both contributions in the reference's order.  The sum and the substep are
+// the expressions of tendency_general_kernel above.
+// =============================================================================================
+template <class FT, int d>
+__global__ void __launch_bounds__(128) boundary_flux_kernel(const GridD<FT> g, const BoundaryFluxes<FT> A, int na, int nb) {
+    constexpr int a = d == 0 ? 1 : 0, b = d == 2 ? 1 : 2;      // tangential dimensions (compile-time: no local-memory indexing)
+    const int ia = 1 + blockIdx.x * blockDim.x + threadIdx.x;
+    const int ib = 1 + blockIdx.y * blockDim.y + threadIdx.y;
+    if (ia > na || ib > nb) return;
+    const long long t = (ia - 1) + (long long)(ib - 1) * na;       // Q[ia, ib], column-major
+    Pt q;
+    q.i[a] = ia; q.i[b] = ib;
+    const Substep<FT>& s = A.ss;
+    for (int n = 0; n < A.n; ++n) {
+        const int c = A.comp[n];
+        const int l[3] = {c == 0 ? OB_F : OB_C, c == 1 ? OB_F : OB_C, c == 2 ? OB_F : OB_C};
+        int lf[3] = {l[0], l[1], l[2]};
+        lf[d] = l[d] == OB_C ? OB_F : OB_C;
+        for (int side = 0; side < 2; ++side) {
+            const FT* Q = A.Q[n][side];
+            if (!Q) continue;
+            q.i[d] = side == 0 ? 1 : g.N[d];
+            q.p = q.i[0] * g.st[0] + q.i[1] * g.st[1] + q.i[2] * g.st[2];
+            FT G = A.Gn[n][q.p];
+            if (side == 0) G += Q[t] * areaA(g, d, q, lf[0], lf[1], lf[2]) / volume(g, q, l[0], l[1], l[2]);
+            else G -= Q[t] * areaA(g, d, sh(g, q, d, 1), lf[0], lf[1], lf[2]) / volume(g, q, l[0], l[1], l[2]);
+            A.Gn[n][q.p] = G;
+            const FT* psi = A.psi[n];
+            FT* psi_new = A.psi_new[n];
+            if (s.mode == SUB_RK3_FIRST) psi_new[q.p] = psi[q.p] + s.c1 * G;
+            else if (s.mode == SUB_RK3) psi_new[q.p] = psi[q.p] + s.dt * (s.c1 * G + s.c2 * A.Gm[n][q.p]);
+            else if (s.mode == SUB_AB2) psi_new[q.p] = psi[q.p] + s.dt * (s.c1 * G - s.c2 * A.Gm[n][q.p]);
+        }
+    }
+}
+
+template <class FT>
+void launch_boundary_fluxes(const GridD<FT>& g, int d, const BoundaryFluxes<FT>& A) {
+    if (A.n == 0) return;
+    const int a = d == 0 ? 1 : 0, b = d == 2 ? 1 : 2;
+    const int na = g.topo[a] == OB_FLAT ? 1 : g.N[a], nb = g.topo[b] == OB_FLAT ? 1 : g.N[b];
+    dim3 blk(a == 0 ? 32 : 16, a == 0 ? 4 : 8);
+    dim3 grd(cdiv(na, blk.x), cdiv(nb, blk.y));
+    if (d == 0) boundary_flux_kernel<FT, 0><<<grd, blk, 0, stream()>>>(g, A, na, nb);
+    else if (d == 1) boundary_flux_kernel<FT, 1><<<grd, blk, 0, stream()>>>(g, A, na, nb);
+    else boundary_flux_kernel<FT, 2><<<grd, blk, 0, stream()>>>(g, A, na, nb);
+    OB_LAUNCH_CHECK();
+}
+template void launch_boundary_fluxes<float>(const GridD<float>&, int, const BoundaryFluxes<float>&);
+template void launch_boundary_fluxes<double>(const GridD<double>&, int, const BoundaryFluxes<double>&);
 
 // =============================================================================================
 // general tendency kernel with SHARED faces (any scheme / closure / BCs on a 3-D grid)

@@ -188,10 +188,75 @@ bc_code(bc::BoundaryCondition{<:Value})    = BC(3, constant_value(bc))
 bc_code(bc::BoundaryCondition{<:Gradient}) = BC(4, constant_value(bc))
 bc_code(bc::BoundaryCondition{<:Open})     = BC(5, constant_value(bc))
 bc_code(bc::BoundaryCondition)             = BC(1, 0.0)                 # Periodic / communication: decided by the topology
+# an array condition crosses as its kind with value 0; its values follow through ob200_field_set_boundary_values
 constant_value(bc) = bc.condition === nothing ? 0.0 : bc.condition isa Number ? Float64(bc.condition) :
-    throw(ArgumentError("B200(): only constant boundary conditions are supported (function and array conditions cannot cross the C ABI)"))
+    bc.condition isa AbstractMatrix ? 0.0 :
+    throw(ArgumentError("B200(): only constant and 2-D array boundary conditions are supported (function conditions cannot cross the C ABI)"))
 bc_codes(bcs::FieldBoundaryConditions) = map(bc_code, (bcs.west, bcs.east, bcs.south, bcs.north, bcs.bottom, bcs.top))
 bc_codes(::Nothing) = ntuple(_ -> BC(0, 0.0), 6)
+
+# ---- array conditions: FluxBoundaryCondition(Q) / ValueBoundaryCondition(Q) / GradientBoundaryCondition(Q), Q a 2-D array
+# indexed by the grid's interior indices along the side's tangential dimensions (getbc(bc::BC{<:Any,<:AbstractArray}, i, j,
+# grid) = bc.condition[i, j], BoundaryConditions/boundary_condition.jl) --------------------------------------------------------
+const SIDES = (:west, :east, :south, :north, :bottom, :top)
+
+"""
+The condition of an array boundary condition once it lives in the library (the reference requires it on the device,
+boundary_condition.jl:143-149).  `copyto!(q, Q)` and `q .= ...` (a callback varying the forcing in time) call
+ob200_field_set_boundary_values, ordered after every step enqueued so far; reads see the host copy of the last values.
+"""
+mutable struct B200BoundaryArray{T} <: AbstractMatrix{T}
+    field :: Ptr{Cvoid}            # ob200_field* of the model field
+    side  :: Int32                 # 0..5 = west, east, south, north, bottom, top
+    host  :: Matrix{T}             # the values last sent
+    owner :: Any                   # keeps the model handle alive
+end
+size(q::B200BoundaryArray) = size(q.host)
+architecture(::B200BoundaryArray) = B200()       # passes the reference's device check of array conditions
+Base.getindex(q::B200BoundaryArray, i::Int, j::Int) = q.host[i, j]
+Base.setindex!(::B200BoundaryArray, v, i...) = error("set the values of a B200 boundary condition with `copyto!` or `.=`")
+function copyto!(q::B200BoundaryArray{T}, h::AbstractMatrix) where T
+    size(h) == size(q.host) || throw(DimensionMismatch("boundary values of size $(size(h)), the side needs $(size(q.host))"))
+    copyto!(q.host, h)
+    GC.@preserve q check(ccall((:ob200_field_set_boundary_values, lib), Int32, (Ptr{Cvoid}, Int32, Ptr{Cvoid}),
+                               q.field, q.side, q.host))
+    return q
+end
+copyto!(q::B200BoundaryArray{T}, bc::Base.Broadcast.Broadcasted) where T = copyto!(q, copyto!(similar(q.host), bc))
+
+"The (N_a, N_b) host table of the array condition of `side` of a field at `loc`, checked as the library does, or nothing."
+function boundary_table(bc, side, grid, loc)
+    bc === nothing && return nothing
+    Q = bc.condition
+    Q isa AbstractArray || return nothing
+    d = (findfirst(==(side), SIDES) - 1) ÷ 2 + 1
+    Q isa AbstractMatrix && eltype(Q) <: Real ||
+        throw(ArgumentError("B200(): the $side boundary condition must be a 2-D real array, got $(typeof(Q))"))
+    any(t -> t === FullyConnected, topology(grid)) &&
+        throw(ArgumentError("B200(): array boundary conditions are not supported on slab-decomposed (FullyConnected) grids"))
+    topology(grid, d) === Bounded ||
+        throw(ArgumentError("B200(): array boundary condition on the $side side of a $(topology(grid, d)) dimension"))
+    bc.classification isa Union{Flux, Value, Gradient} ||
+        throw(ArgumentError("B200(): array boundary conditions must be Flux, Value or Gradient conditions"))
+    loc[d] === Face &&
+        throw(ArgumentError("B200(): the $side side of a field on the $("xyz"[d])-faces is the impenetrable wall"))
+    shape = Tuple(topology(grid, e) === Flat ? 1 : size(grid, e) for e in 1:3 if e != d)
+    size(Q) == shape || throw(ArgumentError("B200(): the $side boundary condition has size $(size(Q)); the grid needs $shape"))
+    return Matrix{eltype(grid)}(Array(Q))
+end
+
+"Push the array conditions of a model field and return its boundary conditions with those conditions as B200BoundaryArrays."
+function attach_boundary_arrays(fbcs::FieldBoundaryConditions, tables, fh::Ptr{Cvoid}, owner)
+    isempty(tables) && return fbcs
+    conds = map(fieldnames(typeof(fbcs))) do name
+        bc = getfield(fbcs, name)
+        haskey(tables, name) || return bc
+        q = B200BoundaryArray(fh, Int32(findfirst(==(name), SIDES) - 1), similar(tables[name]), owner)
+        copyto!(q, tables[name])
+        return BoundaryCondition(bc.classification, q)
+    end
+    return FieldBoundaryConditions(conds...)
+end
 
 "Wrap an ob200_field as the OffsetArray `data` of a Field (same axes as Grids/new_data.jl:56-61 gives on CPU)."
 function wrap_field(FT, grid, loc, fh::Ptr{Cvoid}, owner)
@@ -443,6 +508,11 @@ function b200_nonhydrostatic_model(; grid, clock = Clock{eltype(grid)}(0, 0, 1),
     default_bcs = NamedTuple{names}(FieldBoundaryConditions() for _ in names)
     bcs = regularize_field_boundary_conditions(merge(default_bcs, boundary_conditions), grid, names)
     buoyancy = Oceananigans.BuoyancyModels.regularize_buoyancy(buoyancy)
+    locs = (u = (Face, Center, Center), v = (Center, Face, Center), w = (Center, Center, Face))
+    loc_of(n) = haskey(locs, n) ? locs[n] : (Center, Center, Center)
+    # array boundary conditions: checked before any library call, pushed once the model exists
+    tables = Dict(n => Dict(s => t for s in SIDES for t in (boundary_table(getfield(bcs[n], s), s, grid, loc_of(n)),)
+                            if t !== nothing) for n in names)
     gh = grid_handle(grid)
     desc, keep = model_desc(grid, gh; advection, buoyancy, coriolis, closure, tracers, timestepper,
                             boundary_conditions = bcs, kw...)
@@ -451,9 +521,8 @@ function b200_nonhydrostatic_model(; grid, clock = Clock{eltype(grid)}(0, 0, 1),
     handle = ModelHandle(mh[])
     finalizer(h -> ccall((:ob200_model_destroy, lib), Int32, (Ptr{Cvoid},), h.ptr), handle)
 
-    locs = (u = (Face, Center, Center), v = (Center, Face, Center), w = (Center, Center, Face))
-    loc_of(n) = haskey(locs, n) ? locs[n] : (Center, Center, Center)
     libname(n) = n in (:u, :v, :w) ? String(n) : "c$(findfirst(==(n), tracers) - 1)"
+    bcs = NamedTuple{names}(attach_boundary_arrays(bcs[n], tables[n], model_field(mh[], libname(n)), handle) for n in names)
     wrap(n, prefix = "", fbcs = bcs[n]) = Field(loc_of(n), grid; boundary_conditions = fbcs,
                                                 data = wrap_field(FT, grid, loc_of(n), model_field(mh[], prefix * libname(n)), handle))
     velocities = NamedTuple{(:u, :v, :w)}(wrap(n) for n in (:u, :v, :w))

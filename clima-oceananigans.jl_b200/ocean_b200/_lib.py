@@ -79,6 +79,7 @@ SYMBOLS = {
     "ob200_field_get_parent_async": (C.c_int32, [C.c_void_p, C.c_void_p]),
     "ob200_field_device_view": (C.c_int32, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "ob200_fill_halo_regions": (C.c_int32, [C.POINTER(C.c_void_p), C.c_int32]),
+    "ob200_field_set_boundary_values": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p]),
     "ob200_field_reduce": (C.c_int32, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double),
                                        C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
     "ob200_poisson_create": (C.c_int32, [C.c_void_p, C.c_int32, C.POINTER(C.c_void_p)]),

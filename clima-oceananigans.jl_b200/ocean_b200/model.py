@@ -18,11 +18,26 @@ _BCK = {"Periodic": L.BC_PERIODIC, "Flux": L.BC_FLUX, "Value": L.BC_VALUE, "Grad
 
 # ---- boundary conditions (src/BoundaryConditions/boundary_condition.jl) ----------------------
 class BoundaryCondition:
+    """`condition` is None, a number or a 2-D numpy array (getbc(bc::BC{<:Any,<:AbstractArray}, i, j, grid) = bc.condition[i, j]):
+    indexed by the grid's interior indices along the side's two tangential dimensions, Flat counting as 1."""
+
     def __init__(self, kind, condition=None):
         if callable(condition):
             raise ValueError("function-valued boundary conditions cannot cross the C ABI of the B200 "
-                             "architecture (SURVEY.md 8(b)); use constants")
+                             "architecture (SURVEY.md 8(b)); use constants or 2-D arrays")
+        if isinstance(condition, np.ndarray) and condition.ndim != 0 and not _is_real_matrix(condition):
+            raise ValueError(f"an array boundary condition must be a 2-D real numeric array, got a {condition.ndim}-D "
+                             f"{condition.dtype} array")
         self.kind, self.condition = kind, condition
+
+    @property
+    def is_array(self):
+        return isinstance(self.condition, np.ndarray) and self.condition.ndim != 0
+
+
+def _is_real_matrix(a):
+    return (isinstance(a, np.ndarray) and a.ndim == 2 and a.dtype != bool and
+            (np.issubdtype(a.dtype, np.integer) or np.issubdtype(a.dtype, np.floating)))
 
 
 def FluxBoundaryCondition(v):
@@ -51,14 +66,73 @@ def _default_bc(topo, loc, auxiliary=False):
     return BoundaryCondition(None) if auxiliary else BoundaryCondition("Open", None)
 
 
-def _bc_array(grid, loc, user=None, auxiliary=False):
-    arr = (L.BC * 6)()
+def _resolve_bcs(grid, loc, user=None, auxiliary=False):
+    """{side: BoundaryCondition} with the defaults filled in"""
     user = user or {}
-    for s, name in enumerate(_SIDES):
-        bc = user.get(name) or _default_bc(grid.topology[s // 2], loc[s // 2], auxiliary)
+    return {name: user.get(name) or _default_bc(grid.topology[s // 2], loc[s // 2], auxiliary) for s, name in enumerate(_SIDES)}
+
+
+def _bc_array(grid, loc, user=None, auxiliary=False):
+    """the ob200_bc[6] of a field; an array condition crosses as its kind with value 0 and is pushed after creation"""
+    arr = (L.BC * 6)()
+    for s, (name, bc) in enumerate(_resolve_bcs(grid, loc, user, auxiliary).items()):
         arr[s].kind = _BCK[bc.kind]
-        arr[s].value = 0.0 if bc.condition is None else float(bc.condition)
+        arr[s].value = 0.0 if (bc.condition is None or bc.is_array) else float(bc.condition)
     return arr
+
+
+def boundary_values(grid, loc, side, bc):
+    """The table of an array boundary condition `bc` on `side` of a field at `loc` (anything with .topology, .N and .FT): the
+    array cast to the grid's float type, column-major, after checking it against the grid and the side.  No library call.
+    The shape is (N_a, N_b) of the side's two tangential dimensions in x, y, z order, a Flat dimension counting as 1: the
+    reference's BC kernels run over the grid's interior size, not the field's (fill_halo_regions.jl:163-170)."""
+    if side not in _SIDES:
+        raise ValueError(f"unknown side {side!r}; sides are {_SIDES}")
+    s = _SIDES.index(side)
+    d = s // 2
+    if "FullyConnected" in tuple(grid.topology):
+        raise ValueError("array boundary conditions are not supported on a slab-decomposed (FullyConnected) grid")
+    if grid.topology[d] != Bounded:
+        raise ValueError(f"array boundary condition on the {side} side of a {grid.topology[d]} dimension: only Bounded "
+                         "dimensions have boundary conditions of that kind")
+    if bc.kind not in ("Flux", "Value", "Gradient"):
+        raise ValueError(f"array boundary conditions must be Flux, Value or Gradient conditions, not {bc.kind}")
+    if loc[d] == Face:
+        raise ValueError(f"the {side} side of a field located on the {'xyz'[d]}-faces is the impenetrable wall; it takes no "
+                         "array boundary condition")
+    q = bc.condition
+    if not _is_real_matrix(q):
+        raise ValueError("an array boundary condition must be a 2-D real numeric numpy array")
+    shape = tuple(1 if grid.topology[e] == Flat else int(grid.N[e]) for e in range(3) if e != d)
+    if q.shape != shape:
+        raise ValueError(f"the array boundary condition on the {side} side has shape {q.shape}; the grid needs {shape} "
+                         f"(interior size along {', '.join('xyz'[e] for e in range(3) if e != d)}, Flat = 1)")
+    return np.asfortranarray(q, dtype=grid.FT)
+
+
+def _array_tables(grid, loc, bcs):
+    """{side index: table} of every array condition among the resolved `bcs`, checked before any library call"""
+    return {_SIDES.index(n): boundary_values(grid, loc, n, bc) for n, bc in bcs.items() if bc is not None and bc.is_array}
+
+
+def _push_boundary_values(handle, tables):
+    for s, t in tables.items():
+        check(lib.ob200_field_set_boundary_values(handle, s, t.ctypes.data_as(C.c_void_p)))
+
+
+def set_boundary_condition_values(field, side, values):
+    """Replace the values of the array boundary condition on `side` of `field` (a Field or a model field such as
+    model.tracers["b"]), as `bc.condition .= values` in a callback does in the reference.  The copy is ordered after every step
+    enqueued so far, so it takes effect from the next step on.  Raises ValueError before any library call if the side cannot
+    take an array (see boundary_values) or the shape is wrong."""
+    if side not in _SIDES:
+        raise ValueError(f"unknown side {side!r}; sides are {_SIDES}")
+    bc = field.boundary_conditions[side]
+    if not _is_real_matrix(values):
+        raise ValueError("boundary condition values must be a 2-D real numeric numpy array")
+    t = boundary_values(field.grid, field.loc, side, BoundaryCondition(bc.kind, values))
+    _push_boundary_values(field.handle, {_SIDES.index(side): t})
+    field.boundary_conditions[side] = BoundaryCondition(bc.kind, t)
 
 
 # ---- Field (src/Fields/field.jl:16-31) ---------------------------------------------------------
@@ -66,12 +140,16 @@ class Field:
     def __init__(self, loc, grid, boundary_conditions=None, _handle=None, auxiliary=False):
         self.grid, self.loc = grid, tuple(loc)
         self._owned = _handle is None
+        # the resolved boundary conditions; a model sets those of its fields itself
+        self.boundary_conditions = _resolve_bcs(grid, self.loc, boundary_conditions, auxiliary)
         if _handle is None:
+            tables = _array_tables(grid, self.loc, self.boundary_conditions)
             h = C.c_void_p()
             locs = (C.c_int32 * 3)(*[_LOC[l] for l in self.loc])
             check(lib.ob200_field_create(grid.handle, locs, _bc_array(grid, self.loc, boundary_conditions, auxiliary),
                                          C.byref(h)))
             _handle = h
+            _push_boundary_values(h, tables)
         self.handle = _handle
         ps = (C.c_int32 * 3)()
         check(lib.ob200_field_parent_size(self.handle, ps))
@@ -639,6 +717,9 @@ class NonhydrostaticModel:
             d.g_hat[k] = float(g_hat[k])
         d.ntracers = len(tracers)
         bcs = boundary_conditions or {}
+        # array conditions: checked here, pushed once the model exists (set_model's update_state! then fills the halos with them)
+        resolved = {n: _resolve_bcs(grid, loc, bcs.get(n)) for n, loc in zip(names, locs)}
+        tables = {n: _array_tables(grid, loc, resolved[n]) for n, loc in zip(names, locs)}
         for q, (n, loc) in enumerate(zip(names, locs)):
             arr = _bc_array(grid, loc, bcs.get(n))
             for s in range(6):
@@ -667,6 +748,9 @@ class NonhydrostaticModel:
         self.velocities = {n: self._field(n, n, locs[i]) for i, n in enumerate("uvw")}
         self.tracers = {n: self._field(f"c{k}", n, (Center,) * 3) for k, n in enumerate(tracers)}
         self.fields = {**self.velocities, **self.tracers}
+        for n, f in self.fields.items():
+            f.boundary_conditions = resolved[n]
+            _push_boundary_values(f.handle, tables[n])
         self.pressures = {"pNHS": self._field("pNHS", "pNHS", (Center,) * 3)}
         if grid.topology[2] != Flat:
             self.pressures["pHY′"] = self._field("pHY", "pHY", (Center,) * 3)

@@ -198,6 +198,16 @@ int32_t ob200_field_device_view(const ob200_field* f, void** base, int64_t offse
                                 int64_t strides[3]);
 /* fill_halo_regions!(fields) BoundaryConditions/fill_halo_regions.jl:34-82 */
 int32_t ob200_fill_halo_regions(ob200_field* const* fields, int32_t n);
+/* FluxBoundaryCondition(Q) / ValueBoundaryCondition(Q) / GradientBoundaryCondition(Q) with a 2-D array Q (getbc(bc, i, j, grid)
+ * = bc.condition[i, j], BoundaryConditions/boundary_condition.jl): the condition of `side` becomes the array `values` (grid float
+ * type, column-major, (N_a, N_b) of the grid's two tangential dimensions in x, y, z order, Flat = 1: Q[j, k] on x sides, Q[i, k]
+ * on y sides, Q[i, j] on z sides), or the constant `value` again when values == NULL; kind must be Flux, Value or Gradient.
+ * The field owns the device copy.  The copy is enqueued on the library stream, after every step enqueued so far, so calling
+ * this between steps (model fields through ob200_model_field) varies the condition in time from the next step on.  Fails for a
+ * Periodic, Flat or FullyConnected side, kind Open / None, the side normal to a Face location (u on x sides, v on y, w on z:
+ * the impenetrable wall) and any grid with a FullyConnected (slab-decomposed) dimension.  Array Flux conditions of a model's
+ * prognostic fields are added by one boundary-plane pass per Bounded dimension after the tendency kernels. */
+int32_t ob200_field_set_boundary_values(ob200_field* f, int32_t side, const void* values);
 /* device reductions over the interior (Simulations NaNChecker / wizard / diagnostics) */
 int32_t ob200_field_reduce(const ob200_field* f, double* sum, double* sumsq, double* maxabs,
                            int32_t* has_nan);
@@ -266,7 +276,8 @@ int64_t ob200_debug_cached_tensor_maps(void);
 /* force the general kernels (on = 0) instead of the specialised headline kernels */
 int32_t ob200_model_use_fast_kernels(ob200_model* m, int32_t on);
 /* per-phase CUDA-event timing on the library stream: phases "tendency" (one event pair per
- * tendency-kernel launch), "poisson", "halo", "pressure_correct", "hydrostatic" */
+ * tendency-kernel launch), "poisson", "halo", "pressure_correct", "hydrostatic", "boundary_flux" (the array Flux pass, one pair per
+ * launch, also inside "tendency") */
 int32_t ob200_profile_enable(int32_t on);
 int32_t ob200_profile_reset(void);
 int32_t ob200_profile_query(const char* phase, double* total_ms, int64_t* count);
