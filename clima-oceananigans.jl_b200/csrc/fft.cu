@@ -395,6 +395,10 @@ __global__ void thomas_kernel(int Nx, int Ny, int Nz, const double* a, const dou
         if (k == Nz) return -1 / dzF[Nz] - dzC[Nz] * lam;
         return -(1 / dzF[k + 1] + 1 / dzF[k]) - dzC[k] * lam;
     };
+    // The reference's pivot guard |beta| > 10 eps is absolute.  For the solver's own columns (ONTHEFLY) beta has units of
+    // 1/length and the lowest horizontal mode's last pivot is about lam * H: in Float32 that falls below 10 eps once Lx
+    // reaches ~100 km, and the `break` would return a wrong column.  There the guard is relative to the row's diagonal
+    // (scale free); the singular mean column is pinned explicitly below.  Caller-supplied coefficients keep the reference's.
     const double eps10 = 10 * (sizeof(FT) == 4 ? 1.1920928955078125e-07 : 2.220446049250313e-16);
     double beta = diag(1);
     VT f1 = f[col];
@@ -412,7 +416,7 @@ __global__ void thomas_kernel(int Nx, int Ny, int Nz, const double* a, const dou
         // horizontal-mean column of the Neumann problem is ALWAYS pinned at its last row (its pivot is zero in exact
         // arithmetic, rounding noise otherwise): the constant it leaves open is removed with the mean, and the solution no
         // longer depends on noise / noise or on the solver's history.
-        if (!(fabs(beta) > eps10) || (ONTHEFLY && k == Nz && lam == 0.0)) {
+        if (!(fabs(beta) > (ONTHEFLY ? eps10 * fabs(bk) : eps10)) || (ONTHEFLY && k == Nz && lam == 0.0)) {
             if (ONTHEFLY)
                 for (int q = k; q <= Nz; ++q) phi[col + (q - 1) * pl] = f[col + (q - 1) * pl];
             break;
