@@ -793,6 +793,8 @@ struct ob200_model {
     std::unique_ptr<ob200_field> nue;               // SmagorinskyLilly / AMD eddy viscosity (diffusivity_fields.νₑ)
     std::vector<std::unique_ptr<ob200_field>> kappae;     // AMD eddy diffusivities (diffusivity_fields.κₑ), one per tracer
     std::unique_ptr<ob200_field> ivd_scratch;             // Thomas scratch of the vertically implicit diffusion step
+    std::vector<std::unique_ptr<ob200_field>> bg;         // background_fields per prognostic field (null: none)
+    std::unique_ptr<ob200_field> bg_zero;                 // the missing background velocities when another one is given
     std::unique_ptr<ob200_poisson> solver;
     std::vector<void*> owned;
     Phys<float> P32;
@@ -918,6 +920,8 @@ static void build_phys(ob200_model* m) {
         if (r.md >= 0) r.M = table(F.mask, forcing_table_length(m->grid->desc, q, r.md));
         if (r.td >= 0) r.T = table(F.target, forcing_table_length(m->grid->desc, q, r.td));
     }
+    for (int q = 0; q < 3 + 8; ++q) P.bg[q] = q < m->nf && m->bg[q] ? m->bg[q]->template p0<FT>() : nullptr;
+    for (int d = 0; d < 3; ++d) P.bgU[d] = P.bg[d] ? P.bg[d] : (m->bg_zero ? m->bg_zero->template p0<FT>() : nullptr);
 }
 
 extern "C" int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model** out) {
@@ -986,6 +990,19 @@ extern "C" int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model*
     if (desc->closure == OB200_CLOSURE_AMD)
         for (int t = 0; t < desc->ntracers; ++t) m->kappae.emplace_back(make_field(m->grid, ccc, nullptr, false));
     if (desc->closure_vertically_implicit) m->ivd_scratch.reset(make_field(m->grid, ccc, nullptr, false));
+    // background_fields: model-owned copies of the host's parent arrays (halos included, never filled)
+    m->bg.resize(m->nf);
+    for (int q = 0; q < 3 + OB200_MAX_TRACERS; ++q) {
+        if (!desc->background[q]) continue;
+        if (q >= m->nf) throw Error("background of prognostic field " + std::to_string(q) + ": the model has no such field");
+        int32_t loc[3] = {OB200_CENTER, OB200_CENTER, OB200_CENTER};
+        if (q < 3) loc[q] = OB200_FACE;
+        m->bg[q].reset(make_field(m->grid, loc, nullptr, false));
+        if (m->grid->ftype == OB200_F32) field_set_parent<float>(m->bg[q].get(), desc->background[q], true);
+        else field_set_parent<double>(m->bg[q].get(), desc->background[q], true);
+    }
+    if ((m->bg[0] || m->bg[1] || m->bg[2]) && !(m->bg[0] && m->bg[1] && m->bg[2]))
+        m->bg_zero.reset(make_field(m->grid, ccc, nullptr, false));       // zeroed on creation
     ob200_poisson* s = nullptr;
     if (ob200_poisson_create(m->grid, desc->pressure_solver, &s)) throw Error(ob::g_err);
     m->solver.reset(s);
@@ -993,6 +1010,7 @@ extern "C" int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model*
     else build_phys<double>(m.get());
     for (int d = 0; d < 3; ++d) for (int l = 0; l < 2; ++l) m->desc.weno_coeff[d][l] = nullptr;
     for (ob200_forcing& F : m->desc.forcing) F.mask = F.target = nullptr;      // borrowed host tables: copied to the device
+    for (const void*& p : m->desc.background) p = nullptr;
     *out = m.release();
     if (ob200_model_update_state(*out)) { delete *out; *out = nullptr; throw Error(ob::g_err); }
     API_END
@@ -1019,6 +1037,7 @@ extern "C" int32_t ob200_model_field(ob200_model* m, const char* name, ob200_fie
     else if (s == "pHY") f = m->pHY.get();
     else if (s.rfind("Gn_", 0) == 0) { int q = idx(s.substr(3)); if (q >= 0) f = m->Gn[q].get(); }
     else if (s.rfind("Gm_", 0) == 0) { int q = idx(s.substr(3)); if (q >= 0) f = m->Gm[q].get(); }
+    else if (s.rfind("bg_", 0) == 0) { int q = idx(s.substr(3)); if (q >= 0) f = m->bg[q].get(); }
     else { int q = idx(s); if (q >= 0) f = m->F[q].get(); }
     if (!f) throw Error("no such model field: " + s);
     *out = f;
@@ -1269,7 +1288,22 @@ static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
                 launch_tendency_general<FT>(P, q, U, ff.state[q], pHY, b, ff.fbc[q], ff.Gn[q], ff.Gm[q], nullptr, none, true);
             ff.accumulate = true;
         }
-        if (m->halo_pending) {
+        // background terms of the fused fields: - div(U_bg, ψ) - div(U, ψ_bg) alone into G^n (onto the closure's part), for the
+        // accumulate form to add the rest; it reads the velocities' y halos, so after the exchange has landed.  The variant
+        // without a tracer has no accumulate form: that model takes the per-field kernels
+        bool bg = false;
+        for (int q = 0; q < 3 + std::min(m->nf - 3, 1); ++q) bg = bg || has_background(P, q);
+        if (bg && m->nf > 3 && fz::supported<FT>(P, m->nf) && background_only_supported<FT>(P)) {
+            model_halo_join(m);
+            const Substep<FT> none{SUB_NONE, FT(0), FT(0), FT(0)};
+            for (int q = 0; q < 4; ++q)
+                launch_tendency_general<FT>(P, q, U, ff.state[q], pHY, b, ff.fbc[q], ff.Gn[q], ff.Gm[q], nullptr, none, false,
+                                            ff.accumulate ? 2 : 1);
+            ff.gn_terms = true;
+        }
+        if (bg && !ff.gn_terms) {
+            // no fused launch: the per-field kernels below add the background terms themselves
+        } else if (m->halo_pending) {
             // the neighbour exchange of the previous stage is still in flight on the halo stream: tile rows that read only rows
             // this rank owns go first, the boundary tile rows once the exchange has landed
             first = fz::launch<FT>(P, ff, 1);

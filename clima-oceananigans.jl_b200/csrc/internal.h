@@ -61,10 +61,15 @@ template <class FT> void launch_boundary_fluxes(const GridD<FT>& g, int d, const
 template <class FT>
 void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
                              const FT* pHY, const Buoy<FT>& b, const FluxBC<FT>& fbc, FT* Gn,
-                             const FT* Gm, FT* psi_new, const Substep<FT>& ss, bool closure_only = false);
+                             const FT* Gm, FT* psi_new, const Substep<FT>& ss, bool closure_only = false,
+                             int background_only = 0);
 // true if launch_tendency_general(..., closure_only = true) is available for this model (3-D grid)
 template <class FT> bool closure_only_supported(const Phys<FT>& P);
-// fast path (all non-Flat dimensions periodic, regular, WENO5 uniform, no closure, optional FPlane, field not forced):
+// background_only = 1 / 2: G^n = / += - div(U_bg, ψ) - div(U, ψ_bg) alone (zero for a field without background terms), for the
+// fused kernel's accumulate form; true if available for this model (3-D grid, an advection scheme)
+template <class FT> bool background_only_supported(const Phys<FT>& P);
+// fast path (all non-Flat dimensions periodic, regular, WENO5 uniform, no closure, optional FPlane, field not forced and
+// without background terms):
 // the TMA-staged kernel on 3-D grids, the direct-load kernel on 2-D grids; returns false if the configuration is not
 // covered
 template <class FT>
@@ -86,7 +91,7 @@ struct FusedFields {
     Substep<FT> ss;
     FluxBC<FT> fbc[FUSED_MAXF];      // constant Flux boundary conditions (Bounded z variant)
     bool accumulate = false;         // G^n already holds the closure's part (launch_tendency_general closure_only): add to it
-    bool forcing_in_gn = false;      // G^n already holds the forcing (tendency_fused.cu launch_frc): add to it
+    bool gn_terms = false;           // G^n already holds precomputed terms (background pass, relaxation pass): add to it
 };
 // part: 0 = every tile; 1 = the tile rows whose stencils stay inside the rows this rank owns along a slab-decomposed y (they
 // need no neighbour data); 2 = the remaining (boundary) tile rows.  Returns the number of fields handled, 0 = not applicable.

@@ -352,11 +352,12 @@ struct TendArgs {
     FluxBC<FT> fbc;
     int comp;
     int closure_only;      // G^n = -div(tau) / -div(q) of the closure alone (the fused kernel adds the rest, tendency_fused.cu)
+    int bg_acc;            // background-only mode (tendency_shared_kernel BG = 2): add to G^n instead of overwriting it
 };
 
 // COMP (0, 1, 2 = u, v, w; 3 = any tracer) is a template parameter so that the staggering flags of every operator in
 // the inlined call tree (locations, which spacings and areas, which directions interpolate) are compile-time constants
-template <class FT, int COMP>
+template <class FT, int COMP, bool BG = false>
 __global__ void __launch_bounds__(128) tendency_general_kernel(const __grid_constant__ Phys<FT> P, const __grid_constant__ TendArgs<FT> A) {
     const GridD<FT>& g = P.g;
     int i = 1 + blockIdx.x * blockDim.x + threadIdx.x;
@@ -367,7 +368,7 @@ __global__ void __launch_bounds__(128) tendency_general_kernel(const __grid_cons
     q.i[0] = i; q.i[1] = j; q.i[2] = k;
     q.p = i * g.st[0] + j * g.st[1] + k * g.st[2];
     const FT* U[3] = {A.U[0], A.U[1], A.U[2]};
-    FT G = tendency(P, COMP == 3 ? A.comp : COMP, U, A.psi, A.pHY, A.b, q);
+    FT G = tendency<FT, BG>(P, COMP == 3 ? A.comp : COMP, U, A.psi, A.pHY, A.b, q);
     // apply_x/y/z_bcs! (apply_flux_bcs.jl:35-160): constant Flux BCs of this field
     int l[3] = {OB_C, OB_C, OB_C};
     if (COMP < 3) l[COMP] = OB_F;
@@ -460,8 +461,10 @@ template void launch_boundary_fluxes<double>(const GridD<double>&, int, const Bo
 // constants, so that after inlining every run-time scheme / topology / regularity branch of the operator tree folds away.
 // CO = 1: closure-only (TendArgs::closure_only) as a compile-time flag, so that the advection operators are not part of the
 // kernel at all, with 4 resident blocks per SM (64 registers; C3 with AMD: 3 blocks 64.3, 4 blocks 60.5, 5 blocks 62.0 ms per step)
-template <class FT, int COMP, int SPEC, int CO = 0>
-__global__ void __launch_bounds__(256, (CO ? 4 : 3)) tendency_shared_kernel(const __grid_constant__ Phys<FT> Pin, const __grid_constant__ TendArgs<FT> A, int Kc) {
+// BG = 1: every face flux also carries the background fluxes F(U_bg, ψ) + F(U, ψ_bg) (Phys::bg, bgU).  BG = 2: background-only,
+// G^n = (or +=, TendArgs::bg_acc) -div of those fluxes alone, the analogue of CO for the fused kernel's accumulate form
+template <class FT, int COMP, int SPEC, int CO = 0, int BG = 0>
+__global__ void __launch_bounds__(256, (CO || BG == 2 ? 4 : 3)) tendency_shared_kernel(const __grid_constant__ Phys<FT> Pin, const __grid_constant__ TendArgs<FT> A, int Kc) {
     Phys<FT> Pl;
     if constexpr (SPEC == 1) {
         Pl = Pin;
@@ -489,7 +492,9 @@ __global__ void __launch_bounds__(256, (CO ? 4 : 3)) tendency_shared_kernel(cons
     const bool need_x = outy && i <= g.N[0] + 1, need_y = outx && j <= g.N[1] + 1;
     const FT* U[3] = {A.U[0], A.U[1], A.U[2]};
     const int comp = COMP == 3 ? A.comp : COMP;
-    const bool visc = P.closure != CLO_NONE, adv = !CO && P.scheme != ADV_NONE && !A.closure_only;
+    const bool visc = BG != 2 && P.closure != CLO_NONE, adv = !CO && BG != 2 && P.scheme != ADV_NONE && !A.closure_only;
+    const FT* const* Ub = Pin.bgU;
+    const FT* psib = BG ? Pin.bg[comp] : nullptr;
     const FT kappa = COMP == 3 ? Pin.kappa[comp - 3] : FT(0);
     const FT* kappae = COMP == 3 ? Pin.kappae[comp - 3] : nullptr;
     auto face = [&](int d, Pt q) -> FT {       // area-weighted advective + viscous / diffusive flux at q along d
@@ -503,19 +508,36 @@ __global__ void __launch_bounds__(256, (CO ? 4 : 3)) tendency_shared_kernel(cons
         }
         return f;
     };
+    // the same with the background fluxes F(U_bg, ψ) + F(U, ψ_bg) (BG != 0).  A separate lambda, so that the BG = 0 kernels keep
+    // their code; always inlined, since out of line the call would keep the physics descriptor on the stack
+    auto face_bg = [&](int d, Pt q) __attribute__((always_inline)) -> FT {
+        FT f = FT(0);
+        if (COMP < 3) {
+            if (adv) f = momentum_flux(P, d, B, U[d], A.psi, q);
+            if (Ub[0]) f = f + momentum_flux(P, d, B, Ub[d], A.psi, q);
+            if (psib) f = f + momentum_flux(P, d, B, U[d], psib, q);
+            if (visc) f = f + viscous_Aflux(P, B, d, U, q);
+        } else {
+            if (adv) f = tracer_flux(P, d, U[d], A.psi, q);
+            if (Ub[0]) f = f + tracer_flux(P, d, Ub[d], A.psi, q);
+            if (psib) f = f + tracer_flux(P, d, U[d], psib, q);
+            if (visc) f = f + diffusive_Aflux(P, d, kappa, A.psi, q, kappae);
+        }
+        return f;
+    };
     Pt q;
     q.i[0] = i; q.i[1] = j; q.i[2] = k0;
     q.p = i * g.st[0] + j * g.st[1] + k0 * g.st[2];
     FT Fz_carry = FT(0);
-    if (cell) Fz_carry = face(2, ZLOW ? sh(g, q, 2, -1) : q);
+    if (cell) Fz_carry = BG ? face_bg(2, ZLOW ? sh(g, q, 2, -1) : q) : face(2, ZLOW ? sh(g, q, 2, -1) : q);
     for (int k = k0; k <= k1; ++k) {
         const int buf = (k - k0) & 1;
         FT Fx = FT(0), Fy = FT(0), dFz = FT(0);
-        if (need_x) Fx = face(0, q);
-        if (need_y) Fy = face(1, q);
+        if (need_x) Fx = BG ? face_bg(0, q) : face(0, q);
+        if (need_y) Fy = BG ? face_bg(1, q) : face(1, q);
         sF[buf][ty][tx] = Fy;
         if (cell) {
-            FT Fz_new = face(2, ZLOW ? q : sh(g, q, 2, 1));
+            FT Fz_new = BG ? face_bg(2, ZLOW ? q : sh(g, q, 2, 1)) : face(2, ZLOW ? q : sh(g, q, 2, 1));
             dFz = Fz_new - Fz_carry;
             Fz_carry = Fz_new;
         }
@@ -528,7 +550,9 @@ __global__ void __launch_bounds__(256, (CO ? 4 : 3)) tendency_shared_kernel(cons
             int l[3] = {OB_C, OB_C, OB_C};
             if (COMP < 3) l[COMP] = OB_F;
             FT G = -((1 / volume(g, q, l[0], l[1], l[2])) * ((dFx + dFy) + dFz));
-            if (CO || A.closure_only) {
+            if (BG == 2) {
+                A.Gn[q.p] = A.bg_acc ? A.Gn[q.p] + G : G;
+            } else if (CO || A.closure_only) {
                 A.Gn[q.p] = G;
             } else {
             if (COMP == 0) {
@@ -580,20 +604,31 @@ bool closure_only_supported(const Phys<FT>& P) {
 }
 template bool closure_only_supported<float>(const Phys<float>&);
 template bool closure_only_supported<double>(const Phys<double>&);
+template <class FT>
+bool background_only_supported(const Phys<FT>& P) {
+    if (P.scheme == ADV_NONE) return false;
+    for (int d = 0; d < 3; ++d) if (P.g.topo[d] == OB_FLAT || P.g.N[d] < 2) return false;
+    return true;
+}
+template bool background_only_supported<float>(const Phys<float>&);
+template bool background_only_supported<double>(const Phys<double>&);
 
 template <class FT>
 void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
                              const FT* pHY, const Buoy<FT>& b, const FluxBC<FT>& fbc, FT* Gn,
-                             const FT* Gm, FT* psi_new, const Substep<FT>& ss, bool closure_only) {
+                             const FT* Gm, FT* psi_new, const Substep<FT>& ss, bool closure_only, int background_only) {
     TendArgs<FT> A;
     for (int d = 0; d < 3; ++d) A.U[d] = U[d];
     A.psi = psi; A.pHY = pHY; A.b = b; A.Gn = Gn; A.Gm = Gm; A.psi_new = psi_new;
-    A.ss = ss; A.fbc = fbc; A.comp = comp; A.closure_only = closure_only ? 1 : 0;
+    A.ss = ss; A.fbc = fbc; A.comp = comp; A.closure_only = closure_only ? 1 : 0; A.bg_acc = background_only == 2 ? 1 : 0;
+    const bool bg = has_background(P, comp);
     // shared-face variant: 3-D grids (every direction has two faces to pair) with a halo wide enough for the one
     // extra face position per direction
     bool shared = P.scheme != ADV_NONE || P.closure != CLO_NONE;
     for (int d = 0; d < 3; ++d) shared = shared && P.g.topo[d] != OB_FLAT && P.g.N[d] >= 2;
     if (closure_only && !shared) throw Error("closure-only tendencies need the shared-face kernel (3-D grid)");
+    if (background_only && !(shared && background_only_supported(P)))
+        throw Error("background-only tendencies need the shared-face kernel (3-D grid, an advection scheme)");
     const bool spec = P.g.topo[0] == OB_PERIODIC && P.g.topo[1] == OB_PERIODIC && P.g.topo[2] == OB_BOUNDED &&
                       P.g.regular[0] && P.g.regular[1] && P.scheme == ADV_WENO5 && P.buffer == 2 && !P.tilted && !P.vitd &&
                       !P.wc[0][0] && !P.wc[0][1] && !P.wc[1][0] && !P.wc[1][1];
@@ -602,6 +637,8 @@ void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], 
         dim3 bs(32, 8, 1), gs(cdiv(P.g.N[0], 31), cdiv(P.g.N[1], 7), cdiv(P.g.N[2], Kc));
         switch (comp) {
 #define SHK(C, S) do { if (closure_only) tendency_shared_kernel<FT, C, S, 1><<<gs, bs, 0, stream()>>>(P, A, Kc); \
+                       else if (background_only) tendency_shared_kernel<FT, C, S, 0, 2><<<gs, bs, 0, stream()>>>(P, A, Kc); \
+                       else if (bg) tendency_shared_kernel<FT, C, S, 0, 1><<<gs, bs, 0, stream()>>>(P, A, Kc); \
                        else tendency_shared_kernel<FT, C, S, 0><<<gs, bs, 0, stream()>>>(P, A, Kc); } while (0)
             case 0: if (spec) SHK(0, 1); else SHK(0, 0); break;
             case 1: if (spec) SHK(1, 1); else SHK(1, 0); break;
@@ -614,20 +651,23 @@ void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], 
     }
     dim3 blk(32, 4, 1);
     dim3 grd(cdiv(P.g.N[0], 32), cdiv(P.g.N[1], 4), P.g.N[2]);
+#define GK(C) do { if (bg) tendency_general_kernel<FT, C, true><<<grd, blk, 0, stream()>>>(P, A); \
+                   else tendency_general_kernel<FT, C><<<grd, blk, 0, stream()>>>(P, A); } while (0)
     switch (comp) {
-        case 0: tendency_general_kernel<FT, 0><<<grd, blk, 0, stream()>>>(P, A); break;
-        case 1: tendency_general_kernel<FT, 1><<<grd, blk, 0, stream()>>>(P, A); break;
-        case 2: tendency_general_kernel<FT, 2><<<grd, blk, 0, stream()>>>(P, A); break;
-        default: tendency_general_kernel<FT, 3><<<grd, blk, 0, stream()>>>(P, A); break;
+        case 0: GK(0); break;
+        case 1: GK(1); break;
+        case 2: GK(2); break;
+        default: GK(3); break;
     }
+#undef GK
     OB_LAUNCH_CHECK();
 }
 template void launch_tendency_general<float>(const Phys<float>&, int, const float* const[3], const float*,
                                              const float*, const Buoy<float>&, const FluxBC<float>&, float*,
-                                             const float*, float*, const Substep<float>&, bool);
+                                             const float*, float*, const Substep<float>&, bool, int);
 template void launch_tendency_general<double>(const Phys<double>&, int, const double* const[3], const double*,
                                               const double*, const Buoy<double>&, const FluxBC<double>&, double*,
-                                              const double*, double*, const Substep<double>&, bool);
+                                              const double*, double*, const Substep<double>&, bool, int);
 
 // =============================================================================================
 // pressure source term: rhs = div(U*) / dt (x Δzᶜ for the tridiagonal solver)

@@ -77,7 +77,18 @@ struct Phys {
     FT ghat[3];
     int ntr;
     Relax<FT> frc[3 + 8];            // forcing of u, v, w, tracers (on = 0: none)
+    // background_fields (background_fields.jl): bg[q] = the background of prognostic field q (Julia-(0,0,0) pointer, halos
+    // as given by the host, never filled) or null; bgU = the background velocities, all null without any, a missing one
+    // pointing to a zeroed field (a ZeroField's fluxes are exactly zero)
+    const FT* bg[3 + 8];
+    const FT* bgU[3];
 };
+
+// whether field `comp` has a non-zero background term - div(U_bg, ψ) - div(U, ψ_bg)
+template <class FT>
+__host__ __device__ inline bool has_background(const Phys<FT>& P, int comp) {
+    return P.scheme != ADV_NONE && (P.bgU[0] || P.bg[comp]);
+}
 
 struct Pt {
     long long p;   // linear offset from the Julia-(0,0,0) pointer
@@ -790,18 +801,26 @@ OBD void amd_cell(const Phys<FT>& P, const Buoy<FT>& B, const FT* const* U, int 
 }
 
 // ---- tendencies: nonhydrostatic_tendency_kernel_functions.jl:44-232 (term order kept) -------
-// comp 0,1,2 = u,v,w ; comp >= 3 = tracer (comp-3)
-template <class FT>
+// comp 0,1,2 = u,v,w ; comp >= 3 = tracer (comp-3).  BG: the two background terms after the first advection term
+template <class FT, bool BG = false>
 OBD FT tendency(const Phys<FT>& P, int comp, const FT* const* U, const FT* psi, const FT* pHY,
                 const Buoy<FT>& b, Pt q) {
     const GridD<FT>& g = P.g;
     if (comp >= 3) {
         FT G = -div_Uc(P, U, psi, q);
+        if constexpr (BG) {          // - div_Uc(U_bg, c) - div_Uc(U, c_bg)   (:225-226)
+            if (P.bgU[0]) G = G - div_Uc(P, P.bgU, psi, q);
+            if (P.bg[comp]) G = G - div_Uc(P, U, P.bg[comp], q);
+        }
         G = G - div_q(P, P.kappa[comp - 3], psi, q, P.kappae[comp - 3]);
         if (P.frc[comp].on) G = G + relaxation(P.frc[comp], q.i[0], q.i[1], q.i[2], psi[q.p]);     // + forcing (:231)
         return G;
     }
     FT G = -div_Uu(P, comp, U, psi, q);
+    if constexpr (BG) {              // - div_𝐯u(U_bg, u) - div_𝐯u(U, u_bg)   (:62-63, :119-120, :173-174)
+        if (P.bgU[0]) G = G - div_Uu(P, comp, P.bgU, psi, q);
+        if (P.bg[comp]) G = G - div_Uu(P, comp, U, P.bg[comp], q);
+    }
     if (comp == 0) {
         if (P.fplane) {          // x_f_cross_U = -f ℑxyᶠᶜᵃ(v) = -f ℑyᵃᶜᵃ(ℑxᶠᵃᵃ v)   (f_plane.jl:42)
             FT a0 = IF(g, U[1], q, 0);

@@ -143,7 +143,7 @@ template <class FT>
 bool launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
                           const FT* pHY, FT* Gn, const FT* Gm, FT* psi_new, const Substep<FT>& ss) {
     const GridD<FT>& g = P.g;
-    if (P.frc[comp].on) return false;          // forced fields run on the general kernels
+    if (P.frc[comp].on || has_background(P, comp)) return false;      // forced fields and backgrounds: general kernels
     if (P.scheme != ADV_WENO5 || P.closure != CLO_NONE || P.tilted) return false;
     bool hasz = g.topo[2] != OB_FLAT;
     if (g.topo[0] != OB_PERIODIC || (g.topo[1] != OB_PERIODIC && g.topo[1] != OB_COMM) || (hasz && g.topo[2] != OB_PERIODIC)) return false;

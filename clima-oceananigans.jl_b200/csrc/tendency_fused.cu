@@ -533,10 +533,10 @@ static bool part_applicable(int Ny, int part) {
     return nty - nb_hi - 1 >= 1 && R >= HALO;
 }
 
-// Relaxation forcing of the fused fields as a pointwise pass into G^n (G^n = F, or G^n += F over the closure's part), for the
-// accumulate instantiations to add the rest: the forced FP64 variants with a tracer that would spill with the term in the
-// epilogue (launch_frc).  The accumulate form adds G^n of EVERY field, so without the closure's part the unforced fields'
-// G^n are cleared here
+// Relaxation forcing of the fused fields as a pointwise pass into G^n (G^n = F, or G^n += F over the closure's part and / or
+// the background terms), for the accumulate instantiations to add the rest: the forced FP64 variants with a tracer that would
+// spill with the term in the epilogue (launch_frc).  The accumulate form adds G^n of EVERY field, so without precomputed terms
+// the unforced fields' G^n are cleared here
 template <class FT>
 struct RelaxPass {
     int nf, acc;
@@ -633,14 +633,15 @@ static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part
 template <class FT, bool ZW, int ZT, int NT, int R, bool FRC>
 static bool launch_gm(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
     const bool has_gm = a.ss.mode == SUB_RK3 || a.ss.mode == SUB_AB2;
-    // the accumulate form (closure's part and / or the forcing precomputed into G^n) exists for the variants with a tracer
+    // the accumulate form (closure's part, backgrounds and / or the forcing precomputed into G^n) exists for the variants with
+    // a tracer
     if constexpr (NT == 1) {
-        if (a.accumulate || a.forcing_in_gn) {
+        if (a.accumulate || a.gn_terms) {
             if (has_gm) return launch_variant<FT, ZW, ZT, NT, true, true, R, FRC>(P, a, part);
             return launch_variant<FT, ZW, ZT, NT, false, true, R, FRC>(P, a, part);
         }
     } else {
-        if (a.accumulate || a.forcing_in_gn) return false;
+        if (a.accumulate || a.gn_terms) return false;
     }
     if (has_gm) return launch_variant<FT, ZW, ZT, NT, true, false, R, FRC>(P, a, part);
     return launch_variant<FT, ZW, ZT, NT, false, false, R, FRC>(P, a, part);
@@ -662,7 +663,7 @@ static bool launch_frc(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
         if (!part_applicable<R>(g.N[1], part)) return false;
         if (part != 2) {               // once per stage: before the first (or the only) part
             RelaxPass<FT> r;
-            r.nf = NF; r.acc = a.accumulate ? 1 : 0;
+            r.nf = NF; r.acc = (a.accumulate || a.gn_terms) ? 1 : 0;
             for (int f = 0; f < NF; ++f) { r.psi[f] = a.state[f]; r.Gn[f] = a.Gn[f]; r.frc[f] = P.frc[f]; }
             r.sy = g.st[1]; r.sz = g.st[2];
             for (int d = 0; d < 3; ++d) r.N[d] = g.N[d];
@@ -671,7 +672,7 @@ static bool launch_frc(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
             OB_LAUNCH_CHECK();
         }
         FusedFields<FT> b = a;
-        b.forcing_in_gn = true;
+        b.gn_terms = true;
         return launch_gm<FT, ZW, ZT, NT, R, false>(P, b, part);
     }
 }

@@ -149,6 +149,7 @@ struct ModelDesc
     amd_Cnu::Float64; amd_Ckappa::NTuple{MAX_TRACERS,Float64}; amd_Cb::Float64; amd_has_Cb::Int32
     closure_vertically_implicit::Int32
     forcing::NTuple{3 + MAX_TRACERS, ForcingDesc}
+    background::NTuple{3 + MAX_TRACERS, Ptr{Cvoid}}
 end
 
 topo_code(::Type{Periodic}) = Int32(0); topo_code(::Type{Bounded}) = Int32(1); topo_code(::Type{Flat}) = Int32(2)
@@ -431,12 +432,44 @@ function forcing_desc(forcing, grid, names)
     return descs, keep
 end
 
+# ---- background_fields (Models/NonhydrostaticModels/background_fields.jl) tabulated over each field's parent ----------------
+# The reference's own regularize_background_field builds the FunctionField (a function, or a BackgroundField with parameters) on
+# the CPU twin of the grid; its value at every parent index, halos included, crosses the ABI as a parent array of the grid's float
+# type.  Sampled once, at the clock time of construction: a time-dependent background is advanced by the caller through the model
+# field "bg_<name>", wrapped as `model.auxiliary_fields.b200_background_fields.<name>` (set! on it writes the parent).
+const bg_regularize = Oceananigans.Models.NonhydrostaticModels.regularize_background_field
+function background_table(bf, grid, loc, clock)
+    cpu_grid = Oceananigans.Grids.on_architecture(CPU(), grid)
+    f = bf isa Oceananigans.Fields.AbstractField ? bf :
+        (bf isa Function || bf isa Oceananigans.Models.NonhydrostaticModels.BackgroundField) ?
+        bg_regularize(loc..., bf, cpu_grid, clock) :
+        throw(ArgumentError("B200(): a background field must be a function, a BackgroundField or a field; got $(typeof(bf))"))
+    FT = eltype(grid)
+    ranges = ntuple(3) do d
+        N, H = size(grid, d), halo_size(grid)[d]
+        topology(grid, d) === Flat ? (1:1) : ((1 - H):(N + H + (loc[d] === Face && topology(grid, d) === Bounded ? 1 : 0)))
+    end
+    return FT[f[i, j, k] for i in ranges[1], j in ranges[2], k in ranges[3]]
+end
+function background_desc(background_fields, grid, names, clock)
+    for n in keys(background_fields)
+        n in names || throw(ArgumentError("background field name $n is not one of the model's fields $names"))
+    end
+    locs = (u = (Face, Center, Center), v = (Center, Face, Center), w = (Center, Center, Face))
+    tabs = Dict(n => background_table(background_fields[n], grid, haskey(locs, n) ? locs[n] : (Center, Center, Center), clock)
+                for n in keys(background_fields))
+    ptrs = ntuple(3 + MAX_TRACERS) do q
+        q <= length(names) && haskey(tabs, names[q]) ? Ptr{Cvoid}(pointer(tabs[names[q]])) : Ptr{Cvoid}(C_NULL)
+    end
+    return ptrs, collect(values(tabs))
+end
+
 "Translate the model configuration into ob200_model_desc; everything outside the supported set is an ArgumentError."
 function model_desc(grid, gh; advection, buoyancy, coriolis, closure, tracers, timestepper, boundary_conditions, χ = 0.1,
                     stokes_drift = nothing, forcing = NamedTuple(), background_fields = NamedTuple(), particles = nothing,
-                    immersed_boundary = nothing)
-    isnothing(stokes_drift) && isempty(background_fields) && isnothing(particles) && isnothing(immersed_boundary) ||
-        throw(ArgumentError("B200(): stokes_drift, background_fields, particles and immersed boundaries are not supported"))
+                    immersed_boundary = nothing, clock = Clock{eltype(grid)}(0, 0, 1))
+    isnothing(stokes_drift) && isnothing(particles) && isnothing(immersed_boundary) ||
+        throw(ArgumentError("B200(): stokes_drift, particles and immersed boundaries are not supported"))
     length(tracers) <= MAX_TRACERS || throw(ArgumentError("B200(): at most $MAX_TRACERS tracers"))
     ts = timestepper === :RungeKutta3 ? 1 : timestepper === :QuasiAdamsBashforth2 ? 0 :
          throw(ArgumentError("B200(): timestepper must be :RungeKutta3 or :QuasiAdamsBashforth2"))
@@ -470,13 +503,14 @@ function model_desc(grid, gh; advection, buoyancy, coriolis, closure, tracers, t
         fidx < length(names) ? bc_codes(boundary_conditions[names[fidx + 1]])[side + 1] : BC(0, 0.0)
     end
     frc, frc_tabs = forcing_desc(forcing, grid, names)
+    bg, bg_tabs = background_desc(background_fields, grid, names, clock)
     ptr(v) = isempty(v) ? Ptr{Float64}(C_NULL) : pointer(v)
     desc = ModelDesc(gh, ts, χ, adv_code(advection), advection isa WENO5 ? Int32(advection.zweno) : Int32(1),
                      map(ptr, tabs), clo, ν, κ, fplane, f, btr, tilted, ĝ, length(tracers), bcs, 0,
                      bkind, iT, iS, grav, α, β, smagorinsky_desc(closure, tracers)..., amd_desc(closure, tracers)...,
-                     vertically_implicit(closure), frc)
+                     vertically_implicit(closure), frc, bg)
     # the tables must be GC.@preserve'd across ob200_model_create (host pointers are borrowed)
-    return desc, (tabs, frc_tabs)
+    return desc, (tabs, frc_tabs, bg_tabs)
 end
 
 model_field(mh, name) = (h = Ref{Ptr{Cvoid}}(); check(ccall((:ob200_model_field, lib), Int32,
@@ -515,7 +549,7 @@ function b200_nonhydrostatic_model(; grid, clock = Clock{eltype(grid)}(0, 0, 1),
                             if t !== nothing) for n in names)
     gh = grid_handle(grid)
     desc, keep = model_desc(grid, gh; advection, buoyancy, coriolis, closure, tracers, timestepper,
-                            boundary_conditions = bcs, kw...)
+                            boundary_conditions = bcs, clock, kw...)
     mh = Ref{Ptr{Cvoid}}()
     GC.@preserve keep check(ccall((:ob200_model_create, lib), Int32, (Ref{ModelDesc}, Ref{Ptr{Cvoid}}), desc, mh))
     handle = ModelHandle(mh[])
@@ -538,11 +572,14 @@ function b200_nonhydrostatic_model(; grid, clock = Clock{eltype(grid)}(0, 0, 1),
         (; νₑ = pfield("nu_e"), κₑ = NamedTuple{tracers}(Tuple(pfield("kappa_e$(t - 1)") for t in 1:length(tracers)))) :
         closure isa SmagorinskyLilly ?
         (; νₑ = pfield("nu_e"), κₑ = NamedTuple{tracers}(Tuple(pfield("nu_e") / (closure.Pr isa Number ? closure.Pr : closure.Pr[n]) for n in tracers))) : nothing
+    # the library's background fields "bg_<name>": writing their parent (set!, copyto!) replaces the values from the next step on
+    bgnames = Tuple(n for n in names if haskey(get(kw, :background_fields, NamedTuple()), n))
+    background_fields = NamedTuple{bgnames}(wrap(n, "bg_", FieldBoundaryConditions(grid, loc_of(n))) for n in bgnames)
     solver = B200PoissonSolver(grid)
     return Oceananigans.Models.NonhydrostaticModels.reference_nonhydrostatic_model(;      # the unchanged constructor body (hook 2)
         grid, clock, advection, buoyancy, coriolis, closure, boundary_conditions = bcs, tracers = tracer_fields,
         timestepper = ts, velocities, pressures, diffusivity_fields, pressure_solver = solver,
-        auxiliary_fields = merge(auxiliary_fields, (; b200_handle = handle)))
+        auxiliary_fields = merge(auxiliary_fields, (; b200_handle = handle, b200_background_fields = background_fields)))
 end
 
 const B200Model = NonhydrostaticModel{<:Any, <:Any, <:B200}

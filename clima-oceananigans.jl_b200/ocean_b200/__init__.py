@@ -14,7 +14,8 @@ from .model import (Field, CenterField, XFaceField, YFaceField, ZFaceField, fill
                     HorizontalScalarDiffusivity, FPlane, BuoyancyTracer, Buoyancy, SeawaterBuoyancy,
                     LinearEquationOfState, BoundaryCondition, Relaxation, GaussianMask, LinearTarget,
                     FluxBoundaryCondition, ValueBoundaryCondition, GradientBoundaryCondition,
-                    boundary_values, set_boundary_condition_values, update_state, calculate_tendencies, set_model, time_step, sync)
+                    boundary_values, set_boundary_condition_values, BackgroundField, background_table, set_background,
+                    update_state, calculate_tendencies, set_model, time_step, sync)
 from .output_writers import FieldSlicer, fetch_output, horizontal_average, Checkpointer  # noqa: F401
 from .simulations import (Simulation, run, TimeStepWizard, cell_advection_timescale,  # noqa: F401
                           cell_diffusion_timescale, max_abs_velocities)

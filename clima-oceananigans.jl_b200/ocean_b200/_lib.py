@@ -50,7 +50,8 @@ class ModelDesc(C.Structure):
                 ("smagorinsky_C", C.c_double), ("smagorinsky_Cb", C.c_double), ("prandtl", C.c_double * MAX_TRACERS),
                 ("amd_Cnu", C.c_double), ("amd_Ckappa", C.c_double * MAX_TRACERS), ("amd_Cb", C.c_double),
                 ("amd_has_Cb", C.c_int32), ("closure_vertically_implicit", C.c_int32),
-                ("forcing", Forcing * (3 + MAX_TRACERS))]
+                ("forcing", Forcing * (3 + MAX_TRACERS)),
+                ("background", C.c_void_p * (3 + MAX_TRACERS))]
 
 
 #: every symbol include/ocean_b200.h declares: name -> (restype, argtypes)

@@ -590,6 +590,65 @@ def relaxation_tables(relaxation, loc, grid):
     return md, M, td, T
 
 
+# ---- background fields (src/Models/NonhydrostaticModels/background_fields.jl) ----------------------------
+class BackgroundField:
+    """BackgroundField(func; parameters=nothing) (background_fields.jl): a steady field U(x, y, z, t) that the model's velocities
+    or tracers are perturbations about.  The B200 path tabulates it ONCE, at the clock time of construction: a time-dependent
+    background is updated by the caller, e.g. `set_background(model, "b", func_or_array, time=t)` in a callback."""
+
+    def __init__(self, func, parameters=None):
+        if not callable(func):
+            raise ValueError(f"a BackgroundField needs a callable, got {type(func).__name__}")
+        self.func, self.parameters = func, parameters
+
+
+def _parent_nodes(grid, loc):
+    """x, y, z of every node of the parent array of a field at `loc` (halos included; the extra Face point on Bounded dimensions;
+    the Flat coordinate along Flat dimensions), broadcast-shaped, in double"""
+    out = []
+    for d in range(3):
+        src = grid.F[d] if loc[d] == Face else grid.C[d]
+        if grid.topology[d] == Flat:
+            a = np.asarray(src.span(1, 1))
+        else:
+            n = grid.N[d] + 2 * grid.H[d] + (1 if (loc[d] == Face and grid.topology[d] == Bounded) else 0)
+            a = np.asarray(src.span(1 - grid.H[d], n - grid.H[d]))
+        shape = [1, 1, 1]
+        shape[d] = len(a)
+        out.append(a.astype(np.float64).reshape(shape))
+    return out
+
+
+def background_table(grid, loc, background, time=0.0):
+    """The parent-shaped table of a background (a BackgroundField or a bare callable) for a field at `loc`: the function at every
+    node of the parent, halos included, as the reference's FunctionField evaluates it (its halos are never filled, not even along
+    a Periodic dimension), called as func(x, y, z, t) or func(x, y, z, t, parameters), evaluated in double and rounded once to the
+    grid's float type.  No library call."""
+    bf = background if isinstance(background, BackgroundField) else BackgroundField(background)
+    x, y, z = _parent_nodes(grid, loc)
+    t = np.float64(time)
+    v = bf.func(x, y, z, t) if bf.parameters is None else bf.func(x, y, z, t, bf.parameters)
+    shape = tuple(len(a) for a in (x.ravel(), y.ravel(), z.ravel()))
+    try:
+        v = np.broadcast_to(np.asarray(v, dtype=np.float64), shape)
+    except ValueError:
+        raise ValueError(f"the background function returned shape {np.shape(v)}, which does not broadcast to the field's "
+                         f"parent {shape}") from None
+    return np.asfortranarray(v.astype(grid.FT))
+
+
+def set_background(model, name, value, time=None):
+    """Replace the background of field `name` (one the model was built with): `value` is a parent-shaped array or a function /
+    BackgroundField, evaluated as at construction at `time` (default: the model's clock).  The copy is ordered after every step
+    enqueued so far, so it takes effect from the next step on; this is how a time-dependent background is advanced."""
+    if name not in model.background_fields:
+        raise ValueError(f"{name} has no background field; backgrounds: {tuple(model.background_fields)}")
+    f = model.background_fields[name]
+    if callable(value) or isinstance(value, BackgroundField):
+        value = background_table(model.grid, f.loc, value, model.clock.time if time is None else time)
+    f.set_parent(value)
+
+
 class Clock:
     def __init__(self, model):
         self._m = model
@@ -611,15 +670,17 @@ class NonhydrostaticModel:
     """NonhydrostaticModel(; grid, advection, closure, coriolis, buoyancy, tracers, timestepper,
     boundary_conditions) (src/Models/NonhydrostaticModels/nonhydrostatic_model.jl:102-203).
     Defaults as in the reference: advection = CenteredSecondOrder(), timestepper =
-    :QuasiAdamsBashforth2.  `forcing` = {field name: Relaxation(...)}.  Unsupported pieces (function-valued forcings,
-    function BCs, immersed boundaries, background fields, particles, closures other than ScalarDiffusivity /
-    SmagorinskyLilly / AnisotropicMinimumDissipation) raise ArgumentError-like ValueErrors."""
+    :QuasiAdamsBashforth2.  `forcing` = {field name: Relaxation(...)}.  `background_fields` = {field name: BackgroundField(...)
+    or a callable}: evaluated once, at time 0, over each field's whole parent (background_table); model.background_fields holds
+    the resulting fields and set_background replaces their values.  Unsupported pieces (function-valued forcings, function BCs,
+    immersed boundaries, particles, closures other than ScalarDiffusivity / SmagorinskyLilly / AnisotropicMinimumDissipation)
+    raise ArgumentError-like ValueErrors."""
 
     def __init__(self, grid, advection="default", closure=None, coriolis=None, buoyancy=None, tracers=(),
                  timestepper="QuasiAdamsBashforth2", boundary_conditions=None, forcing=None,
                  background_fields=None, particles=None, immersed_boundary=None, stokes_drift=None,
                  pressure_solver=None, chi=0.1):
-        for name, v in (("background_fields", background_fields), ("particles", particles),
+        for name, v in (("particles", particles),
                         ("immersed_boundary", immersed_boundary), ("stokes_drift", stokes_drift)):
             if v:
                 raise ValueError(f"`{name}` is not supported on the B200 architecture (SURVEY.md 8(b))")
@@ -656,6 +717,14 @@ class NonhydrostaticModel:
                     raise ValueError(f"the forcing of {n} is a {type(fr).__name__}: only Relaxation crosses the C ABI of the B200 "
                                      "architecture (function-valued forcings are outside its supported set)")
                 frc[names.index(n)] = relaxation_tables(fr, locs[names.index(n)], grid)
+        if background_fields is not None and not isinstance(background_fields, dict):
+            raise ValueError("background_fields must be a dict {field name: BackgroundField(...) or a function}")
+        for n, bf in (background_fields or {}).items():
+            if n not in names:
+                raise ValueError(f"{n} is not a prognostic field of the model; background field names must be among {names}")
+            if not (callable(bf) or isinstance(bf, BackgroundField)):
+                raise ValueError(f"the background of {n} is a {type(bf).__name__}: it must be a BackgroundField or a function "
+                                 "(x, y, z, t)")
         # halo inflation (nonhydrostatic_model.jl:140-148)
         H = list(grid.H)
         for term in (advection, closure):
@@ -741,6 +810,11 @@ class NonhydrostaticModel:
                 self._keep.append(a)
                 F.target = a.ctypes.data_as(C.POINTER(C.c_double))
         self.forcing = dict(forcing or {})
+        # backgrounds on the inflated grid (their halos are the function's values there), at the clock time of construction
+        bgt = {n: background_table(grid, locs[names.index(n)], bf, 0.0) for n, bf in (background_fields or {}).items()}
+        for n, t in bgt.items():
+            self._keep.append(t)
+            d.background[names.index(n)] = t.ctypes.data_as(C.c_void_p)
         h = C.c_void_p()
         check(lib.ob200_model_create(C.byref(d), C.byref(h)))
         self.handle = h
@@ -763,6 +837,8 @@ class NonhydrostaticModel:
                    for i, n in enumerate(names)}
         self.Gm = {n: self._field("Gm_" + (n if n in "uvw" else f"c{tracers.index(n)}"), n, locs[i])
                    for i, n in enumerate(names)}
+        self.background_fields = {n: self._field("bg_" + (n if n in "uvw" else f"c{tracers.index(n)}"), n, locs[names.index(n)])
+                                   for n in bgt}
         self.clock = Clock(self)
 
     def _field(self, cname, name, loc):

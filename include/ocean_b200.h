@@ -142,6 +142,13 @@ typedef struct {
     /* forcing = (u = Relaxation(...), ...) (nonhydrostatic_model.jl:102-203, Forcings/model_forcing.jl): per prognostic
      * field u, v, w, tracers...; appended last so that every earlier member keeps its offset */
     ob200_forcing forcing[3 + OB200_MAX_TRACERS];
+    /* background_fields = (u = ..., b = ...) (Models/NonhydrostaticModels/background_fields.jl): per prognostic field u, v, w,
+     * tracers..., a host parent array in the reference layout (grid float type, halos included, at the field's own location)
+     * holding the background at every node, or NULL for none.  The library copies it into a model-owned field ("bg_u",
+     * "bg_v", "bg_w", "bg_c<k>" of ob200_model_field); ob200_field_set_parent on that field replaces the values from the next
+     * step on.  Its halos are never filled.  Each tendency gains - div(U_bg, ψ) - div(U, ψ_bg) with the model's advection
+     * scheme, right after the advection of ψ by U; backgrounds enter no other term.  Appended last like `forcing`. */
+    const void* background[3 + OB200_MAX_TRACERS];
 } ob200_model_desc;
 
 /* ---- library / device ----------------------------------------------------------------- */
@@ -233,7 +240,8 @@ int32_t ob200_batched_tridiagonal_solve(int32_t ftype, int32_t is_complex, int32
 int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model** out);
 int32_t ob200_model_destroy(ob200_model* m);
 /* model.velocities.u / model.tracers.b / model.pressures.pNHS / timestepper.Gⁿ.u ...
- * names: "u","v","w","c<k>" (k-th tracer, 0-based),"pNHS","pHY","Gn_u",...,"Gm_c0","nu_e" (SmagorinskyLilly, AMD),"kappa_e<k>" (AMD).
+ * names: "u","v","w","c<k>" (k-th tracer, 0-based),"pNHS","pHY","Gn_u",...,"Gm_c0","nu_e" (SmagorinskyLilly, AMD),"kappa_e<k>" (AMD),
+ * "bg_u",...,"bg_c<k>" (the background of that field; an error for a field without one).
  * The returned handle is borrowed (owned by the model). */
 int32_t ob200_model_field(ob200_model* m, const char* name, ob200_field** out);
 /* update_state!(model) update_nonhydrostatic_model_state.jl:14-37 */
