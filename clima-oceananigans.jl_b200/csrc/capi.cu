@@ -783,6 +783,15 @@ extern "C" int32_t ob200_batched_tridiagonal_solve(int32_t ftype, int32_t cplx, 
 // ---------------------------------------------------------------------------------------------
 // model
 // ---------------------------------------------------------------------------------------------
+// which kernels compute a model's tendencies (plan_tendencies); per-field kernels:
+enum { TK_TMA, TK_FAST2D, TK_SHARED, TK_CELL };
+struct TendencyPlan {
+    int nfused = 0;                  // leading fields (u, v, w, first tracer) the fused kernel steps: 0, 3 or 4
+    bool closure_pass = false;       // the closure-only pass writes their G^n first, the fused kernel adds the rest
+    bool background_pass = false;    // the background-only pass writes (or adds to) their G^n first, likewise
+    bool split = false;              // the fused launch can run as interior + boundary tile rows (halo overlap)
+    int kernel[3 + OB200_MAX_TRACERS] = {};      // TK_* of every field from nfused on
+};
 struct ob200_model {
     ob200_model_desc desc;
     const ob200_grid* grid;
@@ -802,6 +811,7 @@ struct ob200_model {
     double time = 0, previous_dt = 1.0 / 0.0;
     long long iteration = 0;
     bool use_fast = true;
+    TendencyPlan plan;
     // side streams / events of this model (independent launches of a stage are forked onto them and joined before the
     // stage's next dependent kernel); created on first use, released with the model
     cudaStream_t side[3] = {nullptr, nullptr, nullptr}, hy_stream = nullptr;
@@ -924,6 +934,71 @@ static void build_phys(ob200_model* m) {
     for (int d = 0; d < 3; ++d) P.bgU[d] = P.bg[d] ? P.bg[d] : (m->bg_zero ? m->bg_zero->template p0<FT>() : nullptr);
 }
 
+// The one place that decides which kernels compute the tendencies of a model with `nf` prognostic fields.  It depends only on
+// what is fixed once the model exists: the physics, the forcings and backgrounds, w's Flux conditions (`wbc`: a Bounded z side
+// of w is a wall, which takes no array) and use_fast (false: the general kernels for every field, the reference path of the
+// tests).  The launchers it names rely on it and check nothing.
+template <class FT>
+static TendencyPlan plan_tendencies(const Phys<FT>& P, int nf, const FluxBC<FT>& wbc, bool use_fast) {
+    const GridD<FT>& g = P.g;
+    TendencyPlan t;
+    // the shared-face kernels need a 3-D grid (every direction has two faces to pair) with a halo wide enough for the one extra
+    // face position per direction
+    bool grid3 = true;
+    for (int d = 0; d < 3; ++d) grid3 = grid3 && g.topo[d] != OB_FLAT && g.N[d] >= 2;
+    // the specialised per-field kernels: x and a non-Flat z Periodic, y Periodic or slab-decomposed, all regular with the
+    // uniform WENO5, no closure, vertical gravity; the TMA kernel takes a ragged last tile in y, but Ny % 8 gates 3-D grids too:
+    // which kernel a grid takes decides the rounding of its results
+    const bool hasz = g.topo[2] != OB_FLAT;
+    bool spec = use_fast && P.scheme == ADV_WENO5 && P.closure == CLO_NONE && !P.tilted && g.topo[0] == OB_PERIODIC &&
+                (g.topo[1] == OB_PERIODIC || g.topo[1] == OB_COMM) && (!hasz || g.topo[2] == OB_PERIODIC);
+    for (int d = 0; d < 3; ++d)
+        spec = spec && g.regular[d] && !P.wc[d][0] && !P.wc[d][1] && (g.topo[d] == OB_FLAT || g.H[d] >= 3);
+    spec = spec && g.N[0] % fast::TX == 0 && g.N[1] % fast::TY == 0;
+    if (hasz) spec = spec && (g.S[0] * sizeof(FT)) % 16 == 0;      // tensor-map row strides are multiples of 16 bytes
+    const bool shared = (P.scheme != ADV_NONE || P.closure != CLO_NONE) && grid3;
+    for (int q = 0; q < nf; ++q)      // forced fields and backgrounds: general kernels
+        t.kernel[q] = spec && !P.frc[q].on && !has_background(P, q) ? (hasz ? TK_TMA : TK_FAST2D) : (shared ? TK_SHARED : TK_CELL);
+
+    // the fused kernel (tendency_fused.cu): x Periodic, y Periodic or slab-decomposed, both regular with the uniform WENO5,
+    // vertical gravity, explicit closure; whole tiles in x, 16-byte row strides, 32-bit element offsets
+    bool fused = use_fast && nf >= 3 && P.scheme == ADV_WENO5 && !P.tilted && !P.vitd && g.topo[0] == OB_PERIODIC &&
+                 (g.topo[1] == OB_PERIODIC || g.topo[1] == OB_COMM);
+    for (int d = 0; d < 3; ++d) fused = fused && g.H[d] >= 3 && (d == 2 || (g.regular[d] && !P.wc[d][0] && !P.wc[d][1]));
+    fused = fused && g.N[0] % fz::TX == 0 && (g.S[0] * sizeof(FT)) % 16 == 0 && g.total < (1LL << 31);
+    const int nt = std::min(nf - 3, 1);
+    bool native = false;      // the kernel computes the model's closure itself
+    if (g.topo[2] == OB_PERIODIC) {
+        fused = fused && g.regular[2] && !P.wc[2][0] && !P.wc[2][1];
+        native = P.closure == CLO_NONE;
+    } else if (g.topo[2] == OB_BOUNDED) {
+        // Bounded z (stretched with WENO5(grid) tables, or regular) with a tracer and ScalarDiffusivity (or no closure); it
+        // applies the constant Flux conditions of u, v and the tracer in z, and none of w
+        fused = fused && nt == 1 && g.izC && g.izF && P.wzp[0] && P.wzp[1] && g.N[2] >= 6 && (g.regular[2] || (P.wc[2][0] && P.wc[2][1]));
+        for (int s = 4; s < 6; ++s) fused = fused && !(wbc.kind[s] == 2 && wbc.val[s] != FT(0));
+        native = P.closure == CLO_NONE || P.closure == CLO_3D;
+    } else fused = false;
+    // a closure it does not compute (LES closures; any closure on the triply periodic variant), and background terms: the
+    // shared-face kernel writes them into G^n first, and the accumulate form, which only the variants with a tracer have,
+    // adds the rest
+    bool bg = false;
+    for (int q = 0; q < 3 + nt; ++q) bg = bg || has_background(P, q);
+    if (!native || bg) fused = fused && nt == 1 && grid3;
+    if (!fused) return t;
+    t.nfused = 3 + nt;
+    t.closure_pass = !native;
+    t.background_pass = bg;
+    const int R = fz::rows_per_tile(nt);
+    t.split = R >= fz::HALO && fz::interior_tile_rows(g.N[1], R) >= 1;
+    return t;
+}
+static void plan_model_tendencies(ob200_model* m) {
+    if (m->grid->ftype == OB200_F32)
+        m->plan = plan_tendencies<float>(m->P32, m->nf, constant_flux_bcs<float>(m->F[2].get()), m->use_fast);
+    else
+        m->plan = plan_tendencies<double>(m->P64, m->nf, constant_flux_bcs<double>(m->F[2].get()), m->use_fast);
+}
+
 extern "C" int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model** out) {
     API_BEGIN
     ensure_device();
@@ -1008,6 +1083,7 @@ extern "C" int32_t ob200_model_create(const ob200_model_desc* desc, ob200_model*
     m->solver.reset(s);
     if (m->grid->ftype == OB200_F32) build_phys<float>(m.get());
     else build_phys<double>(m.get());
+    plan_model_tendencies(m.get());
     for (int d = 0; d < 3; ++d) for (int l = 0; l < 2; ++l) m->desc.weno_coeff[d][l] = nullptr;
     for (ob200_forcing& F : m->desc.forcing) F.mask = F.target = nullptr;      // borrowed host tables: copied to the device
     for (const void*& p : m->desc.background) p = nullptr;
@@ -1265,12 +1341,12 @@ static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
         }
     }
     ScopedPhase ph("tendency");
-    // all fields in one persistent launch (tendency_fused.cu) when the configuration allows; `first` = fields it handled
-    int first = 0;
-    if (m->use_fast && m->nf >= 3) {
+    // the leading fields in one persistent launch (tendency_fused.cu), the others per field
+    const TendencyPlan& plan = m->plan;
+    if (plan.nfused) {
         FusedFields<FT> ff;
-        ff.nf = m->nf; ff.pHY = pHY; ff.ss = ss;
-        for (int q = 0; q < m->nf && q < FUSED_MAXF; ++q) {
+        ff.nf = plan.nfused; ff.pHY = pHY; ff.ss = ss;
+        for (int q = 0; q < plan.nfused; ++q) {
             ob200_field* f = m->F[q].get();
             ff.state[q] = f->template p0<FT>();
             ff.Gm[q] = m->Gm[q]->template p0<FT>();
@@ -1278,62 +1354,54 @@ static void model_tendencies(ob200_model* m, const Substep<FT>& ss) {
             ff.nw[q] = ss.mode == SUB_NONE ? nullptr : f->template alt0<FT>();
             ff.fbc[q] = constant_flux_bcs<FT>(f);
         }
-        // a closure the fused kernel does not evaluate itself (LES closures; any closure on the triply periodic variant): its flux
-        // divergence alone goes into G^n through the general shared-face kernel, and the fused kernel adds everything else
-        if (fz::supported<FT>(P, m->nf) == 2 && closure_only_supported<FT>(P)) {
+        const Substep<FT> none{SUB_NONE, FT(0), FT(0), FT(0)};
+        // a closure the fused kernel does not evaluate itself: its flux divergence alone goes into G^n through the shared-face
+        // kernel, and the fused kernel adds everything else
+        if (plan.closure_pass) {
             model_halo_join(m);
-            const int nfused = 3 + std::min(m->nf - 3, 1);
-            const Substep<FT> none{SUB_NONE, FT(0), FT(0), FT(0)};
-            for (int q = 0; q < nfused; ++q)
-                launch_tendency_general<FT>(P, q, U, ff.state[q], pHY, b, ff.fbc[q], ff.Gn[q], ff.Gm[q], nullptr, none, true);
+            for (int q = 0; q < plan.nfused; ++q)
+                launch_tendency_general<FT>(P, q, true, U, ff.state[q], pHY, b, ff.fbc[q], ff.Gn[q], ff.Gm[q], nullptr, none, true);
             ff.accumulate = true;
         }
         // background terms of the fused fields: - div(U_bg, ψ) - div(U, ψ_bg) alone into G^n (onto the closure's part), for the
-        // accumulate form to add the rest; it reads the velocities' y halos, so after the exchange has landed.  The variant
-        // without a tracer has no accumulate form: that model takes the per-field kernels
-        bool bg = false;
-        for (int q = 0; q < 3 + std::min(m->nf - 3, 1); ++q) bg = bg || has_background(P, q);
-        if (bg && m->nf > 3 && fz::supported<FT>(P, m->nf) && background_only_supported<FT>(P)) {
+        // accumulate form to add the rest; it reads the velocities' y halos, so after the exchange has landed
+        if (plan.background_pass) {
             model_halo_join(m);
-            const Substep<FT> none{SUB_NONE, FT(0), FT(0), FT(0)};
-            for (int q = 0; q < 4; ++q)
-                launch_tendency_general<FT>(P, q, U, ff.state[q], pHY, b, ff.fbc[q], ff.Gn[q], ff.Gm[q], nullptr, none, false,
+            for (int q = 0; q < plan.nfused; ++q)
+                launch_tendency_general<FT>(P, q, true, U, ff.state[q], pHY, b, ff.fbc[q], ff.Gn[q], ff.Gm[q], nullptr, none, false,
                                             ff.accumulate ? 2 : 1);
             ff.gn_terms = true;
         }
-        if (bg && !ff.gn_terms) {
-            // no fused launch: the per-field kernels below add the background terms themselves
-        } else if (m->halo_pending) {
+        if (m->halo_pending && plan.split) {
             // the neighbour exchange of the previous stage is still in flight on the halo stream: tile rows that read only rows
             // this rank owns go first, the boundary tile rows once the exchange has landed
-            first = fz::launch<FT>(P, ff, 1);
+            fz::launch<FT>(P, ff, 1);
             model_halo_join(m);
-            if (first) fz::launch<FT>(P, ff, 2);
-            else first = fz::launch<FT>(P, ff, 0);
+            fz::launch<FT>(P, ff, 2);
         } else {
-            first = fz::launch<FT>(P, ff, 0);
+            model_halo_join(m);
+            fz::launch<FT>(P, ff, 0);
         }
     }
     model_halo_join(m);
     if (fork) OB_CUDA(cudaEventRecord(ev_fork, g_stream));
     bool lane_forked[3] = {false, false, false};        // a side stream waits for the fork event before its first launch
-    for (int q = first; q < m->nf; ++q) {
+    for (int q = plan.nfused; q < m->nf; ++q) {
         ob200_field* f = m->F[q].get();
-        const FluxBC<FT> fbc = constant_flux_bcs<FT>(f);
+        const FT* psi = f->template p0<FT>();
+        FT* Gn = m->Gn[q]->template p0<FT>();
+        const FT* Gm = m->Gm[q]->template p0<FT>();
         FT* newp = ss.mode == SUB_NONE ? nullptr : f->template alt0<FT>();
-        bool done = false;
         const int lane = fork ? q % 4 : 0;               // lane 0 = the library stream itself
         if (lane > 0) {
             if (!lane_forked[lane - 1]) { OB_CUDA(cudaStreamWaitEvent(side[lane - 1], ev_fork, 0)); lane_forked[lane - 1] = true; }
             g_override = side[lane - 1];
         }
         try {
-            if (m->use_fast)
-                done = launch_tendency_fast<FT>(P, q, U, f->template p0<FT>(), pHY, m->Gn[q]->template p0<FT>(),
-                                                m->Gm[q]->template p0<FT>(), newp, ss);
-            if (!done)
-                launch_tendency_general<FT>(P, q, U, f->template p0<FT>(), pHY, b, fbc, m->Gn[q]->template p0<FT>(),
-                                            m->Gm[q]->template p0<FT>(), newp, ss);
+            if (plan.kernel[q] == TK_TMA) tma::launch<FT>(P, q, U, psi, pHY, Gn, Gm, newp, ss);
+            else if (plan.kernel[q] == TK_FAST2D) launch_tendency_fast<FT>(P, q, U, psi, pHY, Gn, Gm, newp, ss);
+            else launch_tendency_general<FT>(P, q, plan.kernel[q] == TK_SHARED, U, psi, pHY, b, constant_flux_bcs<FT>(f), Gn, Gm,
+                                             newp, ss);
         } catch (...) { g_override = nullptr; throw; }
         g_override = nullptr;
     }
@@ -1526,7 +1594,11 @@ extern "C" int32_t ob200_model_max_abs_velocities(ob200_model* m, double out[3])
 extern "C" int64_t ob200_debug_cached_tensor_maps(void) { return (int64_t)ob::tmau::cached_maps(); }
 
 // knob used by tests to force the general kernels
-extern "C" int32_t ob200_model_use_fast_kernels(ob200_model* m, int32_t on) { m->use_fast = on != 0; return 0; }
+extern "C" int32_t ob200_model_use_fast_kernels(ob200_model* m, int32_t on) {
+    m->use_fast = on != 0;
+    plan_model_tendencies(m);
+    return 0;
+}
 
 // ---- profiling knobs (not part of the reference interface; bench evidence only) ---------------
 extern "C" int32_t ob200_profile_enable(int32_t on) {

@@ -57,32 +57,40 @@ struct BoundaryFluxes {
     Substep<FT> ss;
 };
 template <class FT> void launch_boundary_fluxes(const GridD<FT>& g, int d, const BoundaryFluxes<FT>& a);
-// general tendency (+ optional fused substep) for prognostic field `comp`
+
+// The tendency launchers below launch what they are given: which of them computes each field, and which instantiation
+// conditions they rely on, is decided once per model by the tendency plan (capi.cu: plan_tendencies).
+//
+// general tendency (+ optional fused substep) for prognostic field `comp`: the shared-face kernel if `shared` (3-D grids),
+// otherwise the one-cell kernel.  closure_only: G^n = the closure's flux divergence alone; background_only = 1 / 2: G^n = / +=
+// - div(U_bg, ψ) - div(U, ψ_bg) alone (zero for a field without background terms); both for the fused kernel's accumulate
+// form, both with the shared-face kernel only
 template <class FT>
-void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
+void launch_tendency_general(const Phys<FT>& P, int comp, bool shared, const FT* const U[3], const FT* psi,
                              const FT* pHY, const Buoy<FT>& b, const FluxBC<FT>& fbc, FT* Gn,
                              const FT* Gm, FT* psi_new, const Substep<FT>& ss, bool closure_only = false,
                              int background_only = 0);
-// true if launch_tendency_general(..., closure_only = true) is available for this model (3-D grid)
-template <class FT> bool closure_only_supported(const Phys<FT>& P);
-// background_only = 1 / 2: G^n = / += - div(U_bg, ψ) - div(U, ψ_bg) alone (zero for a field without background terms), for the
-// fused kernel's accumulate form; true if available for this model (3-D grid, an advection scheme)
-template <class FT> bool background_only_supported(const Phys<FT>& P);
-// fast path (all non-Flat dimensions periodic, regular, WENO5 uniform, no closure, optional FPlane, field not forced and
-// without background terms):
-// the TMA-staged kernel on 3-D grids, the direct-load kernel on 2-D grids; returns false if the configuration is not
-// covered
+// the specialised per-field kernels (all non-Flat dimensions periodic, regular, WENO5 uniform, no closure, optional FPlane,
+// field not forced and without background terms): the TMA-staged kernel on 3-D grids (tendency_tma.cu; 16-byte row strides),
+// the direct-load kernel on 2-D grids (tendency_fast.cu); both on grids of whole TX x TY tiles
+namespace fast {
+constexpr int TX = 32, TY = 8;   // tile of the direct-load kernel = TX x TY cells, one thread per cell
+}
+namespace tma {
 template <class FT>
-bool launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
+void launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, const FT* pHY, FT* Gn, const FT* Gm,
+            FT* psi_new, const Substep<FT>& ss);
+}
+template <class FT>
+void launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
                           const FT* pHY, FT* Gn, const FT* Gm, FT* psi_new, const Substep<FT>& ss);
 
-// tendency_fused.cu: all prognostic fields of the specialised configuration in ONE launch.  Returns how many leading
-// fields (u, v, w, first tracer) it handled: 0 if the configuration is not covered, otherwise 3 + min(ntracers, 1);
-// the caller steps the remaining tracers with the per-field kernels.
+// tendency_fused.cu: the leading prognostic fields (u, v, w and the first tracer if there is one) of the specialised
+// configuration in ONE launch; the caller steps the remaining tracers with the per-field kernels.
 constexpr int FUSED_MAXF = 5;
 template <class FT>
 struct FusedFields {
-    int nf;
+    int nf;                          // fields it steps: 3 or 4
     const FT* state[FUSED_MAXF];     // Julia-(0,0,0) pointers: u, v, w, tracers
     const FT* Gm[FUSED_MAXF];
     FT* Gn[FUSED_MAXF];
@@ -93,13 +101,23 @@ struct FusedFields {
     bool accumulate = false;         // G^n already holds the closure's part (launch_tendency_general closure_only): add to it
     bool gn_terms = false;           // G^n already holds precomputed terms (background pass, relaxation pass): add to it
 };
-// part: 0 = every tile; 1 = the tile rows whose stencils stay inside the rows this rank owns along a slab-decomposed y (they
-// need no neighbour data); 2 = the remaining (boundary) tile rows.  Returns the number of fields handled, 0 = not applicable.
 namespace fz {
-template <class FT> int launch(const Phys<FT>& P, const FusedFields<FT>& a, int part = 0);
-// 0: not applicable; 1: handles the model's closure itself (or there is none); 2: applicable if the closure's flux divergence
-// is precomputed into G^n (FusedFields::accumulate)
-template <class FT> int supported(const Phys<FT>& P, int nf);
+constexpr int TX = 32, HALO = 3;     // tile width (grids of whole tiles in x); stencil reach
+// rows per tile: the largest for which the block (NG (R + 1) + 1 warps) keeps 72 registers per thread and the rings + exchange
+// buffers fit 227 KB; measured at 256^3: R = 12 3.13 ms per step, 11: 3.16, 10: 3.26, 9: 3.19; Bounded z at 512 x 512 x 256:
+// R = 12 15.4 ms per step of tendencies, 10: 17.2, 8: 15.4
+constexpr int rows_per_tile(int ntracers) { return ntracers ? 12 : 8; }
+// part launches: the tile rows 1 .. n of the cdiv(Ny, R) rows of tiles are interior, their stencils (HALO rows beyond the
+// tile) stay inside rows 1 .. Ny (with R >= HALO, row 0 is the only one at the low end that does not); returns n
+inline int interior_tile_rows(int Ny, int R) {
+    const int nty = cdiv(Ny, R);
+    int nb_hi = 0;
+    while (nb_hi < nty && (nty - nb_hi) * R + HALO > Ny) ++nb_hi;
+    return nty - nb_hi - 1;
+}
+// part: 0 = every tile; 1 = the interior tile rows, which read only the rows this rank owns along a slab-decomposed y (they
+// need no neighbour data); 2 = the remaining (boundary) tile rows
+template <class FT> void launch(const Phys<FT>& P, const FusedFields<FT>& a, int part = 0);
 }
 
 // SmagorinskyLilly eddy viscosity over the interior (the caller fills its halos)

@@ -597,24 +597,7 @@ __global__ void __launch_bounds__(256, (CO || BG == 2 ? 4 : 3)) tendency_shared_
 }
 
 template <class FT>
-bool closure_only_supported(const Phys<FT>& P) {
-    if (P.closure == CLO_NONE) return false;
-    for (int d = 0; d < 3; ++d) if (P.g.topo[d] == OB_FLAT || P.g.N[d] < 2) return false;
-    return true;
-}
-template bool closure_only_supported<float>(const Phys<float>&);
-template bool closure_only_supported<double>(const Phys<double>&);
-template <class FT>
-bool background_only_supported(const Phys<FT>& P) {
-    if (P.scheme == ADV_NONE) return false;
-    for (int d = 0; d < 3; ++d) if (P.g.topo[d] == OB_FLAT || P.g.N[d] < 2) return false;
-    return true;
-}
-template bool background_only_supported<float>(const Phys<float>&);
-template bool background_only_supported<double>(const Phys<double>&);
-
-template <class FT>
-void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
+void launch_tendency_general(const Phys<FT>& P, int comp, bool shared, const FT* const U[3], const FT* psi,
                              const FT* pHY, const Buoy<FT>& b, const FluxBC<FT>& fbc, FT* Gn,
                              const FT* Gm, FT* psi_new, const Substep<FT>& ss, bool closure_only, int background_only) {
     TendArgs<FT> A;
@@ -622,13 +605,6 @@ void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], 
     A.psi = psi; A.pHY = pHY; A.b = b; A.Gn = Gn; A.Gm = Gm; A.psi_new = psi_new;
     A.ss = ss; A.fbc = fbc; A.comp = comp; A.closure_only = closure_only ? 1 : 0; A.bg_acc = background_only == 2 ? 1 : 0;
     const bool bg = has_background(P, comp);
-    // shared-face variant: 3-D grids (every direction has two faces to pair) with a halo wide enough for the one
-    // extra face position per direction
-    bool shared = P.scheme != ADV_NONE || P.closure != CLO_NONE;
-    for (int d = 0; d < 3; ++d) shared = shared && P.g.topo[d] != OB_FLAT && P.g.N[d] >= 2;
-    if (closure_only && !shared) throw Error("closure-only tendencies need the shared-face kernel (3-D grid)");
-    if (background_only && !(shared && background_only_supported(P)))
-        throw Error("background-only tendencies need the shared-face kernel (3-D grid, an advection scheme)");
     const bool spec = P.g.topo[0] == OB_PERIODIC && P.g.topo[1] == OB_PERIODIC && P.g.topo[2] == OB_BOUNDED &&
                       P.g.regular[0] && P.g.regular[1] && P.scheme == ADV_WENO5 && P.buffer == 2 && !P.tilted && !P.vitd &&
                       !P.wc[0][0] && !P.wc[0][1] && !P.wc[1][0] && !P.wc[1][1];
@@ -662,10 +638,10 @@ void launch_tendency_general(const Phys<FT>& P, int comp, const FT* const U[3], 
 #undef GK
     OB_LAUNCH_CHECK();
 }
-template void launch_tendency_general<float>(const Phys<float>&, int, const float* const[3], const float*,
+template void launch_tendency_general<float>(const Phys<float>&, int, bool, const float* const[3], const float*,
                                              const float*, const Buoy<float>&, const FluxBC<float>&, float*,
                                              const float*, float*, const Substep<float>&, bool, int);
-template void launch_tendency_general<double>(const Phys<double>&, int, const double* const[3], const double*,
+template void launch_tendency_general<double>(const Phys<double>&, int, bool, const double* const[3], const double*,
                                               const double*, const Buoy<double>&, const FluxBC<double>&, double*,
                                               const double*, double*, const Substep<double>&, bool, int);
 

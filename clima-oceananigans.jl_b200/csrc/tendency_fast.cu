@@ -1,8 +1,8 @@
 // tendency_fast.cu -- specialised tendency (+ fused RK3/AB2 substep) kernel for the headline
 // configuration: every non-Flat dimension Periodic, regular spacing, WENO5 with uniform
 // coefficients (Z or JS weights), closure = nothing, optional FPlane and hydrostatic pressure.
-// launch_tendency_fast sends 3-D grids to the TMA-staged kernel (tendency_tma.cu); the kernel here
-// runs the 2-D grids (z Flat).
+// The tendency plan (capi.cu: plan_tendencies) sends 3-D grids to the TMA-staged kernel (tendency_tma.cu); the kernel
+// here runs the 2-D grids (z Flat).
 //
 // Same quantities as physics.cuh (reference files cited there), reorganised for the FP64 pipe,
 // which is what bounds this kernel on B200 (about 20-30 flop per byte of compulsory traffic):
@@ -22,15 +22,7 @@
 
 namespace ob {
 
-namespace tma {   // tendency_tma.cu
-template <class FT>
-void launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, const FT* pHY, FT* Gn, const FT* Gm,
-            FT* psi_new, const Substep<FT>& ss);
-}
-
 namespace fast {
-
-constexpr int TX = 32, TY = 8;   // tile = TX x TY cells, one thread per cell
 
 template <class FT>
 struct Ctx {
@@ -140,26 +132,9 @@ void launch(const Ctx<FT>& c, int comp) {
 }  // namespace fast
 
 template <class FT>
-bool launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
+void launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi,
                           const FT* pHY, FT* Gn, const FT* Gm, FT* psi_new, const Substep<FT>& ss) {
     const GridD<FT>& g = P.g;
-    if (P.frc[comp].on || has_background(P, comp)) return false;      // forced fields and backgrounds: general kernels
-    if (P.scheme != ADV_WENO5 || P.closure != CLO_NONE || P.tilted) return false;
-    bool hasz = g.topo[2] != OB_FLAT;
-    if (g.topo[0] != OB_PERIODIC || (g.topo[1] != OB_PERIODIC && g.topo[1] != OB_COMM) || (hasz && g.topo[2] != OB_PERIODIC)) return false;
-    for (int d = 0; d < 3; ++d) {
-        if (!g.regular[d]) return false;
-        if (P.wc[d][0] || P.wc[d][1]) return false;
-        if (g.topo[d] != OB_FLAT && g.H[d] < 3) return false;
-    }
-    // the TMA kernel takes a ragged last tile in y, but Ny % 8 gates 3-D grids too: which kernel a grid takes decides
-    // the rounding of its results
-    if (g.N[0] % fast::TX || g.N[1] % fast::TY) return false;
-    if (hasz) {
-        if ((g.S[0] * sizeof(FT)) % 16) return false;     // tensor-map row strides are multiples of 16 bytes
-        tma::launch<FT>(P, comp, U, psi, pHY, Gn, Gm, psi_new, ss);
-        return true;
-    }
     fast::Ctx<FT> c;
     for (int d = 0; d < 2; ++d) { c.U[d] = U[d]; c.N[d] = g.N[d]; c.invd[d] = 1 / g.d[d]; }
     for (int d = 0; d < 3; ++d) c.s[d] = g.st[d];
@@ -168,10 +143,9 @@ bool launch_tendency_fast(const Phys<FT>& P, int comp, const FT* const U[3], con
     c.invV = 1 / ((g.d[0] * g.d[1]) * g.d[2]);
     c.f = P.f; c.fplane = P.fplane;
     if (P.zweno) fast::launch<FT, true>(c, comp); else fast::launch<FT, false>(c, comp);
-    return true;
 }
-template bool launch_tendency_fast<float>(const Phys<float>&, int, const float* const[3], const float*,
+template void launch_tendency_fast<float>(const Phys<float>&, int, const float* const[3], const float*,
                                           const float*, float*, const float*, float*, const Substep<float>&);
-template bool launch_tendency_fast<double>(const Phys<double>&, int, const double* const[3], const double*,
+template void launch_tendency_fast<double>(const Phys<double>&, int, const double* const[3], const double*,
                                            const double*, double*, const double*, double*, const Substep<double>&);
 }  // namespace ob

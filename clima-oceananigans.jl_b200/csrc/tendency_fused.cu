@@ -43,7 +43,7 @@
 namespace ob {
 namespace fz {
 
-constexpr int TX = 32, HALO = 3, COL0 = HALO + 1, BX = TX + 2 * HALO + 2, SLOTS = 8;
+constexpr int COL0 = HALO + 1, BX = TX + 2 * HALO + 2, SLOTS = 8;      // TX, HALO: internal.h
 
 template <int NT> struct Groups {          // field -> group map
     static constexpr int NF = 3 + NT;
@@ -523,16 +523,6 @@ tendency_fused_kernel(const __grid_constant__ KArgs<FT, 3 + NT, FRC> c) {
 }
 
 // ---- host side --------------------------------------------------------------------------------
-// part launches (FusedFields / launch): whether the grid has interior tile rows to split off
-template <int R>
-static bool part_applicable(int Ny, int part) {
-    if (!part) return true;
-    const int nty = cdiv(Ny, R);
-    int nb_hi = 0;
-    while (nb_hi < nty && (nty - nb_hi) * R + HALO > Ny) ++nb_hi;
-    return nty - nb_hi - 1 >= 1 && R >= HALO;
-}
-
 // Relaxation forcing of the fused fields as a pointwise pass into G^n (G^n = F, or G^n += F over the closure's part and / or
 // the background terms), for the accumulate instantiations to add the rest: the forced FP64 variants with a tracer that would
 // spill with the term in the epilogue (launch_frc).  The accumulate form adds G^n of EVERY field, so without precomputed terms
@@ -561,7 +551,7 @@ __global__ void __launch_bounds__(128) relaxation_pass_kernel(const __grid_const
     }
 }
 template <class FT, bool ZW, int ZT, int NT, bool HAS_GM, bool ACC, int R, bool FRC>
-static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
+static void launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
     using GR = Groups<NT>;
     constexpr int NF = GR::NF;
     using G_ = Geo<FT, R, NF>;
@@ -583,12 +573,8 @@ static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part
         c.ntiles = c.ntx * nty;
         c.tile0 = 0; c.tsplit = 1 << 30; c.tskip = 0;
         if (part) {
-            if (!part_applicable<R>(g.N[1], part)) return false;
-            // tile rows at the high end whose stencil (HALO rows beyond the tile) reaches past row Ny
-            int nb_hi = 0;
-            while (nb_hi < nty && (nty - nb_hi) * R + HALO > g.N[1]) ++nb_hi;
-            const int nint = nty - nb_hi - 1;          // tile rows 1 .. nty - nb_hi - 1 (R >= HALO: row 0 is the only low one)
-            if (nint < 1 || R < HALO) return false;
+            // interior tile rows 1 .. nint; boundary tile rows 0 and the nb_hi at the high end
+            const int nint = interior_tile_rows(g.N[1], R), nb_hi = nty - 1 - nint;
             if (part == 1) { c.tile0 = c.ntx; c.ntiles = nint * c.ntx; }
             else { c.ntiles = (1 + nb_hi) * c.ntx; c.tsplit = c.ntx; c.tskip = nint * c.ntx; }
         }
@@ -627,40 +613,37 @@ static bool launch_variant(const Phys<FT>& P, const FusedFields<FT>& a, int part
     c.chunk = cdiv((long long)(c.ntiles - (c.ntiles / grid) * grid) * c.Nz, grid);
     kern<<<grid, TX * (GR::NG * (R + 1) + 1), G_::SMEM, stream()>>>(c);
     OB_LAUNCH_CHECK();
-    return true;
 }
 
 template <class FT, bool ZW, int ZT, int NT, int R, bool FRC>
-static bool launch_gm(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
+static void launch_gm(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
     const bool has_gm = a.ss.mode == SUB_RK3 || a.ss.mode == SUB_AB2;
     // the accumulate form (closure's part, backgrounds and / or the forcing precomputed into G^n) exists for the variants with
-    // a tracer
+    // a tracer; the tendency plan gives the variant without one no precomputed terms
     if constexpr (NT == 1) {
         if (a.accumulate || a.gn_terms) {
-            if (has_gm) return launch_variant<FT, ZW, ZT, NT, true, true, R, FRC>(P, a, part);
-            return launch_variant<FT, ZW, ZT, NT, false, true, R, FRC>(P, a, part);
+            if (has_gm) launch_variant<FT, ZW, ZT, NT, true, true, R, FRC>(P, a, part);
+            else launch_variant<FT, ZW, ZT, NT, false, true, R, FRC>(P, a, part);
+            return;
         }
-    } else {
-        if (a.accumulate || a.gn_terms) return false;
     }
-    if (has_gm) return launch_variant<FT, ZW, ZT, NT, true, false, R, FRC>(P, a, part);
-    return launch_variant<FT, ZW, ZT, NT, false, false, R, FRC>(P, a, part);
+    if (has_gm) launch_variant<FT, ZW, ZT, NT, true, false, R, FRC>(P, a, part);
+    else launch_variant<FT, ZW, ZT, NT, false, false, R, FRC>(P, a, part);
 }
 // a model with a forced field among the fused ones takes the FRC instantiations (the term in the per-cell epilogue); every
 // other keeps the unforced kernels.  The FP64 variants with a tracer are at the 72-register cap already and would spill
 // 16-100 bytes more with the term (ptxas -v, sm_100a): there a pointwise pass writes the forcing into G^n and the
 // accumulate instantiation adds the rest, one extra read and write of G^n and a read of the field per forced field
 template <class FT, bool ZW, int ZT, int NT, int R>
-static bool launch_frc(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
+static void launch_frc(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
     constexpr int NF = 3 + NT;
     bool frc = false;
     for (int f = 0; f < NF; ++f) frc = frc || P.frc[f].on;
     if (!frc) return launch_gm<FT, ZW, ZT, NT, R, false>(P, a, part);
     if constexpr (sizeof(FT) == 4 || NT == 0) {
-        return launch_gm<FT, ZW, ZT, NT, R, true>(P, a, part);
+        launch_gm<FT, ZW, ZT, NT, R, true>(P, a, part);
     } else {
         const GridD<FT>& g = P.g;
-        if (!part_applicable<R>(g.N[1], part)) return false;
         if (part != 2) {               // once per stage: before the first (or the only) part
             RelaxPass<FT> r;
             r.nf = NF; r.acc = (a.accumulate || a.gn_terms) ? 1 : 0;
@@ -673,71 +656,25 @@ static bool launch_frc(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
         }
         FusedFields<FT> b = a;
         b.gn_terms = true;
-        return launch_gm<FT, ZW, ZT, NT, R, false>(P, b, part);
+        launch_gm<FT, ZW, ZT, NT, R, false>(P, b, part);
     }
 }
 
-// the configuration checks: returns -1 (not applicable) or the z variant (0 Periodic regular, 1 Bounded); `native` = the kernel
-// computes the model's closure itself (none, or ScalarDiffusivity ThreeDimensional on the Bounded variant)
+// the z variant: ZT = 0 Periodic regular z, ZT = 1 Bounded z
 template <class FT>
-static int classify(const Phys<FT>& P, int nf, bool& native) {
-    const GridD<FT>& g = P.g;
-    native = false;
-    if (P.scheme != ADV_WENO5 || P.tilted || P.vitd) return -1;
-    if (g.topo[0] != OB_PERIODIC || (g.topo[1] != OB_PERIODIC && g.topo[1] != OB_COMM)) return -1;
-    for (int d = 0; d < 3; ++d)
-        if (g.H[d] < 3 || (d < 2 && (!g.regular[d] || P.wc[d][0] || P.wc[d][1]))) return -1;
-    if (g.N[0] % TX || (g.S[0] * sizeof(FT)) % 16 || g.total >= (1LL << 31)) return -1;
-    if (nf < 3) return -1;
-    const int nt = std::min(nf - 3, 1);
-    // ZT = 1: Bounded z (stretched with WENO5(grid) tables, or regular) with ScalarDiffusivity (or no closure) and constant
-    // Flux BCs in z
-    if (g.topo[2] == OB_PERIODIC) {
-        if (!g.regular[2] || P.wc[2][0] || P.wc[2][1]) return -1;
-        native = P.closure == CLO_NONE;
-        return 0;
+void launch(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
+#define GO(ZTV, NTV)                                                                                                   \
+    {                                                                                                                  \
+        if (P.zweno) launch_frc<FT, true, ZTV, NTV, rows_per_tile(NTV)>(P, a, part);                                   \
+        else launch_frc<FT, false, ZTV, NTV, rows_per_tile(NTV)>(P, a, part);                                          \
     }
-    if (g.topo[2] == OB_BOUNDED) {
-        if (nt == 0 || !g.izC || !g.izF || !P.wzp[0] || !P.wzp[1] || g.N[2] < 6) return -1;
-        if (!g.regular[2] && (!P.wc[2][0] || !P.wc[2][1])) return -1;      // stretched z without coefficient tables
-        native = P.closure == CLO_NONE || P.closure == CLO_3D;
-        return 1;
-    }
-    return -1;
-}
-template <class FT>
-int supported(const Phys<FT>& P, int nf) {
-    bool native;
-    const int zt = classify(P, nf, native);
-    return zt < 0 ? 0 : (native ? 1 : (nf > 3 ? 2 : 0));
-}
-template int supported<float>(const Phys<float>&, int);
-template int supported<double>(const Phys<double>&, int);
-
-template <class FT>
-int launch(const Phys<FT>& P, const FusedFields<FT>& a, int part) {
-    const GridD<FT>& g = P.g;
-    bool native;
-    const int zt = classify(P, a.nf, native);
-    if (zt < 0 || (!native && !a.accumulate)) return 0;
-    const int nt = std::min(a.nf - 3, 1);
-    if (zt == 1)
-        for (int s = 4; s < 6; ++s)
-            if (a.fbc[2].kind[s] == 2 && a.fbc[2].val[s] != FT(0)) return 0;      // w has no Flux BCs on a Bounded z
-    (void)g;
-    bool ok = false;
-#define GO(ZTV, NTV, RV)                                                                        \
-    { ok = P.zweno ? launch_frc<FT, true, ZTV, NTV, RV>(P, a, part) : launch_frc<FT, false, ZTV, NTV, RV>(P, a, part); }
-    // rows per tile: the largest for which the block (NG (R + 1) + 1 warps) keeps 72 registers per thread and the rings
-    // + exchange buffers fit 227 KB; measured at 256^3: R = 12 3.13 ms per step, 11: 3.16, 10: 3.26, 9: 3.19
-    if (zt) GO(1, 1, 12)         // Bounded z at 512 x 512 x 256: R = 12 15.4 ms per step of tendencies, 10: 17.2, 8: 15.4
-    else if (nt == 0) GO(0, 0, 8)
-    else GO(0, 1, 12)
+    if (P.g.topo[2] == OB_BOUNDED) GO(1, 1)
+    else if (a.nf == 3) GO(0, 0)
+    else GO(0, 1)
 #undef GO
-    return ok ? 3 + nt : 0;
 }
-template int launch<float>(const Phys<float>&, const FusedFields<float>&, int);
-template int launch<double>(const Phys<double>&, const FusedFields<double>&, int);
+template void launch<float>(const Phys<float>&, const FusedFields<float>&, int);
+template void launch<double>(const Phys<double>&, const FusedFields<double>&, int);
 
 }  // namespace fz
 }  // namespace ob

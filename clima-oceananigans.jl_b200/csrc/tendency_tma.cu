@@ -277,7 +277,8 @@ static void launch_one(Ctx<FT>& c, const GridD<FT>& g, const FT* const U[3], con
     OB_LAUNCH_CHECK();
 }
 
-// eligibility (3-D grid, Nx % 32 == 0, 16-byte row strides, field not forced) is checked by launch_tendency_fast
+// eligibility (3-D grid, Nx % 32 == 0, 16-byte row strides, field not forced) is decided by the tendency plan
+// (capi.cu: plan_tendencies)
 template <class FT>
 void launch(const Phys<FT>& P, int comp, const FT* const U[3], const FT* psi, const FT* pHY, FT* Gn, const FT* Gm,
             FT* psi_new, const Substep<FT>& ss) {
