@@ -73,9 +73,22 @@ def check(what, cuda, o32, o64, absolute=None):
         assert e_c <= absolute, f"{what}: CUDA Float32 rel err {e_c:.3e} > {absolute:g}"
 
 
-def run_model_case(ob, what, build, cfg, seed, steps=3):
+def run_model_case(ob, what, build, cfg, seed, steps=3, expected_over=()):
     """build(M, cfg, FT) -> (oracle model, M's model).  After set! and the projection: states, pHY′, νₑ / κₑ (halos included);
-    then the tendencies; then states and pNHS after each of `steps` steps"""
+    then the tendencies; then states and pNHS after each of `steps` steps.  The checks named in `expected_over` ("set/w",
+    "G/v", "step1/pNHS", ...) may exceed the relative bound: they are measured and keep any absolute bound, every other check is
+    asserted as usual.  Returns {check: ratio to (the Float32 oracle's error + eps32)} of those checks."""
+    measured = {}
+
+    def check_(label, cuda, o32, o64, absolute=None):
+        if label not in expected_over:
+            return check(f"{what}/{label}", cuda, o32, o64, absolute)
+        e_c, e_o = relerr(cuda, o64), relerr(o32, o64)
+        measured[label] = e_c / (e_o + EPS32)
+        print(f"F32 {what}/{label}: e_cuda {e_c:.3e} e_o32 {e_o:.3e} ratio {measured[label]:.3f} (expected over)")
+        if absolute is not None:
+            assert e_c <= absolute, f"{what}/{label}: CUDA Float32 rel err {e_c:.3e} > {absolute:g}"
+
     mo32, mb = build(ob, cfg, np.float32)
     mo64, _ = build(_OracleOnly(ob), rounded(cfg), np.float64)
     rec = _Recorder()
@@ -85,29 +98,30 @@ def run_model_case(ob, what, build, cfg, seed, steps=3):
 
     def states(when):
         for n in mo64.names:
-            check(f"{what}/{when}/{n}", mb.fields[n].interior(), mo32.fields[n].interior, mo64.fields[n].interior, STATE_TOL)
+            check_(f"{when}/{n}", mb.fields[n].interior(), mo32.fields[n].interior, mo64.fields[n].interior, STATE_TOL)
 
     states("set")
     if mo64.pHY is not None:
-        check(f"{what}/set/pHY", mb.pressures["pHY′"].interior(), mo32.pHY.interior, mo64.pHY.interior)
+        check_("set/pHY", mb.pressures["pHY′"].interior(), mo32.pHY.interior, mo64.pHY.interior)
     if getattr(mo64, "νe", None) is not None:
-        check(f"{what}/set/nu_e", mb.diffusivity_fields["νₑ"].parent(), mo32.νe.parent, mo64.νe.parent)
+        check_("set/nu_e", mb.diffusivity_fields["νₑ"].parent(), mo32.νe.parent, mo64.νe.parent)
         if getattr(mo64, "κe", None) is not None:
             for n in mo64.tracer_names:
-                check(f"{what}/set/kappa_e_{n}", mb.diffusivity_fields["κₑ"][n].parent(), mo32.κe[n].parent, mo64.κe[n].parent)
+                check_(f"set/kappa_e_{n}", mb.diffusivity_fields["κₑ"][n].parent(), mo32.κe[n].parent, mo64.κe[n].parent)
     mo32.calculate_tendencies()
     mo64.calculate_tendencies()
     ob.calculate_tendencies(mb)
     g = mo64.grid
     ijk = O.R(1, g.Nx), O.R(1, g.Ny), O.R(1, g.Nz)
     for n in mo64.names:
-        check(f"{what}/G/{n}", mb.Gn[n].interior()[:g.Nx, :g.Ny, :g.Nz], mo32.Gn[n][ijk], mo64.Gn[n][ijk])
+        check_(f"G/{n}", mb.Gn[n].interior()[:g.Nx, :g.Ny, :g.Nz], mo32.Gn[n][ijk], mo64.Gn[n][ijk])
     for step in range(1, steps + 1):
         mo32.time_step(cfg["dt"])
         mo64.time_step(cfg["dt"])
         ob.time_step(mb, cfg["dt"])
         states(f"step{step}")
-        check(f"{what}/step{step}/pNHS", mb.pressures["pNHS"].interior(), mo32.pNHS.interior, mo64.pNHS.interior)
+        check_(f"step{step}/pNHS", mb.pressures["pNHS"].interior(), mo32.pNHS.interior, mo64.pNHS.interior)
+    return measured
 
 
 # ---- a. every parity configuration ---------------------------------------------------------------------------------------------

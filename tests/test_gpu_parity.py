@@ -329,7 +329,9 @@ CONFIGS = {
 def build_models(ob, cfg, FT):
     go, gb = make_pair(ob, FT, cfg["size"], cfg["topology"], coords=cfg.get("coords"), extent=cfg.get("extent"))
     adv = cfg["adv"]
-    if adv == "WENO5":
+    if adv is None:
+        ao = ab = None
+    elif adv == "WENO5":
         ao, ab = O.WENO5(FT), ob.WENO5(FT)
     elif adv == "WENO5js":
         ao, ab = O.WENO5(FT, zweno=False), ob.WENO5(FT, zweno=False)

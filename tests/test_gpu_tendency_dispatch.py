@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 import oracle as O
+from test_gpu_advection_walls import CASES as WALLS
 from test_gpu_background import SHEAR, STRAT, build_bg
 from test_gpu_parity import CONFIGS, init_state
 
@@ -174,6 +175,28 @@ CASES = {
         "ob::tendency_shared_kernel<double, 1, 1, 0, 0>": 3,
         "ob::tendency_shared_kernel<double, 2, 1, 0, 0>": 3,
         "ob::tendency_shared_kernel<double, 3, 1, 0, 0>": 3}),
+    # the wall cases of test_gpu_advection_walls.py: a Bounded x at the seam size (several x, y tiles and z chunks) and any
+    # scheme but the uniform WENO5 take the generic shared-face kernel, a 2-D Flat-z grid with a Bounded x the one-cell kernel
+    "walls_weno_bounded_x_seam": (WALLS["WENO5-BPP-seam"][0], None, None, np.float64, True, {
+        "ob::tendency_shared_kernel<double, 0, 0, 0, 0>": 3,
+        "ob::tendency_shared_kernel<double, 1, 0, 0, 0>": 3,
+        "ob::tendency_shared_kernel<double, 2, 0, 0, 0>": 3,
+        "ob::tendency_shared_kernel<double, 3, 0, 0, 0>": 3}),
+    "walls_upwind1_bounded_z": (WALLS["U1-PPB-seam"][0], None, None, np.float64, True, {
+        "ob::tendency_shared_kernel<double, 0, 0, 0, 0>": 1,
+        "ob::tendency_shared_kernel<double, 1, 0, 0, 0>": 1,
+        "ob::tendency_shared_kernel<double, 2, 0, 0, 0>": 1,
+        "ob::tendency_shared_kernel<double, 3, 0, 0, 0>": 1}),
+    "walls_upwind3_bounded_x_flat_z": (WALLS["U3-BPF-seam"][0], None, None, np.float64, True, {
+        "ob::tendency_general_kernel<double, 0, false>": 1,
+        "ob::tendency_general_kernel<double, 1, false>": 1,
+        "ob::tendency_general_kernel<double, 2, false>": 1,
+        "ob::tendency_general_kernel<double, 3, false>": 1}),
+    # ... and (P, P, B) with the uniform WENO5 at Nx = 32 the fused Bounded-z kernel, in both precisions
+    "walls_weno_bounded_z_fused": (WALLS["WENO5-PPB-fused"][0], None, None, np.float64, True, {
+        "ob::fz::tendency_fused_kernel<double, true, 1, 1, true, false, 12, false>": 1}),
+    "walls_weno_bounded_z_fused_f32": (WALLS["WENO5-PPB-fused"][0], None, None, np.float32, True, {
+        "ob::fz::tendency_fused_kernel<float, true, 1, 1, true, false, 12, false>": 1}),
 }
 
 
